@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — SINDy train-step throughput on B200 (BASELINE.json metric), one process per GPU.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nproc-per-node N ... bench.py --gpus N --steps K --warmup W
 
 Workload (BASELINE.json configs[4], SURVEY.md §8d "C5"): synthetic library fit, N = 1e8 samples in total,
@@ -22,11 +22,15 @@ the timed region — and a device->host read of the loss; roofline = the fused k
 live by sb_fp32_peak (not in MEASURED_PEAKS.json) and, as roofline_hbm, against the measured HBM copy bandwidth;
 cpu_baseline = the reference arm below, run as a child process on a bounded sample.
 
+`--dump-outputs DIR` writes what the last of the K timed steps returned to its caller — loss.npy (the loss before the
+update), grad.npy, xi.npy (the updated coefficients) and, on the one-launch path, adam_moments.npy (m and v) — for
+comparing two builds on the same seeded inputs.
+
 `--impl reference` (rank 0 only) times the reference's OWN CPU implementation of the same step on the box's host cores:
-`SINDyRegression` imported from baseline/_ref (the unmodified reference, mirrored there by `__graft_entry__.build()`),
+`SINDyRegression` imported from oracle/_ref (the unmodified reference, mirrored there by `__graft_entry__.build()`),
 its forward, `MSELoss`, the `jvp`-based regulariser of `train.py:503-507`, L1, `backward`, `torch.optim.Adam.step()`.
 The reference's library stops at degree 3, so the degree-4/5 columns of C5 are appended to ITS `terms` list in its own
-cat-of-products idiom (oracle.TorchPolyN) — `cpu_baseline.kind` = "reference"; without baseline/_ref the oracle port
+cat-of-products idiom (oracle.TorchPolyN) — `cpu_baseline.kind` = "reference"; without oracle/_ref the oracle port
 is timed instead ("port"). `extra.reference_unmodified` holds the rows the reference can run with NO extension: its
 degree-3 (K = 20) closure at 1e6 and 4e6 samples, `solve_SINDy_one_step`, `solve_ode_batch`, `WSINDyWrapper.solve`.
 """
@@ -43,7 +47,7 @@ PKG = os.path.join(ROOT, "symmetry-ode-discovery_b200")
 if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
 # PKG (this repo's `sindy`, `train`, ...) is put on sys.path by the B200 arm only: the reference arm imports the
-# reference's modules of the same names from baseline/_ref
+# reference's modules of the same names from oracle/_ref
 
 import torch  # noqa: E402
 
@@ -135,7 +139,7 @@ class ClockSampler:
 
 
 def reference_dir():
-    for c in (os.environ.get("SINDY_B200_REFERENCE"), os.path.join(ROOT, "baseline", "_ref")):
+    for c in (os.environ.get("SINDY_B200_REFERENCE"), os.path.join(ROOT, "oracle", "_ref")):
         if c and os.path.isfile(os.path.join(c, "sindy.py")) and os.path.isfile(os.path.join(c, "train.py")):
             return os.path.abspath(c)
     return None
@@ -173,12 +177,12 @@ def run_reference(args, rank):
         torch.manual_seed(0)
         reg.Xi = torch.nn.Parameter(torch.randn(D, K))
         reg.mask = torch.ones(D, K)
-        how = ("reference's SINDyRegression.forward from baseline/_ref (terms extended to degree 5), MSELoss, jvp-based "
+        how = ("reference's SINDyRegression.forward from oracle/_ref (terms extended to degree 5), MSELoss, jvp-based "
                "Lie-derivative regulariser (train.py:503-507, intended [1]), L1, backward, torch.optim.Adam.step()")
     else:
         torch.manual_seed(0)
         reg = O.TorchRegressor(D, P)
-        how = "oracle port of the same step (no baseline/_ref on this box)"
+        how = "oracle port of the same step (no reference checkout in oracle/_ref)"
     gens = so3_basis() if not args.no_symreg else []
     mse = torch.nn.MSELoss()
     opt = torch.optim.Adam(reg.parameters(), lr=1e-3)
@@ -243,7 +247,7 @@ def run_reference(args, rank):
 
 
 def reference_extras(ref, step5, make_data):
-    """Side rows on the host cores. With baseline/_ref: the UNMODIFIED reference (no extension) — its degree-3 closure
+    """Side rows on the host cores. With oracle/_ref: the UNMODIFIED reference (no extension) — its degree-3 closure
     (`train.py:645-690`) at 1e6 and 4e6 samples, `solve_SINDy_one_step` (`sindy.py:250-315`), `solve_ode_batch`
     (`data_utils/ode.py:7-28`), `WSINDyWrapper.solve` (`sindy.py:352-395`). Always: the degree-5 step without sym-reg."""
     import numpy as np
@@ -315,7 +319,14 @@ def main():
     ap.add_argument("--no-peer", action="store_true", help="multi-GPU: NCCL all-reduce instead of the in-kernel peer all-reduce")
     ap.add_argument("--skip-extras", action="store_true")
     ap.add_argument("--no-symreg", action="store_true", help="step without the so(3) Lie-derivative regulariser")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step returned (loss, gradient, updated coefficients, Adam moments) "
+                         "as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of the B200 path; it does not apply to --impl reference")
 
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -388,6 +399,10 @@ def main():
 
         def one_step(record=False):
             return stepper.step()
+
+        def last_outputs(loss):
+            return {"loss": loss, "grad": stepper.grad, "xi": stepper.xi,
+                    "adam_moments": stepper.state[:2 * D * K].view(2, D, K)}
     else:
         use_graph = (world > 1) and not args.no_graph
         stepper = ShardedTrainStep(lib, x, dx, flags=flags, use_graph=use_graph, sgd_lr=1e-3, use_peer=not args.no_peer)
@@ -396,8 +411,10 @@ def main():
         stepper.step(Xi0, mask, w_l1)  # loads the static parameters (and captures the graph when enabled)
         stepper.xi.copy_(Xi0)
         launches_per_step = 2 if (world == 1 or stepper.peer is not None) else 3
+        last_grad = None
 
         def one_step(record=False):
+            nonlocal last_grad
             if record and not use_graph:
                 e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
                 e0.record()
@@ -412,9 +429,13 @@ def main():
                     native.step_epilogue(packed, stepper.xi, stepper.mask, lib, w_l1, loss=loss_t, grad=grad_t)
                 kern_events.append((e0, e1))
                 stepper.xi.add_(grad_t, alpha=-1e-3)
+                last_grad = grad_t
                 return loss_t
-            loss_t, _ = stepper.step(None, None, w_l1)
+            loss_t, last_grad = stepper.step(None, None, w_l1)
             return loss_t
+
+        def last_outputs(loss):
+            return {"loss": loss, "grad": last_grad, "xi": stepper.xi}
 
     def barrier():
         if world > 1:
@@ -463,6 +484,10 @@ def main():
     elapsed_ms = float(elapsed_ms)
     value = n_total * args.steps / (elapsed_ms * 1e-3)
     final_loss = float(loss)
+    if args.dump_outputs and rank == 0:   # before the checks below reload the stepper
+        if not legacy:
+            stepper.check()   # a peer lost in the exchange leaves the outputs stale: fail before writing them
+        dump_outputs(args.dump_outputs, last_outputs(loss))
 
     # ---- N > 1: the sharded step against an UNSHARDED recompute on rank 0 (all shards gathered on one GPU) ----
     sharded_check = None
@@ -656,6 +681,15 @@ def main():
     if world > 1:
         torch.cuda.synchronize()
         os._exit(0)
+
+
+def dump_outputs(out_dir, tensors):
+    """`--dump-outputs`: each tensor as out_dir/<name>.npy in its own dtype (float32 here; a few KB in all). The inputs
+    are seeded, so two builds run with the same arguments can be compared output for output."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in tensors.items():
+        np.save(os.path.join(out_dir, name + ".npy"), t.detach().cpu().numpy())
 
 
 def cpu_baseline_child(args):

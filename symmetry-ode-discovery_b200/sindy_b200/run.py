@@ -15,7 +15,7 @@ this repo's module directory has been put first and the reference's directory se
     `evaluation` — the parts of the reference outside the hot path (`main.py:9-15`, `dataset.py:12`).
 
 Options (before the script): `--reference DIR` (default: the script's directory, else $SINDY_B200_REFERENCE, else
-<repo>/baseline/_ref), `--reference-train` (keep the reference's own `train.py`: its loops then run operator by operator
+<repo>/oracle/_ref), `--reference-train` (keep the reference's own `train.py`: its loops then run operator by operator
 on this repo's `sindy` / `model_utils` through autograd), `--where` (print where the hot-path modules resolve, and exit),
 `--seeds A-B[,C...]` (run the script once per seed IN THIS PROCESS with `--seed k` appended: what `run_scripts/*.sh` does
 with one interpreter start — ≈8 s of imports and CUDA start-up — per seed; any cfg, the runs stay independent and write
@@ -43,9 +43,9 @@ def _looks_like_reference(path):
 
 def find_reference(explicit=None, script=None):
     """Directory of the reference checkout: --reference, the script's own directory, $SINDY_B200_REFERENCE,
-    <repo>/baseline/_ref, an entry of sys.path — in that order."""
+    <repo>/oracle/_ref, an entry of sys.path — in that order."""
     cands = [explicit, os.path.dirname(os.path.abspath(script)) if script else None,
-             os.environ.get("SINDY_B200_REFERENCE"), os.path.join(REPO_DIR, "baseline", "_ref")]
+             os.environ.get("SINDY_B200_REFERENCE"), os.path.join(REPO_DIR, "oracle", "_ref")]
     cands += [p for p in sys.path if p and os.path.abspath(p) != PKG_DIR]
     for c in cands:
         if _looks_like_reference(c):

@@ -45,7 +45,7 @@ CONFIGS = {
 
 
 def find_reference():
-    for c in (os.environ.get("SINDY_B200_REFERENCE"), os.path.join(ROOT, "baseline", "_ref"), "/root/reference"):
+    for c in (os.environ.get("SINDY_B200_REFERENCE"), os.path.join(ROOT, "oracle", "_ref")):
         if c and os.path.isfile(os.path.join(c, "main.py")) and os.path.isfile(os.path.join(c, "sindy.py")):
             return os.path.abspath(c)
     return None

@@ -6,7 +6,8 @@ modules are outside the hot path. These minimal modules expose exactly the attri
 (`encode`, `decode`, `decoder`, `encoder[-2].bias`, `get_full_basis_list`, `get_deterministic_group_elems`,
 `Li`) with the same tensor shapes: x (B, n_comps, input_dim) <-> z (B, n_comps, latent_dim), generators
 (n_comps·latent_dim)². Used identically by the golden generator (with the reference's regularisers) and by the
-GPU parity tests (with ours).
+GPU parity tests (with ours). `make_reference_tree` lays out an empty stand-in of the reference checkout for the
+launcher's import-resolution tests.
 """
 import torch
 import torch.nn as nn
@@ -65,6 +66,27 @@ class StandInGenerator(nn.Module):
 
     def get_deterministic_group_elems(self, split_channel=False, scale=1.0):
         return [torch.matrix_exp(s * L * scale) for s, L in zip(self.sigma, self.Li)]
+
+
+STANDIN_REFERENCE_MODULES = ("sindy.py", "model_utils.py", "gan.py", "autoencoder.py", "dataset.py", "parser_utils.py",
+                             "evaluation/__init__.py", "evaluation/eval_eq.py", "data_utils/__init__.py",
+                             "data_utils/ode.py", "data_utils/smoothing.py", "data_utils/damped_oscillator.py",
+                             "data_utils/growth.py", "data_utils/lotka.py", "data_utils/selkov.py")
+
+
+def make_reference_tree(path):
+    """A directory laid out like the reference checkout (the module names the launcher and the drop-in modules resolve,
+    `train.py` with a `train_lassi`), each module empty: enough to test where imports resolve without the reference's
+    code. Returns the directory."""
+    import os
+    for rel in STANDIN_REFERENCE_MODULES:
+        f = os.path.join(path, rel)
+        os.makedirs(os.path.dirname(f), exist_ok=True)
+        with open(f, "w") as fh:
+            fh.write('"""Stand-in for the reference module of the same name."""\n')
+    with open(os.path.join(path, "train.py"), "w") as fh:
+        fh.write('"""Stand-in for the reference\'s train.py."""\n\n\ndef train_lassi(*args, **kwargs):\n    pass\n')
+    return path
 
 
 def make_standins(seed=0, input_dim=2, n_comps=2, hidden=32, latent_dim=None, state_dict=None, device="cpu"):

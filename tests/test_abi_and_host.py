@@ -153,11 +153,18 @@ def test_constraint_basis_matches_reference(golden):
         reg = sindy.SINDyRegression(2, 2, False, False, L_list=[L], threshold=0.05, device="cpu", constrain_constant=True)
         np.testing.assert_allclose(reg.get_M_list()[0].numpy(), g[name + "_M"], atol=1e-6)
         assert int(reg.use_kron_product) == int(g[name + "_kron"])
-        # same SVD routine on the same matrix: identical basis, hence identical Ξ from the same RNG draws
-        np.testing.assert_allclose(reg.Q.numpy(), g[name + "_Q"], atol=1e-6)
-        np.testing.assert_allclose(reg.beta.detach().numpy(), g[name + "_beta0"], atol=0)
+        # same SVD routine on the same matrix: the same basis up to the sign of each vector, which the LAPACK library
+        # chooses differently on different CPUs (MKL on an AMD EPYC host negates so(2)'s first vector against the
+        # golden, taken on an Intel host); the same RNG draws on the sign-aligned basis give the same Ξ
+        Q, Qr, beta0 = reg.Q.numpy(), g[name + "_Q"], g[name + "_beta0"]
+        sign = np.sign((Q * Qr).sum(axis=0))
+        np.testing.assert_allclose(Q, Qr * sign, atol=1e-6)
+        np.testing.assert_allclose(reg.beta.detach().numpy(), beta0, atol=0)
         np.testing.assert_allclose(reg.const.detach().numpy(), g[name + "_const0"], atol=0)
-        np.testing.assert_allclose(reg.get_Xi().detach().numpy(), g[name + "_Xi0"], atol=1e-6)
+        # Ξ = Q·β in the equation-major layout of the invertible-generator (Kronecker) form, no constant column
+        assert reg.use_kron_product and not reg.allow_constant
+        np.testing.assert_allclose((Qr @ beta0).reshape(2, -1), g[name + "_Xi0"], atol=1e-6)
+        np.testing.assert_allclose(reg.get_Xi().detach().numpy(), ((Qr * sign) @ beta0).reshape(2, -1), atol=1e-6)
     L3 = torch.tensor([[0.0, 1.0, 0.0], [-1.0, 0.0, 0.0], [0.0, 0.0, 0.0]])
     reg = sindy.SINDyRegression(3, 2, False, False, L_list=[L3], threshold=0.05, device="cpu", constrain_constant=True)
     assert int(reg.use_kron_product) == int(g["sing3_kron"]) == 0
@@ -343,17 +350,17 @@ def test_python_right_hand_sides_are_identified_as_library_members():
         ode.identify_library_ode(lambda x: np.tanh(x), rng.uniform(-1, 1, (8, 2)))
 
 
-def test_launcher_puts_the_hot_path_modules_first():
+def test_launcher_puts_the_hot_path_modules_first(tmp_path):
     """`python <reference>/main.py` with PYTHONPATH resolves `sindy` to the reference (the script's directory comes
-    first); the launcher must resolve the hot-path modules to this repo and everything else to the reference."""
+    first); the launcher must resolve the hot-path modules to this repo and everything else to the reference (a
+    stand-in tree with the reference's module names)."""
     import subprocess
     import sys
     import config_runs
-    ref = config_runs.find_reference()
-    if ref is None:
-        pytest.skip("no reference checkout")
+    import standins
+    ref = standins.make_reference_tree(str(tmp_path / "reference"))
     res = subprocess.run([sys.executable, config_runs.LAUNCHER, "--reference", ref, "--where"], capture_output=True,
-                         text=True, timeout=600, cwd="/tmp")
+                         text=True, timeout=600, cwd=str(tmp_path))
     assert res.returncode == 0, res.stderr[-2000:]
     table = dict(line.split(None, 1) for line in res.stdout.strip().splitlines())
     pkg = config_runs.PKG
@@ -365,7 +372,7 @@ def test_launcher_puts_the_hot_path_modules_first():
     # train_lassi (outside the hot path) is re-exported from the reference so that `main.py:90-91` keeps resolving
     res = subprocess.run([sys.executable, "-c", "import sys; sys.path[:0] = [%r, %r]; import train; "
                           "print(train.train_lassi.__module__, 'train_lassi' in train.__all__)" % (pkg, ref)],
-                         capture_output=True, text=True, timeout=600, cwd="/tmp")
+                         capture_output=True, text=True, timeout=600, cwd=str(tmp_path))
     assert res.returncode == 0 and res.stdout.split() == ["_sindy_b200_reference_train", "True"], res.stdout + res.stderr
 
 
@@ -620,10 +627,8 @@ def test_launcher_seed_loop_runs_the_script_once_per_seed_in_one_process(tmp_pat
     (the replacement for run_scripts/*.sh's 50 interpreter starts)."""
     import subprocess
     import sys
-    import config_runs
-    ref = config_runs.find_reference()
-    if ref is None:
-        pytest.skip("no reference checkout")
+    import standins
+    ref = standins.make_reference_tree(str(tmp_path / "reference"))
     script = tmp_path / "probe.py"
     script.write_text("import os, sys\nprint('RUN', os.getpid(), sys.argv[1:])\n")
     launcher = os.path.join(ROOT, "symmetry-ode-discovery_b200", "sindy_b200", "run.py")

@@ -3,8 +3,8 @@ the drop-in launcher (`sindy_b200/run.py`) on the B200, against goldens of the s
 alone on the CPU (`oracle/gen_config_golden.py` -> tests/golden/configs.npz; data sets tests/golden/data).
 
 Needs a reference checkout for the parts of the reference OUTSIDE the hot path (argument parser, dataset loader,
-autoencoder / generator classes, evaluation): `baseline/_ref` (copied by `__graft_entry__.build()`, git-ignored, travels
-with gpurun) or $SINDY_B200_REFERENCE. Bar (north_star): identical sparsity pattern, coefficients within 1e-4 relative
+autoencoder / generator classes, evaluation): `oracle/_ref` (mirrored by `__graft_entry__.build()`, git-ignored) or
+$SINDY_B200_REFERENCE. Bar (north_star): identical sparsity pattern, coefficients within 1e-4 relative
 (of the largest coefficient) — stated per test where a config needs more room, with the reason.
 
 SINDY_B200_INIT_RNG=cpu makes `SINDyRegression` draw its initial parameters from the CPU generator like the reference's
@@ -21,7 +21,7 @@ import config_runs
 pytestmark = pytest.mark.gpu
 
 REF = config_runs.find_reference()
-needs_ref = pytest.mark.skipif(REF is None, reason="no reference checkout (baseline/_ref) for main.py / dataset.py")
+needs_ref = pytest.mark.skipif(REF is None, reason="no reference checkout (oracle/_ref) for main.py / dataset.py")
 ENV = {"SINDY_B200_INIT_RNG": "cpu"}
 
 
@@ -114,7 +114,7 @@ def test_config4_wsindy_selkov_through_the_dropin(golden, tmp_path):
 @pytest.mark.parametrize("key,tol", [("C1", 2e-4), ("C2", 2e-4), ("C1w", 2e-4)])
 def test_live_against_the_reference_on_the_same_gpu(key, tol, tmp_path):
     """The strongest drop-in statement available: the reference's entry point run TWICE on this B200, same seed —
-    once alone (`python baseline/_ref/main.py --gpu 0`: PyTorch-eager CUDA, initial Ξ from the CUDA generator) and once
+    once alone (`python oracle/_ref/main.py --gpu 0`: PyTorch-eager CUDA, initial Ξ from the CUDA generator) and once
     through the launcher (this repo's sindy / model_utils / train / data_utils, same draws from the same generator).
     Same mask, coefficients within 2e-4 of the largest (LBFGS stops at a parameter update of 1e-3, `train.py:643`)."""
     a, _ = config_runs.run_entry(key, str(tmp_path / "ref"), REF, dropin=False, gpu=0)

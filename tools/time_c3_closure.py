@@ -2,7 +2,7 @@
 512x5 autoencoder of the reference's own class, B = 20 000) on the GPU and prints where the time goes. Run through the
 launcher so that the reference's parser / autoencoder / gan import next to this repo's modules:
 
-    python symmetry-ode-discovery_b200/sindy_b200/run.py --reference baseline/_ref tools/time_c3_closure.py [B]
+    python symmetry-ode-discovery_b200/sindy_b200/run.py --reference oracle/_ref tools/time_c3_closure.py [B]
 """
 import os
 import sys

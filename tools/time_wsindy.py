@@ -1,5 +1,6 @@
-import sys, torch
-sys.path[:0]=['/root/repo','/root/repo/symmetry-ode-discovery_b200']
+import os, sys, torch
+ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+sys.path[:0] = [ROOT, os.path.join(ROOT, "symmetry-ode-discovery_b200")]
 from sindy_b200 import native
 dev=torch.device('cuda')
 for (d,p,ntr) in ((2,3,8192),(2,3,18944),(3,5,2048),(3,5,4736),(2,2,18944),(3,3,9472)):
