@@ -265,6 +265,20 @@ int sb_rollout(const void* x0, int64_t n_ics, const sb_library* lib, const void*
 int sb_wsindy_integrals(const float* x, int64_t n_traj, int64_t T, const sb_library* lib, float dt,
                         double t_max, int n_test, double* G, double* b, void* stream);
 
+/* WSINDy weak-form integrals with compactly supported test functions (Messenger & Bortz, Weak SINDy for ODEs, 2021):
+ * every test function is the same window of `support` = L samples at its own start
+ *   s_j = ⌊j·(T−L)/(n_test−1)⌋ (s_0 = 0 when n_test = 1),
+ *   G[traj,j,k] = sum_q phi[q]·Θ_k(x[traj, s_j+q]),   b[traj,j,i] = −sum_q dphi[q]·x[traj, s_j+q, i],  q = 0..L−1.
+ * phi, dphi: device arrays of L floats, the rows' values on their support with dt folded in (for the piecewise
+ * polynomial family of WSINDyWrapper(test_func_family='poly'): phi[q] = fp32(dt·c·φ_q), dphi[q] = fp32(dt·c·φ'_q),
+ * φ_q = (4u(1−u))^p, u = q/(L−1), c = 1/sqrt(dt·Σφ²)). x is (n_traj × T × d); G (n_traj×n_test×K) and b
+ * (n_traj×n_test×d) are fp64. Sums run in fp32 over blocks of at most 2048 consecutive support samples, then in fp64;
+ * no atomics: G[traj] and b[traj] have the same bits alone, in any batch and on every repeat.
+ * SB_ERR_INVALID unless 3 ≤ L ≤ T and 1 ≤ n_test ≤ T − L + 1, or for a NULL pointer (n_traj = 0 is a no-op);
+ * SB_ERR_UNSUPPORTED for a library sb_library_size rejects. */
+int sb_wsindy_local_integrals(const float* x, int64_t n_traj, int64_t T, const sb_library* lib, const float* phi,
+                              const float* dphi, int support, int n_test, double* G, double* b, void* stream);
+
 /* Frozen-MLP chains on the tensor cores (SURVEY §8f-3): the encoder / decoder of the frozen autoencoder
  * (`autoencoder.py:38-66`: Linear [+ BatchNorm in eval mode, folded into the weights by the host] + ReLU, hidden width a
  * multiple of 256, thin first / last layers of width ≤ 8) as evaluated inside `symmreg_i` / `symmreg_f` /

@@ -400,6 +400,23 @@ int sb_wsindy_integrals(const float* x, int64_t n_traj, int64_t T, const sb_libr
   return wsindy_integrals(x, n_traj, T, t, dt, t_max, n_test, G, b, (cudaStream_t)stream);
 }
 
+int sb_wsindy_local_integrals(const float* x, int64_t n_traj, int64_t T, const sb_library* lib, const float* phi,
+                              const float* dphi, int support, int n_test, double* G, double* b, void* stream) {
+  LibTab t;
+  SB_TRY(build_table(lib, &t));
+  // 3 <= L <= T, 1 <= n_test <= T - L + 1 (distinct starts), and j·(T − L) must fit in int64 for every start
+  if (n_traj < 0 || support < 3 || T < support || n_test < 1 || n_test > T - support + 1 ||
+      (n_test > 1 && T - support > INT64_MAX / (n_test - 1))) {
+    set_error("bad wsindy_local sizes n_traj=%lld T=%lld support=%d n_test=%d", (long long)n_traj, (long long)T,
+              support, n_test);
+    return SB_ERR_INVALID;
+  }
+  if (n_traj == 0) return SB_OK;
+  SB_TRY(check_ptr(x, "x")); SB_TRY(check_ptr(phi, "phi")); SB_TRY(check_ptr(dphi, "dphi"));
+  SB_TRY(check_ptr(G, "G")); SB_TRY(check_ptr(b, "b"));
+  return wsindy_local_integrals(x, n_traj, T, t, phi, dphi, support, n_test, G, b, (cudaStream_t)stream);
+}
+
 int sb_symreg_supported(const sb_library* lib) {
   LibTab t;
   if (build_table(lib, &t) != SB_OK) return 0;

@@ -293,6 +293,9 @@ int rollout(const void* x0, int64_t n_ics, const LibTab& t, const void* w, doubl
 // WSINDy integrals
 int wsindy_integrals(const float* x, int64_t n_traj, int64_t T, const LibTab& t, float dt, double t_max,
                      int n_test, double* G, double* b, cudaStream_t s);
+// WSINDy integrals with compactly supported test functions (sb_wsindy_local.cu); sizes validated by the caller
+int wsindy_local_integrals(const float* x, int64_t n_traj, int64_t T, const LibTab& t, const float* phi,
+                           const float* dphi, int L, int n_test, double* G, double* b, cudaStream_t s);
 
 // fused symmetry-regulariser kernels (sb_symreg.cu): Euler flow map with JVP and its reverse sweep, reversed regulariser
 bool symreg_supported(const LibTab& t);

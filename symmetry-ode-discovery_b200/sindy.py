@@ -512,22 +512,82 @@ def solve_SINDy(regressor, x, y, w_sindy_reg, st_threshold, max_iter=5, **kwargs
     return residual
 
 
+def _local_test_functions(T, dt, n_test, support=None, degree=None):
+    """The compactly supported piecewise-polynomial family of WSINDyWrapper(test_func_family='poly') (Messenger &
+    Bortz, Weak SINDy for ODEs, 2021): every row is the same window of L samples at its own start
+      φ_q = (4u(1−u))^p,  φ'_q = p·(4u(1−u))^(p−1)·4(1−2u)/((L−1)·dt),  u = q/(L−1),  q = 0..L−1,
+      phi = fp32(dt·c·φ),  dphi = fp32(dt·c·φ'),  c = 1/sqrt(dt·Σφ²)   (Σ_t V[j,t]² = dt, the scale of the trig rows),
+      s_j = ⌊j·(T−L)/(n_test−1)⌋  (s_0 = 0 when n_test = 1).
+    Defaults: L = min(T, 2·⌊T/(n_test+1)⌋ + 1) (about two-fold overlap), p = 6. Returns (L, p, starts, phi, dphi) with
+    numpy fp32 tables; raises ValueError unless 3 ≤ L ≤ T, 1 ≤ p ≤ 32 and 1 ≤ n_test ≤ T − L + 1."""
+    def integer(v, name):
+        if isinstance(v, bool) or not isinstance(v, (int, np.integer)):
+            raise ValueError(f"{name} must be an integer, got {v!r}")
+        return int(v)
+    T, n_test = integer(T, "the number of time samples"), integer(n_test, "num_test_funcs")
+    if n_test < 1:
+        raise ValueError(f"num_test_funcs must be at least 1, got {n_test}")
+    L = min(T, 2 * (T // (n_test + 1)) + 1) if support is None else integer(support, "test_func_support")
+    p = 6 if degree is None else integer(degree, "test_func_degree")
+    if not 3 <= L <= T:
+        raise ValueError(f"test_func_support must lie in [3, T = {T}], got {L}")
+    if not 1 <= p <= 32:
+        raise ValueError(f"test_func_degree must lie in [1, 32], got {p}")
+    if n_test > T - L + 1:
+        raise ValueError(f"num_test_funcs = {n_test} exceeds T − L + 1 = {T - L + 1}: the windows would not have "
+                         f"distinct starts")
+    if not (math.isfinite(dt) and dt > 0):
+        raise ValueError(f"the time step must be positive, got {dt}")
+    u = np.arange(L, dtype=np.float64) / (L - 1)
+    s = 4.0 * u * (1.0 - u)
+    phi = s ** p
+    dphi = p * s ** (p - 1) * 4.0 * (1.0 - 2.0 * u) / ((L - 1) * dt)
+    c = 1.0 / math.sqrt(dt * float(np.sum(phi * phi)))
+    starts = [0] if n_test == 1 else [j * (T - L) // (n_test - 1) for j in range(n_test)]
+    return L, p, starts, (dt * c * phi).astype(np.float32), (dt * c * dphi).astype(np.float32)
+
+
 class WSINDyWrapper():
     """Weak SINDy as a regularised least-squares problem (reference `sindy.py:327-395`).
 
-    Test functions g_k(t) = sqrt(2/T)·sin(kπt/T), k = 1..num_test_funcs. `t` must be the uniform grid
-    t_i = i·dt starting at 0 that `main_wsindy.py:41` builds.
+    test_func_family='trig' (the reference's): g_k(t) = sqrt(2/T)·sin(kπt/T), k = 1..num_test_funcs, each spanning the
+    whole window. test_func_family='poly': compactly supported piecewise polynomials (`_local_test_functions`) of
+    test_func_support samples (default about 2·T/num_test_funcs) and degree test_func_degree (default 6); a sample then
+    costs only the few windows that cover it, so hundreds or thousands of test functions can be placed along a long
+    trajectory. `t` must be the uniform grid t_i = i·dt starting at 0 that `main_wsindy.py:41` builds.
     """
 
-    def __init__(self, regressor, t, t_max, num_test_funcs=50, test_func_family='trig', device='cuda', **kwargs):
-        if test_func_family != 'trig':
+    def __init__(self, regressor, t, t_max, num_test_funcs=50, test_func_family='trig', device='cuda',
+                 test_func_support=None, test_func_degree=None, **kwargs):
+        if test_func_family not in ('trig', 'poly'):
             raise NotImplementedError(f'test_func_family={test_func_family} not implemented')
+        if test_func_family == 'trig' and (test_func_support is not None or test_func_degree is not None):
+            raise ValueError("test_func_support / test_func_degree apply to test_func_family='poly' only")
+        if test_func_family == 'poly':
+            layout = _local_test_functions(int(t.shape[0]), float(t[1] - t[0]), num_test_funcs, test_func_support,
+                                           test_func_degree)
+        self.test_func_family = test_func_family
         self.t = t.to(device)
         self.dt = self.t[1] - self.t[0]
         self.t_max = float(t_max)
         self.num_test_funcs = int(num_test_funcs)
         self.regressor = regressor
         self.kwargs = {'lstsq_driver': kwargs.get('lstsq_driver')}
+        if test_func_family == 'poly':
+            L, p, starts, phi, dphi = layout
+            self.test_func_support, self.test_func_degree = L, p
+            self.phi = torch.from_numpy(phi).to(device)
+            self.dphi = torch.from_numpy(dphi).to(device)
+            # dense V, V' (n_test × T) for attribute parity with the trig family and for M = V·Vᵀ; the kernel reads
+            # only the L-sample tables
+            T = self.t.shape[0]
+            cols = (torch.tensor(starts, dtype=torch.int64).view(-1, 1) + torch.arange(L).view(1, -1)).to(device)
+            self.V = torch.zeros(self.num_test_funcs, T, dtype=torch.float32, device=device)
+            self.V_drv = torch.zeros_like(self.V)
+            self.V.scatter_(1, cols, self.phi.expand(self.num_test_funcs, L).contiguous())
+            self.V_drv.scatter_(1, cols, self.dphi.expand(self.num_test_funcs, L).contiguous())
+            self.M = self.V.double() @ self.V.double().T
+            return
         # dense V only to form the n_test×n_test weight M = V·Vᵀ once (the reference multiplies by Vᵀ on the
         # left of both sides, `sindy.py:369-370`); the data-dependent integrals never read V.
         k = torch.arange(1, num_test_funcs + 1, dtype=torch.float32, device=device).view(-1, 1)
@@ -538,27 +598,40 @@ class WSINDyWrapper():
         self.M = self.V.double() @ self.V.double().T
 
     def integrals(self, x):
-        """G = V·Θ(x) (n_test×K) and b = −V'·x (n_test×d), fp64, from the fused kernel."""
+        """G = V·Θ(x) (n_test×K) and b = −V'·x (n_test×d), fp64, from the fused kernel; x of shape (T, d), or
+        (n_traj, T, d) for per-trajectory (n_traj×n_test×K, n_traj×n_test×d)."""
+        if self.test_func_family == 'poly':
+            return native.wsindy_local_integrals(x, self.regressor.library, self.phi, self.dphi, self.num_test_funcs)
         return native.wsindy_integrals(x, self.regressor.library, float(self.dt), self.t_max, self.num_test_funcs)
 
     def solve(self, x, w_sindy_reg, st_threshold, **kwargs):
         '''
         x: (seq_len, dim) on the wrapper's uniform grid. Solves [VᵀG; sqrt(w)·I] ξ = [Vᵀb; 0] on the current
         support through its normal equations (GᵀMG + w·I) ξ = GᵀM b, then thresholds.
+        x: (n_traj, seq_len, dim): one equation from all trajectories, pooled through the summed normal equations
+        (Σ_r G_rᵀMG_r + w·I) ξ = Σ_r G_rᵀMb_r.
         Returns (mean squared residual of that system, converged).
         '''
         with torch.no_grad():
-            if x.shape[0] != self.t.shape[0]:
-                raise ValueError(f'x has {x.shape[0]} time samples, the wrapper was built for {self.t.shape[0]}')
+            if x.shape[-2] != self.t.shape[0] or x.dim() not in (2, 3):
+                raise ValueError(f'x has {x.shape[-2]} time samples, the wrapper was built for {self.t.shape[0]}')
             Gw, bw = self.integrals(x)
-            MG = self.M @ Gw
-            A = Gw.T @ MG                                        # K×K
-            rhs = MG.T @ bw                                      # K×d
+            if x.dim() == 2:
+                MG = self.M @ Gw
+                A = Gw.T @ MG                                    # K×K
+                rhs = MG.T @ bw                                  # K×d
+                bb = torch.einsum('ji,jl,li->i', bw, self.M, bw)
+                n_rows = x.shape[0]
+            else:
+                MG = self.M @ Gw                                 # n_traj × n_test × K
+                A = (Gw.transpose(1, 2) @ MG).sum(0)
+                rhs = (MG.transpose(1, 2) @ bw).sum(0)
+                bb = torch.einsum('rji,jl,rli->i', bw, self.M, bw)
+                n_rows = x.shape[0] * x.shape[1]
             K = A.shape[0]
-            converged = _stlsq_update(self.regressor, A, rhs, float(w_sindy_reg), x.shape[0] + K, st_threshold,
+            converged = _stlsq_update(self.regressor, A, rhs, float(w_sindy_reg), n_rows + K, st_threshold,
                                       _lstsq_driver(kwargs if kwargs.get('lstsq_driver') else self.kwargs))
             Xi = self.regressor._current_Xi().to(torch.float64)
-            bb = torch.einsum('ji,jl,li->i', bw, self.M, bw)
             quad = torch.einsum('ik,kl,il->i', Xi, A, Xi) - 2.0 * torch.einsum('ik,ki->i', Xi, rhs) + bb
             quad = quad + float(w_sindy_reg) * (Xi ** 2).sum(1)
         return quad.mean().item(), converged

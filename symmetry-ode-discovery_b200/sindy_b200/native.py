@@ -72,6 +72,8 @@ _SIGNATURES = {
                            c_int, c_int, c_void_p, c_void_p, c_void_p, c_void_p]),
     "sb_wsindy_integrals": (c_int, [c_void_p, c_int64, c_int64, POINTER(_CLibrary), c_float, c_double, c_int,
                                     c_void_p, c_void_p, c_void_p]),
+    "sb_wsindy_local_integrals": (c_int, [c_void_p, c_int64, c_int64, POINTER(_CLibrary), c_void_p, c_void_p, c_int,
+                                          c_int, c_void_p, c_void_p, c_void_p]),
     "sb_symreg_supported": (c_int, [POINTER(_CLibrary)]),
     "sb_euler_flow": (c_int, [c_void_p, c_void_p, c_int64, POINTER(_CLibrary), c_void_p, c_float, c_int, c_void_p,
                               c_void_p, c_void_p]),
@@ -545,6 +547,33 @@ def wsindy_integrals(x: torch.Tensor, lib: Library, dt: float, t_max: float, n_t
         _check(load().sb_wsindy_integrals(xf.data_ptr(), n_traj, T, ctypes.byref(lib.c()), float(dt), float(t_max),
                                           int(n_test), G.data_ptr(), b.data_ptr(), _stream(dev)),
                "sb_wsindy_integrals")
+    return (G[0], b[0]) if single else (G, b)
+
+
+def wsindy_local_integrals(x: torch.Tensor, lib: Library, phi: torch.Tensor, dphi: torch.Tensor, n_test: int):
+    """G (n_traj×n_test×K) and b (n_traj×n_test×d), fp64, for x of shape (n_traj, T, d) or (T, d), with the compactly
+    supported test functions whose values on their support are phi, dphi (1-D, `support` = len(phi) floats on x's
+    device; starts s_j = ⌊j·(T−L)/(n_test−1)⌋). See sb_wsindy_local_integrals in include/sindy_b200.h."""
+    xf = _f32c(x, "x")
+    ph = _f32c(phi, "phi").reshape(-1)
+    dph = _f32c(dphi, "dphi").reshape(-1)
+    if ph.numel() != dph.numel():
+        raise ValueError(f"phi has {ph.numel()} values, dphi {dph.numel()}")
+    if ph.device != xf.device or dph.device != xf.device:
+        raise ValueError("phi and dphi must be on the device of x")
+    single = xf.dim() == 2
+    if single:
+        xf = xf.unsqueeze(0)
+    n_traj, T, d = xf.shape
+    if d != lib.dim:
+        raise ValueError(f"x has last dimension {d}, library expects {lib.dim}")
+    dev = xf.device
+    G = torch.empty(n_traj, n_test, lib.K, dtype=torch.float64, device=dev)
+    b = torch.empty(n_traj, n_test, d, dtype=torch.float64, device=dev)
+    with torch.cuda.device(dev):
+        _check(load().sb_wsindy_local_integrals(xf.data_ptr(), n_traj, T, ctypes.byref(lib.c()), ph.data_ptr(),
+                                                dph.data_ptr(), ph.numel(), int(n_test), G.data_ptr(), b.data_ptr(),
+                                                _stream(dev)), "sb_wsindy_local_integrals")
     return (G[0], b[0]) if single else (G, b)
 
 
