@@ -257,6 +257,22 @@ int sb_rollout(const void* x0, int64_t n_ics, const sb_library* lib, const void*
                int64_t n_steps, int64_t stride, int method, int dtype, int record_dx,
                void* x_out, void* dx_out, void* x_last, void* stream);
 
+/* Fused rollout and scoring of many models (model selection along a threshold path, Mangan et al. 2017): for every
+ * (model m, initial condition n) integrate dx/dt = Θ(x)·W_mᵀ from x0[n] (fp32, SB_EULER / SB_RK4, the operation order of
+ * sb_rollout's odeint mode) and, after every `steps_per_row` steps r = 1..n_rows, add
+ * Σ_j ((double)x_j − (double)y_obs[r−1, n, j])² (the row sum formed in j order) to sse[m, n] in row order (fp64). A pair
+ * stops at the first row whose state has a non-finite component or |x_j| > blowup (blowup ≤ 0: no bound);
+ * valid_rows[m, n] = rows compared before that (n_rows if none), sse holds those rows only. The compared states are
+ * bit-identical to the rows sb_rollout(x0, W_m, dt, n_rows·steps_per_row, stride = steps_per_row) stores.
+ * w: n_models × d × K fp32 (already masked). y_obs: n_rows × n_ics × d (the x_out layout of sb_rollout, x0 excluded).
+ * sse, valid_rows: n_models × n_ics. One thread owns a pair: no atomics; a pair's outputs have the same bits alone, in
+ * any batch, in any model order and on every repeat. SB_ERR_INVALID for a NULL pointer, n_ics < 0, n_models < 1,
+ * steps_per_row < 1, n_rows outside 1..INT32_MAX, an unknown method or dt not > 0 (n_ics = 0 is a no-op);
+ * SB_ERR_UNSUPPORTED for a library sb_library_size rejects. */
+int sb_rollout_score(const float* x0, int64_t n_ics, const sb_library* lib, const float* w, int n_models, double dt,
+                     int64_t steps_per_row, int64_t n_rows, int method, const float* y_obs, float blowup,
+                     double* sse, int32_t* valid_rows, void* stream);
+
 /* WSINDy weak-form integrals with trigonometric test functions (`sindy.py:332-347,361-362`):
  *   V[j,t]  = dt·sqrt(2/T)·sin((j+1)π t/T),  V'[j,t] = dt·sqrt(2/T)·(j+1)π/T·cos((j+1)π t/T),  t = t_idx·dt
  *   G[traj,j,k] = sum_t V[j,t]·Θ_k(x[traj,t]),   b[traj,j,i] = −sum_t V'[j,t]·x[traj,t,i]

@@ -387,6 +387,26 @@ int sb_rollout(const void* x0, int64_t n_ics, const sb_library* lib, const void*
                  (cudaStream_t)stream);
 }
 
+int sb_rollout_score(const float* x0, int64_t n_ics, const sb_library* lib, const float* w, int n_models, double dt,
+                     int64_t steps_per_row, int64_t n_rows, int method, const float* y_obs, float blowup,
+                     double* sse, int32_t* valid_rows, void* stream) {
+  LibTab t;
+  SB_TRY(build_table(lib, &t));
+  if (n_ics < 0 || n_models < 1 || steps_per_row < 1 || n_rows < 1 || n_rows > INT32_MAX ||
+      steps_per_row > INT64_MAX / n_rows) {
+    set_error("bad rollout_score sizes n_ics=%lld n_models=%d steps_per_row=%lld n_rows=%lld", (long long)n_ics,
+              n_models, (long long)steps_per_row, (long long)n_rows);
+    return SB_ERR_INVALID;
+  }
+  if (method != SB_EULER && method != SB_RK4) { set_error("unknown method %d", method); return SB_ERR_INVALID; }
+  if (!(dt > 0.0)) { set_error("dt=%g is not positive", dt); return SB_ERR_INVALID; }
+  SB_TRY(check_ptr(x0, "x0")); SB_TRY(check_ptr(w, "w")); SB_TRY(check_ptr(y_obs, "y_obs"));
+  SB_TRY(check_ptr(sse, "sse")); SB_TRY(check_ptr(valid_rows, "valid_rows"));
+  if (n_ics == 0) return SB_OK;
+  return rollout_score(x0, n_ics, t, w, n_models, dt, steps_per_row, n_rows, method, y_obs, blowup, sse, valid_rows,
+                       (cudaStream_t)stream);
+}
+
 int sb_wsindy_integrals(const float* x, int64_t n_traj, int64_t T, const sb_library* lib, float dt,
                         double t_max, int n_test, double* G, double* b, void* stream) {
   LibTab t;

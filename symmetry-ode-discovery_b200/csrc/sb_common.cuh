@@ -290,6 +290,11 @@ int rollout(const void* x0, int64_t n_ics, const LibTab& t, const void* w, doubl
             int64_t stride, int method, int dtype, int record_dx, void* x_out, void* dx_out, void* x_last,
             cudaStream_t s);
 
+// M models × N ICs integrated and scored against observed rows (sb_rollout_score.cu); arguments validated by the caller
+int rollout_score(const float* x0, int64_t n_ics, const LibTab& t, const float* w, int n_models, double dt,
+                  int64_t steps_per_row, int64_t n_rows, int method, const float* y_obs, float blowup, double* sse,
+                  int32_t* valid_rows, cudaStream_t s);
+
 // WSINDy integrals
 int wsindy_integrals(const float* x, int64_t n_traj, int64_t T, const LibTab& t, float dt, double t_max,
                      int n_test, double* G, double* b, cudaStream_t s);

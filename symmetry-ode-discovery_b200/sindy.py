@@ -28,7 +28,7 @@ from sindy_b200 import native, ops
 from sindy_b200.native import Library
 
 __all__ = ["SINDyRegression", "solve_SINDy_one_step", "solve_SINDy", "WSINDyWrapper", "stlsq_statistics",
-           "allreduce_statistics", "SINDyConst", "SINDyPoly1", "SINDyPoly2", "SINDyPoly3", "SINDySine", "SINDyExp"]
+           "allreduce_statistics", "stlsq_path", "score_path", "information_criteria", "apply_candidate", "SINDyConst", "SINDyPoly1", "SINDyPoly2", "SINDyPoly3", "SINDySine", "SINDyExp"]
 
 
 # ---- the reference's per-block library functions (`sindy.py:7-30`) --------------------------------------------------
@@ -349,40 +349,55 @@ def _masked_solve_batched(H, b, mask, rcond):
     support m_i = mask[i]. Same equilibration, same rank rule (threshold relative to the largest eigenvalue over ALL
     equations, dimension = number of live coefficients — K when every coefficient is live, as the reference then solves
     one K×K system with d right-hand sides). Returns Ξ (d × K, fp64), zero off the support."""
-    d, K = mask.shape
-    M = mask.to(H.dtype)
+    return _masked_solve_path(H, b, mask.unsqueeze(0), rcond)[0]
+
+
+def _masked_solve_path(H, b, masks, rcond):
+    """`_masked_solve_batched` for P supports at once (masks P × d × K -> Ξ P × d × K, fp64). Every decision that
+    function takes over its d equations — the Cholesky fast path, the rank threshold and the largest eigenvalue it is
+    relative to — is taken here per candidate p, so a rank-deficient candidate leaves the others' numerics alone."""
+    P, d, K = masks.shape
+    M = masks.to(H.dtype)
     if rcond > 0.0:
         scale = torch.ones(K, dtype=H.dtype, device=H.device)
     else:
         diag = torch.diagonal(H)
         scale = torch.where(diag > 0, diag.clamp_min(torch.finfo(H.dtype).tiny).rsqrt(), torch.zeros_like(diag))
     Hs = H * scale.unsqueeze(0) * scale.unsqueeze(1)
-    Hb = M.unsqueeze(2) * Hs.unsqueeze(0) * M.unsqueeze(1)
-    rhs = (scale.unsqueeze(1) * b).T * M                                   # d × K
+    Hb = M.unsqueeze(-1) * Hs * M.unsqueeze(-2)                           # P × d × K × K
+    rhs = (scale.unsqueeze(1) * b).T * M                                   # P × d × K
+    sol = None
     if rcond > 0.0:
-        cut = rcond * rcond
+        cut = torch.full((P,), rcond * rcond, dtype=H.dtype, device=H.device)
     else:
-        n_live = M.sum()
+        n_live = M.sum(dim=(1, 2))
         cut = torch.where(n_live == d * K, torch.full_like(n_live, float(K)), n_live) * torch.finfo(H.dtype).eps
         # Fast path for the full-rank case, which is every well-posed fit: Cholesky of the equilibrated blocks (dead
         # coordinates padded with ones). λ_min ≥ 1/‖L⁻¹‖_F² and λ_max ≤ K (unit diagonal), so when the bound clears the
         # rank rule's threshold no direction would have been dropped and the Cholesky solution IS the min-norm solution;
         # a 56 × 56 fp64 syevd costs ~0.6 ms on the device, nine of them per `solve_SINDy`, the batched Cholesky ~0.1.
         L, info = torch.linalg.cholesky_ex(Hb + torch.diag_embed(1.0 - M))
-        Linv = torch.linalg.solve_triangular(L, torch.eye(K, dtype=H.dtype, device=H.device).expand(d, K, K), upper=False)
+        Linv = torch.linalg.solve_triangular(L, torch.eye(K, dtype=H.dtype, device=H.device).expand(P, d, K, K),
+                                             upper=False)
         lam_min_bound = 1.0 / (Linv * Linv).sum(dim=(-1, -2)).clamp_min(torch.finfo(H.dtype).tiny)
-        full_rank = (info == 0).all() & (lam_min_bound.min() > cut * K) & torch.isfinite(Linv).all()
-        if bool(full_rank):                                                # one host sync (the loop has one per step anyway)
+        full_rank = ((info == 0).all(1) & (lam_min_bound.amin(1) > cut * K)
+                     & torch.isfinite(Linv).flatten(1).all(1))
+        n_full = int(full_rank.sum())                                      # one host sync (the loop has one per step anyway)
+        if n_full:
             # two triangular solves (cuBLAS trsm); `torch.cholesky_solve` costs ~1 s of solver-library start-up on its
             # first call, a third of a whole `main_wsindy.py` run on the test fixture
             y = torch.linalg.solve_triangular(L, rhs.unsqueeze(-1), upper=False)
             sol = torch.linalg.solve_triangular(L.transpose(-1, -2), y, upper=True).squeeze(-1)
-            return sol * scale * M
+            if n_full == P:
+                return sol * scale * M
     lam, U = torch.linalg.eigh(Hb)
-    keep = lam > cut * lam.max().clamp_min(0)
+    keep = lam > cut.view(P, 1, 1) * lam.amax(dim=(1, 2), keepdim=True).clamp_min(0)
     inv = torch.where(keep, 1.0 / lam.clamp_min(torch.finfo(lam.dtype).tiny), torch.zeros_like(lam))
     proj = torch.matmul(U.transpose(-1, -2), rhs.unsqueeze(-1)).squeeze(-1)
-    return torch.matmul(U, (inv * proj).unsqueeze(-1)).squeeze(-1) * scale * M
+    eig = torch.matmul(U, (inv * proj).unsqueeze(-1)).squeeze(-1)
+    if sol is not None:
+        eig = torch.where(full_rank.view(P, 1, 1), sol, eig)
+    return eig * scale * M
 
 
 def _stlsq_update(regressor, G, b, ridge, n_rows, st_threshold, driver='gels'):
@@ -512,6 +527,202 @@ def solve_SINDy(regressor, x, y, w_sindy_reg, st_threshold, max_iter=5, **kwargs
     return residual
 
 
+# --------------------------------------------------------------------------------------------------------
+# model selection along the threshold path (Mangan et al., Model selection for dynamical systems via sparse regression
+# and information criteria, Proc. R. Soc. A 2017): sweep the threshold, keep each candidate model, simulate every
+# candidate on held-out trajectories and rank them by an information criterion of the simulation error
+# --------------------------------------------------------------------------------------------------------
+def _path_thresholds(thresholds):
+    thr = np.asarray(thresholds, dtype=np.float64)
+    if thr.ndim != 1 or thr.size == 0:
+        raise ValueError(f"thresholds must be a non-empty 1-D sequence, got shape {thr.shape}")
+    if not np.all(np.isfinite(thr)) or np.any(thr < 0):
+        raise ValueError("thresholds must be finite and non-negative")
+    return thr
+
+
+def _path_max_iter(max_iter):
+    if isinstance(max_iter, bool) or not isinstance(max_iter, (int, np.integer)) or max_iter < 1:
+        raise ValueError(f"max_iter must be a positive integer, got {max_iter!r}")
+    return int(max_iter)
+
+
+def _stlsq_path_solve(regressor, A, rhs, bb, ridge, n_rows, thr, max_iter, driver, step):
+    """Candidate p = what `reset_mask()` and up to max_iter STLSQ updates with threshold thr[p] on the normal equations
+    (A + ridge·I) ξ = rhs leave, stopping at the first converged update. Returns the path dict with Ξ (fp32, masked),
+    the masks, convergence flags and the quadratic residual Σ-per-equation q_i = ξᵢᵀAξᵢ − 2ξᵢᵀrhsᵢ + bbᵢ + ridge·‖ξᵢ‖²
+    of each candidate's last solve (fp64, P × d). Unconstrained: the P·d masked solves of each iteration are one batch
+    (`_masked_solve_path`). Constrained: `step()` (one update of the regressor itself) in a loop; the regressor's
+    parameters and mask are restored afterwards."""
+    d, K = regressor.latent_dim, A.shape[0]
+    dev = A.device
+    P = thr.shape[0]
+    out = {"thresholds": torch.from_numpy(thr.copy())}
+    if not regressor.constraint:
+        H = A + ridge * torch.eye(K, dtype=A.dtype, device=dev)
+        rcond = float(torch.finfo(torch.float32).eps) * min(max(n_rows, K), 1 << 14) if driver == 'gelsy' else 0.0
+        thr32 = torch.as_tensor(thr, dtype=torch.float64, device=dev).to(torch.float32).view(P, 1, 1)
+        masks = torch.ones(P, d, K, dtype=torch.bool, device=dev)
+        xi = torch.zeros(P, d, K, dtype=torch.float32, device=dev)
+        converged = torch.zeros(P, dtype=torch.bool, device=dev)
+        active = torch.arange(P, device=dev)
+        for _ in range(max_iter):
+            sol = _masked_solve_path(H, rhs, masks[active], rcond).to(torch.float32)
+            keep = (sol.abs() > thr32[active]) & masks[active]     # set_threshold: |Ξ| > threshold in fp32
+            conv = (keep == masks[active]).flatten(1).all(1)
+            xi[active], masks[active], converged[active] = sol, keep, conv
+            active = active[~conv]
+            if active.numel() == 0:
+                break
+        out.update(xi=xi * masks, mask=masks, converged=converged)
+    else:
+        saved = ({n: p.data for n, p in regressor.named_parameters()}, regressor.mask.data, regressor.Xi)
+        xis, betas, consts, masks, converged = [], [], [], [], []
+        try:
+            for t in thr.tolist():
+                regressor.reset_mask()
+                for _ in range(max_iter):
+                    conv = step(float(t))
+                    if conv:
+                        break
+                xi = regressor._current_Xi().detach()
+                xis.append(xi.to(torch.float32))
+                betas.append(regressor.beta.data.clone())
+                consts.append(regressor.const.data.clone())
+                masks.append(regressor.mask > 0)
+                converged.append(bool(conv))
+        finally:
+            params, regressor.mask.data, regressor.Xi = saved
+            for n, p in regressor.named_parameters():
+                p.data = params[n]
+        xi, masks = torch.stack(xis), torch.stack(masks)
+        out.update(xi=xi, beta=torch.stack(betas), const=torch.stack(consts), mask=masks,
+                   converged=torch.tensor(converged, device=dev))
+        out["xi"] = xi * masks
+    # residual from the last solve's parameters (zero off the previous support, not yet masked by the new one) — for
+    # live coefficients equal to out["xi"], for thresholded ones the values just cut
+    raw = xi.to(torch.float64)
+    quad = torch.einsum('pik,kl,pil->pi', raw, A, raw) - 2.0 * torch.einsum('pik,ki->pi', raw, rhs) + bb
+    out["quad"] = quad + ridge * (raw ** 2).sum(-1)
+    out["n_terms"] = out["mask"].flatten(1).sum(1)
+    return out
+
+
+def stlsq_path(regressor, x, y, thresholds, w_sindy_reg=0.0, max_iter=5, **kwargs):
+    """The STLSQ threshold path from ONE statistics pass: candidate p is what
+    `solve_SINDy(regressor, x, y, w_sindy_reg, thresholds[p], max_iter)` leaves in the regressor. Takes `sharded` /
+    `group` / `lstsq_driver` as solve_SINDy does. Returns a dict of
+      thresholds (P,) fp64 (host), xi (P, d, K) fp32 = Ξ⊙mask, mask (P, d, K) bool, residual (P,) fp32 (solve_SINDy's
+      return value), n_terms (P,), converged (P,) bool,
+    and, for an equivariance-constrained regressor, the raw beta (P, ·) / const (P, d, 1). The regressor's parameters
+    and mask are left as they were; `apply_candidate` writes one candidate into it."""
+    thr = _path_thresholds(thresholds)
+    max_iter = _path_max_iter(max_iter)
+    lib = regressor.library
+    stats = stlsq_statistics(regressor, x, y)
+    if kwargs.get('sharded'):
+        stats = allreduce_statistics(stats, kwargs.get('group'))
+    driver = _lstsq_driver(kwargs)
+    G, b, yy, n = stats["G"], stats["b"], stats["yy"], stats["n"]
+    ridge = float(w_sindy_reg) ** 2
+
+    def step(t):
+        return _stlsq_update(regressor, G, b, ridge, n + lib.K, t, driver)
+
+    with torch.no_grad():
+        out = _stlsq_path_solve(regressor, G, b, yy, ridge, n + lib.K, thr, max_iter, driver, step)
+        out["residual"] = (out.pop("quad").mean(-1) / n).to(torch.float32)
+    return out
+
+
+def score_path(library, path, x_val, dt, steps_per_row=1, method='rk4', blowup=None, criterion='aicc'):
+    """Scores the candidates of `stlsq_path` / `WSINDyWrapper.solve_path` by simulation on held-out trajectories.
+
+    x_val (n_traj, T, d): trajectories with rows dt·steps_per_row apart. Every distinct candidate model is integrated
+    once (`native.rollout_score`, one launch for all of them) from x_val[:, 0] with step dt and compared with rows
+    1..T−1. Per candidate: sse (fp64), diverged (some IC hit a non-finite state or |x| > blowup), k = live
+    coefficients, and, with n = n_obs = n_traj·(T−1)·d,
+      AIC = n·ln(SSE/n) + 2k,  AICc = AIC + 2k(k+1)/(n−k−1),  BIC = n·ln(SSE/n) + k·ln n
+    (+inf for a diverged candidate; AICc also when n−k−1 ≤ 0). `chosen` is the argmin of `criterion` ('aic', 'aicc' or
+    'bic'); ties go to the smaller k, then the larger threshold; None if every candidate scores +inf. `library` is a
+    `native.Library` or a SINDyRegression."""
+    lib = getattr(library, 'library', library)
+    if not isinstance(lib, Library):
+        raise ValueError(f"library must be a native.Library or a SINDyRegression, got {type(library).__name__}")
+    if criterion not in ('aic', 'aicc', 'bic'):
+        raise ValueError(f"criterion must be 'aic', 'aicc' or 'bic', got {criterion!r}")
+    if method not in ('euler', 'rk4'):
+        raise ValueError(f"method must be 'euler' or 'rk4', got {method!r}")
+    if isinstance(steps_per_row, bool) or not isinstance(steps_per_row, (int, np.integer)) or steps_per_row < 1:
+        raise ValueError(f"steps_per_row must be a positive integer, got {steps_per_row!r}")
+    dt = float(dt)
+    if not (math.isfinite(dt) and dt > 0):
+        raise ValueError(f"dt must be positive, got {dt}")
+    if blowup is not None and not (math.isfinite(float(blowup)) and float(blowup) > 0):
+        raise ValueError(f"blowup must be a positive number or None, got {blowup!r}")
+    x_val = torch.as_tensor(x_val)
+    if x_val.dim() != 3 or x_val.shape[-1] != lib.dim:
+        raise ValueError(f"x_val must be (n_traj, T, {lib.dim}), got {tuple(x_val.shape)}")
+    n_traj, T, d = x_val.shape
+    if T < 2 or n_traj < 1:
+        raise ValueError(f"x_val needs at least one trajectory of T >= 2 rows, got {tuple(x_val.shape)}")
+    if not bool(torch.isfinite(x_val).all()):
+        raise ValueError("x_val has non-finite values")
+    W, masks = path["xi"], path["mask"]
+    if W.dim() != 3 or W.shape[1:] != (d, lib.K) or masks.shape != W.shape:
+        raise ValueError(f"path['xi'] / path['mask'] must be (P, {d}, {lib.K}), got {tuple(W.shape)} / "
+                         f"{tuple(masks.shape)}")
+    thr = torch.as_tensor(path["thresholds"], dtype=torch.float64).cpu()
+    P = W.shape[0]
+    dev = W.device
+    xv = x_val.to(device=dev, dtype=torch.float32)
+    models, inverse = torch.unique(W.reshape(P, -1), dim=0, return_inverse=True)
+    with torch.no_grad():
+        sse, valid = native.rollout_score(xv[:, 0].contiguous(), models.view(-1, d, lib.K), lib, dt, int(steps_per_row),
+                                          xv[:, 1:].transpose(0, 1).contiguous(), method, blowup)
+    sse = sse.sum(1).cpu()[inverse.cpu()]
+    diverged = (valid < T - 1).any(1).cpu()[inverse.cpu()]
+    k = masks.flatten(1).sum(1).cpu().to(torch.float64)
+    n = n_traj * (T - 1) * d
+    crit = information_criteria(sse, n, k)
+    for c in crit.values():
+        c[diverged] = math.inf
+    out = {"sse": sse, "diverged": diverged, "n_obs": n, "k": k.to(torch.int64), **crit, "criterion": criterion}
+    c = crit[criterion].numpy()
+    order = np.lexsort((-thr.numpy(), k.numpy(), c))                      # last key sorts first
+    out["chosen"] = int(order[0]) if c[order[0]] < math.inf else None
+    return out
+
+
+def information_criteria(sse, n, k):
+    """AIC, AICc and BIC of Gaussian residuals with sum of squares `sse` over n observations and k parameters (fp64
+    tensors of one shape, or scalars): n·ln(SSE/n) + 2k, that + 2k(k+1)/(n−k−1) (+inf when n−k−1 ≤ 0), and
+    n·ln(SSE/n) + k·ln n."""
+    sse = torch.as_tensor(sse, dtype=torch.float64)
+    k = torch.as_tensor(k, dtype=torch.float64)
+    fit = n * torch.log(sse / n)
+    aic = fit + 2.0 * k
+    den = n - k - 1.0
+    aicc = torch.where(den > 0, aic + 2.0 * k * (k + 1.0) / den.clamp_min(1.0), torch.full_like(aic, math.inf))
+    bic = fit + k * math.log(n)
+    return {"aic": aic, "aicc": aicc, "bic": bic}
+
+
+def apply_candidate(regressor, path, i):
+    """Writes candidate i of a threshold path into the regressor: Ξ (or β / const) and the mask."""
+    i = int(i)
+    with torch.no_grad():
+        mask = path["mask"][i].to(device=regressor.mask.device, dtype=regressor.mask.dtype)
+        if regressor.constraint:
+            regressor.beta.data = path["beta"][i].to(regressor.beta.device).clone()
+            regressor.const.data = path["const"][i].to(regressor.const.device).clone()
+            regressor.Xi = regressor.get_Xi()
+        else:
+            regressor.Xi.data = path["xi"][i].to(regressor.Xi.device).clone()
+        regressor.mask.data = mask.clone()
+    return regressor
+
+
 def _local_test_functions(T, dt, n_test, support=None, degree=None):
     """The compactly supported piecewise-polynomial family of WSINDyWrapper(test_func_family='poly') (Messenger &
     Bortz, Weak SINDy for ODEs, 2021): every row is the same window of L samples at its own start
@@ -604,6 +815,26 @@ class WSINDyWrapper():
             return native.wsindy_local_integrals(x, self.regressor.library, self.phi, self.dphi, self.num_test_funcs)
         return native.wsindy_integrals(x, self.regressor.library, float(self.dt), self.t_max, self.num_test_funcs)
 
+    def _normal_equations(self, x):
+        """(GᵀMG, GᵀMb, bᵀMb per equation, row count of the reference's least-squares matrix) for (T, d) or pooled
+        (n_traj, T, d) input."""
+        if x.shape[-2] != self.t.shape[0] or x.dim() not in (2, 3):
+            raise ValueError(f'x has {x.shape[-2]} time samples, the wrapper was built for {self.t.shape[0]}')
+        Gw, bw = self.integrals(x)
+        if x.dim() == 2:
+            MG = self.M @ Gw
+            A = Gw.T @ MG                                    # K×K
+            rhs = MG.T @ bw                                  # K×d
+            bb = torch.einsum('ji,jl,li->i', bw, self.M, bw)
+            n_rows = x.shape[0]
+        else:
+            MG = self.M @ Gw                                 # n_traj × n_test × K
+            A = (Gw.transpose(1, 2) @ MG).sum(0)
+            rhs = (MG.transpose(1, 2) @ bw).sum(0)
+            bb = torch.einsum('rji,jl,rli->i', bw, self.M, bw)
+            n_rows = x.shape[0] * x.shape[1]
+        return A, rhs, bb, n_rows
+
     def solve(self, x, w_sindy_reg, st_threshold, **kwargs):
         '''
         x: (seq_len, dim) on the wrapper's uniform grid. Solves [VᵀG; sqrt(w)·I] ξ = [Vᵀb; 0] on the current
@@ -613,21 +844,7 @@ class WSINDyWrapper():
         Returns (mean squared residual of that system, converged).
         '''
         with torch.no_grad():
-            if x.shape[-2] != self.t.shape[0] or x.dim() not in (2, 3):
-                raise ValueError(f'x has {x.shape[-2]} time samples, the wrapper was built for {self.t.shape[0]}')
-            Gw, bw = self.integrals(x)
-            if x.dim() == 2:
-                MG = self.M @ Gw
-                A = Gw.T @ MG                                    # K×K
-                rhs = MG.T @ bw                                  # K×d
-                bb = torch.einsum('ji,jl,li->i', bw, self.M, bw)
-                n_rows = x.shape[0]
-            else:
-                MG = self.M @ Gw                                 # n_traj × n_test × K
-                A = (Gw.transpose(1, 2) @ MG).sum(0)
-                rhs = (MG.transpose(1, 2) @ bw).sum(0)
-                bb = torch.einsum('rji,jl,rli->i', bw, self.M, bw)
-                n_rows = x.shape[0] * x.shape[1]
+            A, rhs, bb, n_rows = self._normal_equations(x)
             K = A.shape[0]
             converged = _stlsq_update(self.regressor, A, rhs, float(w_sindy_reg), n_rows + K, st_threshold,
                                       _lstsq_driver(kwargs if kwargs.get('lstsq_driver') else self.kwargs))
@@ -635,3 +852,23 @@ class WSINDyWrapper():
             quad = torch.einsum('ik,kl,il->i', Xi, A, Xi) - 2.0 * torch.einsum('ik,ki->i', Xi, rhs) + bb
             quad = quad + float(w_sindy_reg) * (Xi ** 2).sum(1)
         return quad.mean().item(), converged
+
+    def solve_path(self, x, w_sindy_reg, thresholds, max_iter=5, **kwargs):
+        """The threshold path of `solve` from one evaluation of the integrals (x of shape (T, d) or (n_traj, T, d)):
+        candidate p is what `reset_mask()` followed by up to max_iter calls of `solve(x, w_sindy_reg, thresholds[p])`,
+        stopping at the first converged call, leaves in the regressor. Returns the dict of `stlsq_path` with `residual`
+        (P,) fp64 = the value the last `solve` returns; the regressor is left as it was."""
+        thr = _path_thresholds(thresholds)
+        max_iter = _path_max_iter(max_iter)
+        driver = _lstsq_driver(kwargs if kwargs.get('lstsq_driver') else self.kwargs)
+        with torch.no_grad():
+            A, rhs, bb, n_rows = self._normal_equations(x)
+            K = A.shape[0]
+            ridge = float(w_sindy_reg)
+
+            def step(t):
+                return _stlsq_update(self.regressor, A, rhs, ridge, n_rows + K, t, driver)
+
+            out = _stlsq_path_solve(self.regressor, A, rhs, bb, ridge, n_rows + K, thr, max_iter, driver, step)
+            out["residual"] = out.pop("quad").mean(-1)
+        return out

@@ -8,6 +8,7 @@ is missing or the tensors are not on a CUDA device.
 from __future__ import annotations
 
 import ctypes
+import math
 import os
 import threading
 from ctypes import POINTER, c_char_p, c_double, c_float, c_int, c_int32, c_int64, c_uint32, c_void_p
@@ -70,6 +71,8 @@ _SIGNATURES = {
     "sb_train_step_variant": (c_char_p, [POINTER(_CLibrary), c_uint32]),
     "sb_rollout": (c_int, [c_void_p, c_int64, POINTER(_CLibrary), c_void_p, c_double, c_int64, c_int64, c_int,
                            c_int, c_int, c_void_p, c_void_p, c_void_p, c_void_p]),
+    "sb_rollout_score": (c_int, [c_void_p, c_int64, POINTER(_CLibrary), c_void_p, c_int, c_double, c_int64, c_int64,
+                                 c_int, c_void_p, c_float, c_void_p, c_void_p, c_void_p]),
     "sb_wsindy_integrals": (c_int, [c_void_p, c_int64, c_int64, POINTER(_CLibrary), c_float, c_double, c_int,
                                     c_void_p, c_void_p, c_void_p]),
     "sb_wsindy_local_integrals": (c_int, [c_void_p, c_int64, c_int64, POINTER(_CLibrary), c_void_p, c_void_p, c_int,
@@ -529,6 +532,48 @@ def rollout(x0: torch.Tensor, w: torch.Tensor, lib: Library, dt: float, n_steps:
                                  int(n_steps), int(stride), meth, dtype, int(bool(record_dx)), _ptr(x_out),
                                  _ptr(dx_out), _ptr(x_last), _stream(dev)), "sb_rollout")
     return x_out, dx_out, x_last
+
+
+def rollout_score(x0: torch.Tensor, W: torch.Tensor, lib: Library, dt: float, steps_per_row: int, y_obs: torch.Tensor,
+                  method: str = "rk4", blowup: Optional[float] = None) -> Tuple[torch.Tensor, torch.Tensor]:
+    """Every model W[m] (M × d × K, already masked; one d × K model is M = 1) integrated in fp32 from every initial
+    condition x0 (N × d) and compared with y_obs (n_rows × N × d: the states after steps_per_row, 2·steps_per_row, ...
+    steps). Returns sse (M × N fp64, summed over the rows compared) and valid_rows (M × N int32: rows compared before
+    the first non-finite state or |x_j| > blowup; n_rows if none). The compared states are bit-identical to
+    rollout(x0, W[m], lib, dt, n_rows·steps_per_row, stride=steps_per_row, method). See sb_rollout_score."""
+    x0f = _flat(_f32c(x0, "x0"), lib.dim, "x0")
+    n_ics, d = x0f.shape
+    dev = x0f.device
+    W = _f32c(W, "W")
+    if W.dim() == 2:
+        W = W.unsqueeze(0)
+    if W.dim() != 3 or W.shape[1:] != (d, lib.K):
+        raise ValueError(f"W has shape {tuple(W.shape)}, expected (n_models, {d}, {lib.K})")
+    y = _f32c(y_obs, "y_obs")
+    if y.dim() != 3 or y.shape[1:] != (n_ics, d) or y.shape[0] < 1:
+        raise ValueError(f"y_obs has shape {tuple(y.shape)}, expected (n_rows >= 1, {n_ics}, {d})")
+    if W.device != dev or y.device != dev:
+        raise ValueError("x0, W and y_obs must be on one device")
+    meth = {"euler": SB_EULER, "rk4": SB_RK4}.get(method)
+    if meth is None:
+        raise ValueError("Unrecognized ODEInt method.")
+    if isinstance(steps_per_row, bool) or int(steps_per_row) != steps_per_row or steps_per_row < 1:
+        raise ValueError(f"steps_per_row must be a positive integer, got {steps_per_row!r}")
+    if not (math.isfinite(dt) and dt > 0):
+        raise ValueError(f"dt must be positive, got {dt}")
+    if blowup is not None and not blowup > 0:
+        raise ValueError(f"blowup must be positive or None, got {blowup}")
+    n_models = W.shape[0]
+    sse = torch.empty(n_models, n_ics, dtype=torch.float64, device=dev)
+    valid = torch.empty(n_models, n_ics, dtype=torch.int32, device=dev)
+    if n_models == 0 or n_ics == 0:
+        return sse, valid
+    with torch.cuda.device(dev):
+        _check(load().sb_rollout_score(x0f.data_ptr(), n_ics, ctypes.byref(lib.c()), W.data_ptr(), n_models, float(dt),
+                                       int(steps_per_row), y.shape[0], meth, y.data_ptr(),
+                                       0.0 if blowup is None else float(blowup), sse.data_ptr(), valid.data_ptr(),
+                                       _stream(dev)), "sb_rollout_score")
+    return sse, valid
 
 
 def wsindy_integrals(x: torch.Tensor, lib: Library, dt: float, t_max: float, n_test: int = 50):
