@@ -42,7 +42,8 @@ class EulerFlowMap:
     kernel launch (sb_euler_flow) with a one-launch backward, where the reference runs two reverse passes through
     n Python Euler steps with create_graph=True (`model_utils.py:55-56`). `symmreg_i` uses it when it is handed one;
     any other callable takes the reference's double-vjp path. Falls back to the operator-by-operator composition for
-    libraries without a fused kernel or off the GPU."""
+    libraries without a fused kernel, off the GPU, and for flows longer than the fused backward handles
+    (native.EULER_FLOW_MAX_STEPS)."""
 
     def __init__(self, regressor, t, dt):
         self.regressor, self.t, self.dt = regressor, t, dt
@@ -50,7 +51,7 @@ class EulerFlowMap:
 
     def _fused(self, x):
         return (_is_regressor(self.regressor) and torch.is_tensor(x) and x.is_cuda
-                and native.symreg_supported(self.regressor.library))
+                and self.n_steps <= native.EULER_FLOW_MAX_STEPS and native.symreg_supported(self.regressor.library))
 
     def _w(self):
         reg = self.regressor

@@ -627,6 +627,11 @@ def symreg_supported(lib: Library) -> bool:
     return bool(load().sb_symreg_supported(ctypes.byref(lib.c())))
 
 
+# Longest flow euler_flow_backward accepts: the backward kernel keeps every step's state in a fixed per-thread array
+# (`kMaxSteps` in csrc/sb_symreg.cu) and returns SB_ERR_UNSUPPORTED beyond it. The forward has no limit.
+EULER_FLOW_MAX_STEPS = 32
+
+
 def euler_flow(x: torch.Tensor, v: Optional[torch.Tensor], w: torch.Tensor, lib: Library, dt: float, n_steps: int):
     """fx = n_steps explicit-Euler steps of h(x) = Θ(x)Wᵀ from x (`model_utils.py:236-240`) and, with v, jv = J_f(x)·v
     (`model_utils.py:55-56`), one launch. Shapes of x are kept; returns (fx, jv or None)."""

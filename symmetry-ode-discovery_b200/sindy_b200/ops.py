@@ -213,7 +213,12 @@ class _EulerFlowValue(Function):
 
 
 def euler_flow(x, v, w, lib: Library, dt: float, n_steps: int):
-    """Differentiable (f(x), J_f(x)·v) — v may be None: (f(x), None)."""
+    """Differentiable (f(x), J_f(x)·v) — v may be None: (f(x), None). The backward handles at most
+    native.EULER_FLOW_MAX_STEPS steps: a longer flow that will need a gradient is refused here, at forward time."""
+    if (n_steps > native.EULER_FLOW_MAX_STEPS and torch.is_grad_enabled()
+            and any(t is not None and t.requires_grad for t in (x, v, w))):
+        raise ValueError(f"euler_flow: the fused backward handles at most {native.EULER_FLOW_MAX_STEPS} steps, got "
+                         f"{n_steps}; differentiate a longer flow by composing its steps (model_utils.odeint)")
     if v is None:
         return _EulerFlowValue.apply(x, w, lib, dt, n_steps), None
     return _EulerFlow.apply(x, v, w, lib, dt, n_steps)
