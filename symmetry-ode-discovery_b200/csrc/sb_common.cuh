@@ -140,19 +140,30 @@ __host__ __device__ inline bool lib_matches(const LibTab& t) {
   using L = LibCode<D, PC>;
   return t.d == D && t.n_poly == L::NP && (t.sine != 0) == (L::S != 0) && (t.exp_ != 0) == (L::E != 0);
 }
-// Θ(x) for a library code: the polynomial block, then sin(x_j), then exp(x_j) (`sindy.py:7-30`)
-template <int D, int PC>
-__device__ __forceinline__ void expand_lib(const float (&x)[D], float (&m)[LibCode<D, PC>::K]) {
+// Θ(x) for a library code: the polynomial block, then sin(x_j), then exp(x_j) (`sindy.py:7-30`); sin / exp are
+// sinf / expf for float by overload
+template <int D, int PC, class T>
+__device__ __forceinline__ void expand_lib(const T (&x)[D], T (&m)[LibCode<D, PC>::K]) {
   using L = LibCode<D, PC>;
   if constexpr (L::S == 0 && L::E == 0) {
     expand_poly<D, L::P>(x, m);
   } else {
-    float mp[L::NP];
+    T mp[L::NP];
     expand_poly<D, L::P>(x, mp);
     static_for<0, L::NP>([&](auto k) { m[k] = mp[k]; });
-    if constexpr (L::S) static_for<0, D>([&](auto j) { m[L::NP + j] = sinf(x[j]); });
-    if constexpr (L::E) static_for<0, D>([&](auto j) { m[L::NP + D * L::S + j] = expf(x[j]); });
+    if constexpr (L::S) static_for<0, D>([&](auto j) { m[L::NP + j] = sin(x[j]); });
+    if constexpr (L::E) static_for<0, D>([&](auto j) { m[L::NP + D * L::S + j] = exp(x[j]); });
   }
+}
+// Θ(x) for a runtime table, in the same column order; m holds at least t.K values
+template <class T>
+__device__ __forceinline__ void expand_table(const LibTab& t, const T* x, T* m) {
+  m[0] = T(1);
+  for (int j = 0; j < t.d; ++j) m[1 + j] = x[j];
+  for (int k = 1 + t.d; k < t.n_poly; ++k) m[k] = m[t.parent[k]] * x[t.var[k]];
+  int k = t.n_poly;
+  if (t.sine) for (int j = 0; j < t.d; ++j) m[k++] = sin(x[j]);
+  if (t.exp_) for (int j = 0; j < t.d; ++j) m[k++] = exp(x[j]);
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -290,7 +301,8 @@ int rollout(const void* x0, int64_t n_ics, const LibTab& t, const void* w, doubl
             int64_t stride, int method, int dtype, int record_dx, void* x_out, void* dx_out, void* x_last,
             cudaStream_t s);
 
-// M models × N ICs integrated and scored against observed rows (sb_rollout_score.cu); arguments validated by the caller
+// M models × N ICs integrated and scored against observed rows with the rollout's own step and right-hand sides
+// (sb_rollout.cu), so the compared states are the ones `rollout` stores; arguments validated by the caller
 int rollout_score(const float* x0, int64_t n_ics, const LibTab& t, const float* w, int n_models, double dt,
                   int64_t steps_per_row, int64_t n_rows, int method, const float* y_obs, float blowup, double* sse,
                   int32_t* valid_rows, cudaStream_t s);

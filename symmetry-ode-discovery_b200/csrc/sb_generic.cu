@@ -28,17 +28,6 @@ __device__ __forceinline__ void load_x(const float* __restrict__ x, int64_t s, i
     if (j < d) xv[j] = __ldg(x + s * d + j);
 }
 
-// Θ(x): `sindy.py:201-203`
-template <int KMAX>
-__device__ __forceinline__ void expand(const LibTab& t, const float* xv, float* m) {
-  m[0] = 1.f;
-  for (int j = 0; j < t.d; ++j) m[1 + j] = xv[j];
-  for (int k = 1 + t.d; k < t.n_poly; ++k) m[k] = m[t.parent[k]] * xv[t.var[k]];
-  int k = t.n_poly;
-  if (t.sine) for (int j = 0; j < t.d; ++j) m[k++] = sinf(xv[j]);
-  if (t.exp_) for (int j = 0; j < t.d; ++j) m[k++] = expf(xv[j]);
-}
-
 // tt = J_Θ(x)·u by forward differentiation of the recurrence
 template <int KMAX>
 __device__ __forceinline__ void tangent(const LibTab& t, const float* xv, const float* uv, const float* m,
@@ -70,7 +59,7 @@ __global__ void __launch_bounds__(kThreads) theta_kernel(LibTab t, const float* 
   float m[KMAX], xv[SB_MAX_DIM];
   for (int64_t s = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; s < n; s += (int64_t)gridDim.x * blockDim.x) {
     load_x<KMAX>(x, s, t.d, xv);
-    expand<KMAX>(t, xv, m);
+    expand_table(t, xv, m);
     for (int k = 0; k < t.K; ++k) theta[s * t.K + k] = m[k];
   }
 }
@@ -81,7 +70,7 @@ __global__ void __launch_bounds__(kThreads) forward_kernel(LibTab t, const float
   float m[KMAX], xv[SB_MAX_DIM];
   for (int64_t s = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; s < n; s += (int64_t)gridDim.x * blockDim.x) {
     load_x<KMAX>(x, s, t.d, xv);
-    expand<KMAX>(t, xv, m);
+    expand_table(t, xv, m);
     for (int i = 0; i < t.d; ++i) y[s * t.d + i] = dot_w<KMAX>(w, i, t.K, m);
   }
 }
@@ -94,7 +83,7 @@ __global__ void __launch_bounds__(kThreads) jvp_kernel(LibTab t, const float* __
   for (int64_t s = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; s < n; s += (int64_t)gridDim.x * blockDim.x) {
     load_x<KMAX>(x, s, t.d, xv);
     load_x<KMAX>(u, s, t.d, uv);
-    expand<KMAX>(t, xv, m);
+    expand_table(t, xv, m);
     tangent<KMAX>(t, xv, uv, m, tt);
     for (int i = 0; i < t.d; ++i) out[s * t.d + i] = dot_w<KMAX>(w, i, t.K, tt);
   }
@@ -110,7 +99,7 @@ __global__ void __launch_bounds__(kThreads) backward_x_kernel(LibTab t, const fl
   for (int64_t s = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; s < n; s += (int64_t)gridDim.x * blockDim.x) {
     load_x<KMAX>(x, s, t.d, xv);
     load_x<KMAX>(gy, s, t.d, gv);
-    expand<KMAX>(t, xv, m);
+    expand_table(t, xv, m);
     for (int k = 0; k < t.K; ++k) {
       float c = 0.f;
       for (int i = 0; i < t.d; ++i) c = fmaf(gv[i], __ldg(w + i * t.K + k), c);
@@ -144,7 +133,7 @@ __global__ void __launch_bounds__(kThreads) jvp_backward_xu_kernel(LibTab t, con
     load_x<KMAX>(x, s, t.d, xv);
     load_x<KMAX>(u, s, t.d, uv);
     load_x<KMAX>(g, s, t.d, gv);
-    expand<KMAX>(t, xv, m);
+    expand_table(t, xv, m);
     tangent<KMAX>(t, xv, uv, m, tt);
     for (int k = 0; k < t.K; ++k) {
       float c = 0.f;
@@ -234,7 +223,7 @@ __global__ void __launch_bounds__(kThreads) rows_kernel(LibTab t, RowsArgs a) {
 
   for (int64_t s = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; s < a.n; s += (int64_t)a.nbx * blockDim.x) {
     load_x<KMAX>(a.x, s, d, xv);
-    expand<KMAX>(t, xv, m);
+    expand_table(t, xv, m);
     float L;
     const float* feat = m;
     if (MODE == MODE_STEP) {

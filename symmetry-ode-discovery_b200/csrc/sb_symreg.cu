@@ -33,11 +33,7 @@ struct Lib {
   using T = Poly<D, P>;
 
   __device__ static __forceinline__ void expand(const float (&x)[D], float (&m)[K]) {
-    float mp[NP];
-    expand_poly<D, P>(x, mp);
-    static_for<0, NP>([&](auto k) { m[k] = mp[k]; });
-    if constexpr (S) static_for<0, D>([&](auto j) { m[NP + j] = sinf(x[j]); });
-    if constexpr (E) static_for<0, D>([&](auto j) { m[NP + D * S + j] = expf(x[j]); });
+    expand_lib<D, P + 10 * E + 20 * S>(x, m);
   }
   // t = J_Θ(x)·u (forward differentiation of the recurrence); cs = cos(x) when S
   __device__ static __forceinline__ void tangent(const float (&x)[D], const float (&u)[D], const float (&m)[K],

@@ -77,12 +77,7 @@ __global__ void __launch_bounds__(kThreads) wsindy_kernel(LibTab t, WsArgs a) {
 #pragma unroll
     for (int q = 0; q < SB_MAX_DIM; ++q)
       if (q < d) xv[q] = __ldg(xt + ti * d + q);
-    m[0] = 1.f;
-    for (int q = 0; q < d; ++q) m[1 + q] = xv[q];
-    for (int k = 1 + d; k < t.n_poly; ++k) m[k] = m[t.parent[k]] * xv[t.var[k]];
-    int k = t.n_poly;
-    if (t.sine) for (int q = 0; q < d; ++q) m[k++] = sinf(xv[q]);
-    if (t.exp_) for (int q = 0; q < d; ++q) m[k++] = expf(xv[q]);
+    expand_table(t, xv, m);
     for (int q = 0; q < K; ++q) acc[q] = fmaf(v, m[q], acc[q]);
 #pragma unroll
     for (int q = 0; q < SB_MAX_DIM; ++q)

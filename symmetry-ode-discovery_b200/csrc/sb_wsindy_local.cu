@@ -104,8 +104,8 @@ __global__ void __launch_bounds__(32 * kWarps) wsindy_local_kernel(WlArgs a) {
   }
 }
 
-// Any library: the same rows, blocks and summation structure with a runtime Θ table (`sb_wsindy.cu`'s per-sample
-// expansion) and per-column warp sums instead of the fold.
+// Any library: the same rows, blocks and summation structure with a runtime Θ table (expand_table, as in
+// sb_wsindy.cu) and per-column warp sums instead of the fold.
 template <int KMAX>
 __global__ void __launch_bounds__(32 * kWarps) wsindy_local_generic_kernel(LibTab t, WlArgs a) {
   __shared__ double tot[kWarps][KMAX + SB_MAX_DIM];
@@ -130,12 +130,7 @@ __global__ void __launch_bounds__(32 * kWarps) wsindy_local_generic_kernel(LibTa
           for (int i = 0; i < SB_MAX_DIM; ++i)
             if (i < d) xv[i] = __ldg(xs + (int64_t)q * d + i);
           const float w = __ldg(a.phi + q), wd = __ldg(a.dphi + q);
-          m[0] = 1.f;
-          for (int i = 0; i < d; ++i) m[1 + i] = xv[i];
-          for (int k = 1 + d; k < t.n_poly; ++k) m[k] = m[t.parent[k]] * xv[t.var[k]];
-          int k = t.n_poly;
-          if (t.sine) for (int i = 0; i < d; ++i) m[k++] = sinf(xv[i]);
-          if (t.exp_) for (int i = 0; i < d; ++i) m[k++] = expf(xv[i]);
+          expand_table(t, xv, m);
           for (int c = 0; c < K; ++c) acc[c] = fmaf(w, m[c], acc[c]);
 #pragma unroll
           for (int i = 0; i < SB_MAX_DIM; ++i)

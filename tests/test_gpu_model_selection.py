@@ -47,7 +47,7 @@ def reference(nat, x0, W, lib, dt, spr, y, method):
     return torch.stack(out)
 
 
-# the specialised shapes of SB_ROLL_SHAPES, config 3's (2, 2) + exp, and two runtime-table libraries
+# the specialised shapes of SB_SPEC_SHAPES (config 3's (2, 2) + exp among them) and two runtime-table libraries
 LIBS = [(2, 2, 0, 0), (2, 3, 0, 0), (3, 2, 0, 0), (3, 3, 0, 0), (3, 5, 0, 0), (2, 2, 0, 1), (2, 2, 1, 0), (4, 2, 0, 0)]
 
 
