@@ -273,6 +273,24 @@ int sb_rollout_score(const float* x0, int64_t n_ics, const sb_library* lib, cons
                      int64_t steps_per_row, int64_t n_rows, int method, const float* y_obs, float blowup,
                      double* sse, int32_t* valid_rows, void* stream);
 
+/* Gradient of the fused scores (trajectory refit of the candidates): with the arguments of sb_rollout_score, sse and
+ * valid_rows are bit-identical to what sb_rollout_score returns, and grad (n_models × d × K fp64) = ∂/∂W_m of
+ * Σ_n sse[m, n], the SSE as reported: a pair that stopped after valid_rows[m, n] = v rows contributes the gradient of its
+ * sum over rows 1..v (nothing for v = 0). It is the discrete adjoint of the fp32 recurrence that was scored (same step,
+ * same right-hand side), so it is exact up to fp32 rounding of the reverse sweep; the per-thread sums are added in fp64
+ * every 32 steps. No atomics on values: a model's gradient has the same bits alone, in any batch, in any model order and
+ * on every repeat (it may change in the last bits when the ICs are split into different batches).
+ * ws: device workspace of at least sb_rollout_score_grad_workspace_bytes(n_ics, lib, n_models, steps_per_row, n_rows)
+ * bytes (the state every 32 steps of every pair, fp32, and one fp64 d×K row per model and block of 64 ICs); it need not
+ * be initialised. SB_ERR_WORKSPACE if it is shorter; otherwise the status codes of sb_rollout_score, and NULL grad or ws
+ * is SB_ERR_INVALID. n_ics = 0 sets grad to 0. The workspace size is negative (a status) for invalid sizes. */
+int64_t sb_rollout_score_grad_workspace_bytes(int64_t n_ics, const sb_library* lib, int n_models,
+                                              int64_t steps_per_row, int64_t n_rows);
+int sb_rollout_score_grad(const float* x0, int64_t n_ics, const sb_library* lib, const float* w, int n_models,
+                          double dt, int64_t steps_per_row, int64_t n_rows, int method, const float* y_obs,
+                          float blowup, double* sse, int32_t* valid_rows, double* grad, void* ws, int64_t ws_bytes,
+                          void* stream);
+
 /* WSINDy weak-form integrals with trigonometric test functions (`sindy.py:332-347,361-362`):
  *   V[j,t]  = dt·sqrt(2/T)·sin((j+1)π t/T),  V'[j,t] = dt·sqrt(2/T)·(j+1)π/T·cos((j+1)π t/T),  t = t_idx·dt
  *   G[traj,j,k] = sum_t V[j,t]·Θ_k(x[traj,t]),   b[traj,j,i] = −sum_t V'[j,t]·x[traj,t,i]

@@ -166,6 +166,38 @@ __device__ __forceinline__ void expand_table(const LibTab& t, const T* x, T* m) 
   if (t.exp_) for (int j = 0; j < t.d; ++j) m[k++] = exp(x[j]);
 }
 
+// Value-only reverse sweep of expand_lib: xb += J_Θ(x)ᵀ·mb for the cotangent mb on Θ(x) (consumed: the parents' entries
+// receive their children's contributions). m = Θ(x). m_k = m_p·x_v gives mb_p += mb_k·x_v and xb_v += mb_k·m_p.
+template <int D, int PC, class T>
+__device__ __forceinline__ void reverse_lib(const T (&x)[D], const T (&m)[LibCode<D, PC>::K],
+                                            T (&mb)[LibCode<D, PC>::K], T (&xb)[D]) {
+  using L = LibCode<D, PC>;
+  using Tab = Poly<D, L::P>;
+  constexpr int NP = L::NP;
+  if constexpr (L::S) static_for<0, D>([&](auto j) { xb[j] = fma(mb[NP + j], cos(x[j]), xb[j]); });
+  if constexpr (L::E) static_for<0, D>([&](auto j) { xb[j] = fma(mb[NP + D * L::S + j], m[NP + D * L::S + j], xb[j]); });
+  static_for<0, NP - 1 - D>([&](auto qc) {
+    constexpr int k = NP - 1 - qc;  // NP-1 down to D+1
+    constexpr int p = Tab::tab.parent[k], v = Tab::tab.var[k];
+    mb[p] = fma(mb[k], x[v], mb[p]);
+    xb[v] = fma(mb[k], m[p], xb[v]);
+  });
+  static_for<0, D>([&](auto j) { xb[j] += mb[1 + j]; });
+}
+// the same sweep over a runtime table; m, mb hold t.K values, x, xb t.d
+template <class T>
+__device__ __forceinline__ void reverse_table(const LibTab& t, const T* x, const T* m, T* mb, T* xb) {
+  int k = t.n_poly;
+  if (t.sine) for (int j = 0; j < t.d; ++j, ++k) xb[j] = fma(mb[k], cos(x[j]), xb[j]);
+  if (t.exp_) for (int j = 0; j < t.d; ++j, ++k) xb[j] = fma(mb[k], m[k], xb[j]);
+  for (k = t.n_poly - 1; k > t.d; --k) {
+    const int p = t.parent[k], v = t.var[k];
+    mb[p] = fma(mb[k], x[v], mb[p]);
+    xb[v] = fma(mb[k], m[p], xb[v]);
+  }
+  for (int j = 0; j < t.d; ++j) xb[j] += mb[1 + j];
+}
+
 // ---------------------------------------------------------------------------------------------
 // reductions
 // ---------------------------------------------------------------------------------------------
@@ -306,6 +338,13 @@ int rollout(const void* x0, int64_t n_ics, const LibTab& t, const void* w, doubl
 int rollout_score(const float* x0, int64_t n_ics, const LibTab& t, const float* w, int n_models, double dt,
                   int64_t steps_per_row, int64_t n_rows, int method, const float* y_obs, float blowup, double* sse,
                   int32_t* valid_rows, cudaStream_t s);
+// the same scores and ∂/∂W_m Σ_n sse[m, n] by the discrete adjoint of the scored recurrence; arguments validated by the
+// caller. The workspace size is -1 when it does not fit in int64.
+int64_t rollout_score_grad_workspace_bytes(int64_t n_ics, const LibTab& t, int n_models, int64_t steps_per_row,
+                                           int64_t n_rows);
+int rollout_score_grad(const float* x0, int64_t n_ics, const LibTab& t, const float* w, int n_models, double dt,
+                       int64_t steps_per_row, int64_t n_rows, int method, const float* y_obs, float blowup, double* sse,
+                       int32_t* valid_rows, double* grad, void* ws, int64_t ws_bytes, cudaStream_t s);
 
 // WSINDy integrals
 int wsindy_integrals(const float* x, int64_t n_traj, int64_t T, const LibTab& t, float dt, double t_max,

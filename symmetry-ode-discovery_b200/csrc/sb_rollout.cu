@@ -1,5 +1,6 @@
 // sb_rollout.cu — lock-step fixed-step integration of dx/dt = Θ(x)·Wᵀ for a batch of initial conditions (sb_rollout),
-// and M models × N initial conditions integrated and scored against observed rows in one launch (sb_rollout_score).
+// M models × N initial conditions integrated and scored against observed rows in one launch (sb_rollout_score), and
+// the gradient of those scores with respect to every model's W by the discrete adjoint (sb_rollout_score_grad).
 //
 // Two reference functions share the rollout kernels:
 //   * `model_utils.py:223-255` odeint(f, x0, t, dt, method, full_traj): torch fp32, Euler or classic RK4,
@@ -493,6 +494,295 @@ __global__ void __launch_bounds__(kThreads) rollout_score_gen_kernel(LibTab t, i
   a.valid[model * a.n_ics + ic] = (int32_t)valid;
 }
 
+// ---- gradient of the scores -----------------------------------------------------------------------------------------
+// ∂/∂W_m Σ_n sse[m, n] by the discrete adjoint of the fp32 recurrence the scorer executes. One thread owns one (model,
+// IC) pair; grid = (IC blocks, models), W staged per block as the scorer stages it.
+//   forward:  the scorer's loop (same step, same right-hand side, same row test), so sse / valid are its bits; the state
+//             at every step c·kCkpt is stored to the workspace, [checkpoint][model][ic][d].
+//   backward: the pair's objective ends at step S = valid·steps_per_row. Segments [c·kCkpt, (c+1)·kCkpt) ∩ [0, S) are
+//             walked last to first: the segment's step-start states are recomputed from its checkpoint into a
+//             per-thread array, then each step is reversed, its stages recomputed from its step-start state (nothing is
+//             stored per stage). RK4, x' = x + sdt·(((k1 + 2k2) + 2k3) + k4), k_s = h(y_s): with a = sdt·λ,
+//             k̄4 = a, k̄3 = k̄2 = 2a, k̄1 = a; for s = 4..1, ȳ_s = J_h(y_s)ᵀk̄_s and W̄ += k̄_s ⊗ Θ(y_s), ȳ_s enters λ and
+//             k̄_{s−1} (times dt, hdt, hdt). Every compared row adds 2(x_r − y_r) to λ. Euler is the one-stage case.
+//   sums:     W̄ in d·K fp32 registers per thread, added to an fp64 row per warp in shared memory at every segment end
+//             (a warp-shuffle sum in fixed order), so an fp32 sum spans at most kCkpt steps; the warps' rows are added in
+//             warp order into one fp64 partial row per (model, IC block), and grad_sum_kernel adds those in block order.
+// Nothing depends on which other models share the launch: a model's gradient has the same bits alone, in any batch and
+// any model order, on every repeat (not across IC batch splits, which regroup the sums).
+constexpr int kCkpt = 32;             // checkpoint interval: kCkpt + 1 states per thread in local memory
+constexpr int kGradThreads = kMultiThreads;
+constexpr int kGradWarps = kGradThreads / 32;
+
+struct GradArgs {
+  ScoreArgs s;         // this launch's models, as the scorer gets them
+  int64_t n_models;    // models of the whole call (checkpoint layout)
+  int64_t model0;      // first model of this launch
+  float* ckpt;         // [checkpoint][model][ic][d]
+  double* partial;     // [model][IC block][d·K], from this launch's first model
+};
+
+// specialised library: W from the block-staged shared copy (SharedW rows of KQ float4)
+template <int D, int PC>
+struct SpecGrad {
+  static constexpr bool kStatic = true;
+  static constexpr int DN = D, K = LibCode<D, PC>::K, ACC = D * K, KQ = SharedW<K>::KQ;
+  const float4* sw;
+  __device__ __forceinline__ int dim() const { return D; }
+  __device__ __forceinline__ int dk() const { return D * K; }
+  __device__ __forceinline__ void eval(const float (&y)[D], float (&k)[D], int off) const {
+    eval_pairs<D, PC, 1>(SharedW<K>{sw + off}, reinterpret_cast<const float (&)[1][D]>(y),
+                         reinterpret_cast<float (&)[1][D]>(k));
+  }
+  // xb = J_h(y)ᵀu = J_Θ(y)ᵀ(Wᵀu);  acc += u ⊗ Θ(y)
+  __device__ __forceinline__ void vjp(const float (&y)[D], const float (&u)[D], float (&xb)[D], float (&acc)[ACC],
+                                      int off) const {
+    const float* w = reinterpret_cast<const float*>(sw + off);
+    float m[K], mb[K];
+    expand_lib<D, PC>(y, m);
+    static_for<0, K>([&](auto kc) {
+      constexpr int k = kc;
+      float s = 0.f;
+      static_for<0, D>([&](auto ic) {
+        constexpr int i = ic;
+        s = fmaf(w[i * KQ * 4 + k], u[i], s);
+        acc[i * K + k] = fmaf(u[i], m[k], acc[i * K + k]);
+      });
+      mb[k] = s;
+    });
+    static_for<0, D>([&](auto j) { xb[j] = 0.f; });
+    reverse_lib<D, PC>(y, m, mb, xb);
+  }
+};
+
+// runtime-table library: GenRhs with the model's W in global memory
+template <int KMAX>
+struct GenGrad {
+  static constexpr bool kStatic = false;
+  static constexpr int DN = SB_MAX_DIM, ACC = SB_MAX_DIM * KMAX;
+  const LibTab& t;
+  const float* w;
+  __device__ __forceinline__ int dim() const { return t.d; }
+  __device__ __forceinline__ int dk() const { return t.d * t.K; }
+  __device__ __forceinline__ void eval(const float (&y)[DN], float (&k)[DN], int) const {
+    GenRhs<float, KMAX>{t, w}.eval(y, k);
+  }
+  __device__ __forceinline__ void vjp(const float (&y)[DN], const float (&u)[DN], float (&xb)[DN], float (&acc)[ACC],
+                                      int) const {
+    float m[KMAX], mb[KMAX];
+    expand_table(t, y, m);
+    for (int k = 0; k < t.K; ++k) {
+      float s = 0.f;
+      for (int i = 0; i < t.d; ++i) {
+        s = fmaf(__ldg(w + i * t.K + k), u[i], s);
+        acc[i * t.K + k] = fmaf(u[i], m[k], acc[i * t.K + k]);
+      }
+      mb[k] = s;
+    }
+#pragma unroll
+    for (int j = 0; j < DN; ++j) xb[j] = 0.f;
+    reverse_table(t, y, m, mb, xb);
+  }
+};
+
+__device__ __forceinline__ int64_t warp_max(int64_t v) {
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) {
+    const int64_t u = __shfl_xor_sync(0xffffffffu, (long long)v, o);
+    v = u > v ? u : v;
+  }
+  return v;
+}
+
+// every thread of the block takes part (warp shuffles, block barrier), including those past the last IC
+template <class G>
+__device__ __forceinline__ void grad_body(const G& g, int method, const GradArgs& a, double* sacc) {
+  constexpr int DN = G::DN;
+  const int d = g.dim(), dk = g.dk();
+  const ScoreArgs& sa = a.s;
+  const int64_t model = blockIdx.y, N = sa.n_ics, spr = sa.steps_per_row;
+  const int64_t ic = (int64_t)blockIdx.x * kGradThreads + threadIdx.x;
+  const bool live = ic < N;
+  const int64_t ck_stride = a.n_models * N * d;
+  float* ck = a.ckpt + ((a.model0 + model) * N + (live ? ic : 0)) * d;
+  const Odeint<float> ode(sa.dt);
+  auto step = [&](float (&x)[1][DN], int64_t s) {
+    ode.step(method, x, [&](const auto& y, auto& k, int st) { g.eval(y[0], k[0], (int)((s + st) & sa.opaque)); });
+  };
+
+  // ---- forward: the scorer's loop, with checkpoints ----
+  float x[1][DN];
+#pragma unroll
+  for (int j = 0; j < DN; ++j) x[0][j] = (live && j < d) ? sa.x0[ic * d + j] : 0.f;
+  int64_t valid = 0;
+  if (live) {
+    double sse = 0.0;
+    valid = sa.n_rows;
+    int64_t row = 0, until = spr, tock = 0, c = 0;
+    for (int64_t s = 1;; ++s) {
+      if (tock == 0) {                              // the state after step s − 1 = c·kCkpt
+#pragma unroll
+        for (int j = 0; j < DN; ++j)
+          if (j < d) ck[c * ck_stride + j] = x[0][j];
+        ++c;
+        tock = kCkpt;
+      }
+      --tock;
+      step(x, s);
+      if (--until == 0) {
+        if (!score_row<DN>(x[0], d, sa.y_obs + (row * N + ic) * d, sa.blowup, sse)) { valid = row; break; }
+        if (++row == sa.n_rows) break;
+        until = spr;
+      }
+    }
+    sa.sse[model * N + ic] = sse;
+    sa.valid[model * N + ic] = (int32_t)valid;
+  }
+
+  // ---- backward over the segments of [0, S) ----
+  const int64_t S = valid * spr;
+  const int64_t n_seg = warp_max((S + kCkpt - 1) / kCkpt);
+  float acc[G::ACC];
+  if constexpr (G::kStatic) static_for<0, G::ACC>([&](auto e) { acc[e] = 0.f; });
+  else for (int e = 0; e < dk; ++e) acc[e] = 0.f;
+  float lam[DN];
+#pragma unroll
+  for (int j = 0; j < DN; ++j) lam[j] = 0.f;
+  float seg[kCkpt + 1][DN];
+  double* mine = sacc + (threadIdx.x >> 5) * G::ACC;
+  const bool lane0 = (threadIdx.x & 31) == 0;
+  for (int64_t c = n_seg - 1; c >= 0; --c) {
+    const int64_t s0 = c * kCkpt;
+    const int n = S > s0 ? (int)(S - s0 < kCkpt ? S - s0 : kCkpt) : 0;
+    if (n > 0) {
+#pragma unroll
+      for (int j = 0; j < DN; ++j) x[0][j] = j < d ? ck[c * ck_stride + j] : 0.f;
+#pragma unroll
+      for (int j = 0; j < DN; ++j) seg[0][j] = x[0][j];
+      for (int q = 1; q <= n; ++q) {
+        step(x, s0 + q);
+#pragma unroll
+        for (int j = 0; j < DN; ++j) seg[q][j] = x[0][j];
+      }
+      int64_t r_until = (s0 + n) % spr, row = (s0 + n) / spr;   // steps back to the next compared row, its number
+      for (int q = n; q >= 1; --q) {
+        if (r_until == 0) {                          // λ += ∂/∂x_s of ‖x_s − y_row‖²
+          const float* y = sa.y_obs + ((row - 1) * N + ic) * d;
+#pragma unroll
+          for (int j = 0; j < DN; ++j)
+            if (j < d) lam[j] += 2.f * (seg[q][j] - __ldg(y + j));
+          --row;
+          r_until = spr;
+        }
+        --r_until;
+        const int off = (int)((s0 + q) & sa.opaque);
+        float y1[DN];
+#pragma unroll
+        for (int j = 0; j < DN; ++j) y1[j] = seg[q - 1][j];
+        float xb[DN];
+        if (method == SB_EULER) {
+          float u[DN];
+#pragma unroll
+          for (int j = 0; j < DN; ++j) u[j] = ode.dt * lam[j];
+          g.vjp(y1, u, xb, acc, off);
+#pragma unroll
+          for (int j = 0; j < DN; ++j) lam[j] += xb[j];
+          continue;
+        }
+        // the stages y_1..y_4 of Odeint::step, recomputed bit for bit
+        float ys[4][DN], k[DN];
+#pragma unroll
+        for (int j = 0; j < DN; ++j) ys[0][j] = y1[j];
+        g.eval(y1, k, off);
+#pragma unroll
+        for (int j = 0; j < DN; ++j) ys[1][j] = add_rn(y1[j], mul_rn(ode.hdt, k[j]));
+        g.eval(ys[1], k, off);
+#pragma unroll
+        for (int j = 0; j < DN; ++j) ys[2][j] = add_rn(y1[j], mul_rn(ode.hdt, k[j]));
+        g.eval(ys[2], k, off);
+#pragma unroll
+        for (int j = 0; j < DN; ++j) ys[3][j] = add_rn(y1[j], mul_rn(ode.dt, k[j]));
+        float av[DN];
+#pragma unroll
+        for (int j = 0; j < DN; ++j) { av[j] = ode.sdt * lam[j]; k[j] = av[j]; }   // k̄4 = sdt·λ
+        // one copy of the stage sweep: a library's vjp inlined four times does not fit the register file at d·K = 168
+#pragma unroll 1
+        for (int st = 3; st >= 0; --st) {
+          float ysd[DN];
+#pragma unroll
+          for (int j = 0; j < DN; ++j) ysd[j] = ys[st][j];
+          g.vjp(ysd, k, xb, acc, off);
+          const float route = st == 3 ? ode.dt : ode.hdt, base = st == 1 ? 1.f : 2.f;
+#pragma unroll
+          for (int j = 0; j < DN; ++j) { lam[j] += xb[j]; k[j] = base * av[j] + route * xb[j]; }   // k̄_{st}
+        }
+      }
+    }
+    // segment end: fp32 sums into the warp's fp64 row
+    if constexpr (G::kStatic) {
+      static_for<0, G::ACC>([&](auto e) {
+        const double v = warp_sum((double)acc[e]);
+        if (lane0) mine[e] += v;
+        acc[e] = 0.f;
+      });
+    } else {
+      for (int e = 0; e < dk; ++e) {
+        const double v = warp_sum((double)acc[e]);
+        if (lane0) mine[e] += v;
+        acc[e] = 0.f;
+      }
+    }
+  }
+  __syncthreads();
+  double* part = a.partial + (model * gridDim.x + blockIdx.x) * dk;
+  for (int e = threadIdx.x; e < dk; e += kGradThreads) {
+    double v = 0.0;
+#pragma unroll
+    for (int w = 0; w < kGradWarps; ++w) v += sacc[w * G::ACC + e];
+    part[e] = v;
+  }
+}
+
+template <int D, int PC, int METHOD>
+__global__ void __launch_bounds__(kGradThreads) rollout_grad_spec_kernel(GradArgs a) {
+  using G = SpecGrad<D, PC>;
+  constexpr int K = G::K, KQ = G::KQ;
+  __shared__ float4 sw[D * KQ];
+  __shared__ double sacc[kGradWarps * G::ACC];
+  {
+    const float* wm = a.s.w + (int64_t)blockIdx.y * (D * K);
+    float* s = reinterpret_cast<float*>(sw);
+    for (int q = threadIdx.x; q < D * KQ * 4; q += kGradThreads) {
+      const int i = q / (KQ * 4), c = q % (KQ * 4);
+      s[q] = c < K ? wm[i * K + c] : 0.f;
+    }
+    for (int q = threadIdx.x; q < kGradWarps * G::ACC; q += kGradThreads) sacc[q] = 0.0;
+  }
+  __syncthreads();
+  grad_body(G{sw}, METHOD, a, sacc);
+}
+
+template <int KMAX>
+__global__ void __launch_bounds__(kGradThreads) rollout_grad_gen_kernel(LibTab t, int method, GradArgs a) {
+  using G = GenGrad<KMAX>;
+  __shared__ double sacc[kGradWarps * G::ACC];
+  for (int q = threadIdx.x; q < kGradWarps * G::ACC; q += kGradThreads) sacc[q] = 0.0;
+  __syncthreads();
+  grad_body(G{t, a.s.w + (int64_t)blockIdx.y * t.d * t.K}, method, a, sacc);
+}
+
+// grad[m, e] = Σ_b partial[m, b, e] in block order
+__global__ void __launch_bounds__(256) grad_sum_kernel(const double* partial, int64_t n_blocks, int dk, int64_t n,
+                                                       double* grad) {
+  const int64_t i = (int64_t)blockIdx.x * 256 + threadIdx.x;
+  if (i >= n) return;
+  const int64_t m = i / dk, e = i % dk;
+  const double* p = partial + m * n_blocks * dk + e;
+  double v = 0.0;
+  for (int64_t b = 0; b < n_blocks; ++b) v += p[b * dk];
+  grad[i] = v;
+}
+
 // ---- launch ---------------------------------------------------------------------------------------------------------
 // The specialised libraries as (D, library code PC): the polynomials and, for config 3 (Lotka-Volterra in canonical
 // coordinates, `data_utils/lotka.py:33-41`), degree 2 + exp. Everything else runs on the runtime table.
@@ -559,7 +849,96 @@ int launch_score(const LibTab& t, const ScoreArgs& a, int method, int n_models, 
   return SB_OK;
 }
 
+int64_t grad_blocks(int64_t n_ics) { return (n_ics + kGradThreads - 1) / kGradThreads; }
+
+template <int D, int PC>
+int launch_grad_spec(const GradArgs& a, int method, int n_models, cudaStream_t s) {
+  const dim3 grid((unsigned)grad_blocks(a.s.n_ics), (unsigned)n_models);
+  if (method == SB_EULER) rollout_grad_spec_kernel<D, PC, SB_EULER><<<grid, kGradThreads, 0, s>>>(a);
+  else rollout_grad_spec_kernel<D, PC, SB_RK4><<<grid, kGradThreads, 0, s>>>(a);
+  SB_LAUNCH_CHECK("rollout_grad_spec_kernel");
+  return SB_OK;
+}
+
+int launch_grad(const LibTab& t, const GradArgs& a, int method, int n_models, cudaStream_t s) {
+#define X(D, PC) \
+  if (lib_matches<D, PC>(t)) return launch_grad_spec<D, PC>(a, method, n_models, s);
+  SB_SPEC_SHAPES(X)
+#undef X
+  const dim3 grid((unsigned)grad_blocks(a.s.n_ics), (unsigned)n_models);
+  if (t.K <= 16) rollout_grad_gen_kernel<16><<<grid, kGradThreads, 0, s>>>(t, method, a);
+  else if (t.K <= 64) rollout_grad_gen_kernel<64><<<grid, kGradThreads, 0, s>>>(t, method, a);
+  else rollout_grad_gen_kernel<256><<<grid, kGradThreads, 0, s>>>(t, method, a);
+  SB_LAUNCH_CHECK("rollout_grad_gen_kernel");
+  return SB_OK;
+}
+
+// workspace: [partial rows: n_models × IC blocks × d·K fp64, padded to 256 bytes][checkpoints: n_ckpt × n_models ×
+// n_ics × d fp32], n_ckpt = ⌈n_rows·steps_per_row / kCkpt⌉
+struct GradLayout {
+  int64_t partial_bytes, ckpt_bytes;
+};
+bool grad_layout(int64_t n_ics, const LibTab& t, int n_models, int64_t steps_per_row, int64_t n_rows, GradLayout* L) {
+  int64_t steps, rows_el, part, ck;
+  if (__builtin_mul_overflow(n_rows, steps_per_row, &steps)) return false;
+  const int64_t n_ckpt = (steps - 1) / kCkpt + 1;
+  if (__builtin_mul_overflow(grad_blocks(n_ics), (int64_t)n_models, &part)) return false;
+  if (__builtin_mul_overflow(part, (int64_t)(t.d * t.K) * 8, &part)) return false;
+  if (__builtin_mul_overflow((int64_t)n_models * n_ics, (int64_t)t.d * 4, &rows_el)) return false;
+  if (__builtin_mul_overflow(rows_el, n_ckpt, &ck)) return false;
+  part = (part + 255) / 256 * 256;
+  if (part > INT64_MAX - ck) return false;
+  L->partial_bytes = part;
+  L->ckpt_bytes = ck;
+  return true;
+}
+
 }  // namespace
+
+int64_t rollout_score_grad_workspace_bytes(int64_t n_ics, const LibTab& t, int n_models, int64_t steps_per_row,
+                                           int64_t n_rows) {
+  GradLayout L;
+  if (!grad_layout(n_ics, t, n_models, steps_per_row, n_rows, &L)) return -1;
+  return L.partial_bytes + L.ckpt_bytes;
+}
+
+int rollout_score_grad(const float* x0, int64_t n_ics, const LibTab& t, const float* w, int n_models, double dt,
+                       int64_t steps_per_row, int64_t n_rows, int method, const float* y_obs, float blowup, double* sse,
+                       int32_t* valid_rows, double* grad, void* ws, int64_t ws_bytes, cudaStream_t s) {
+  GradLayout L;
+  if (!grad_layout(n_ics, t, n_models, steps_per_row, n_rows, &L)) {
+    set_error("rollout_score_grad workspace size overflows int64");
+    return SB_ERR_INVALID;
+  }
+  if (ws_bytes < L.partial_bytes + L.ckpt_bytes) {
+    set_error("workspace too small: %lld < %lld bytes", (long long)ws_bytes,
+              (long long)(L.partial_bytes + L.ckpt_bytes));
+    return SB_ERR_WORKSPACE;
+  }
+  const int dk = t.d * t.K;
+  const int64_t nblk = grad_blocks(n_ics);
+  double* partial = reinterpret_cast<double*>(ws);
+  GradArgs a{};
+  a.s.x0 = x0; a.s.n_ics = n_ics; a.s.dt = dt; a.s.steps_per_row = steps_per_row; a.s.n_rows = n_rows;
+  a.s.y_obs = y_obs; a.s.blowup = blowup; a.s.opaque = 0;
+  a.n_models = n_models;
+  a.ckpt = reinterpret_cast<float*>(reinterpret_cast<char*>(ws) + L.partial_bytes);
+  // more models than gridDim.y allows: further launches on the same stream
+  for (int m0 = 0; m0 < n_models; m0 += kMaxGridY) {
+    const int nm = n_models - m0 < kMaxGridY ? n_models - m0 : kMaxGridY;
+    a.s.w = w + (int64_t)m0 * dk;
+    a.s.sse = sse + (int64_t)m0 * n_ics;
+    a.s.valid = valid_rows + (int64_t)m0 * n_ics;
+    a.model0 = m0;
+    a.partial = partial + (int64_t)m0 * nblk * dk;
+    const int st = launch_grad(t, a, method, nm, s);
+    if (st != SB_OK) return st;
+  }
+  const int64_t n = (int64_t)n_models * dk;
+  grad_sum_kernel<<<(unsigned)((n + 255) / 256), 256, 0, s>>>(partial, nblk, dk, n, grad);
+  SB_LAUNCH_CHECK("grad_sum_kernel");
+  return SB_OK;
+}
 
 int rollout(const void* x0, int64_t n_ics, const LibTab& t, const void* w, double dt, int64_t n_steps,
             int64_t stride, int method, int dtype, int record_dx, void* x_out, void* dx_out, void* x_last,

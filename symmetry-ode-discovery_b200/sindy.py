@@ -28,7 +28,7 @@ from sindy_b200 import native, ops
 from sindy_b200.native import Library
 
 __all__ = ["SINDyRegression", "solve_SINDy_one_step", "solve_SINDy", "WSINDyWrapper", "stlsq_statistics",
-           "allreduce_statistics", "stlsq_path", "score_path", "information_criteria", "apply_candidate", "SINDyConst", "SINDyPoly1", "SINDyPoly2", "SINDyPoly3", "SINDySine", "SINDyExp"]
+           "allreduce_statistics", "stlsq_path", "score_path", "refine_path", "information_criteria", "apply_candidate", "SINDyConst", "SINDyPoly1", "SINDyPoly2", "SINDyPoly3", "SINDySine", "SINDyExp"]
 
 
 # ---- the reference's per-block library functions (`sindy.py:7-30`) --------------------------------------------------
@@ -651,23 +651,8 @@ def score_path(library, path, x_val, dt, steps_per_row=1, method='rk4', blowup=N
         raise ValueError(f"library must be a native.Library or a SINDyRegression, got {type(library).__name__}")
     if criterion not in ('aic', 'aicc', 'bic'):
         raise ValueError(f"criterion must be 'aic', 'aicc' or 'bic', got {criterion!r}")
-    if method not in ('euler', 'rk4'):
-        raise ValueError(f"method must be 'euler' or 'rk4', got {method!r}")
-    if isinstance(steps_per_row, bool) or not isinstance(steps_per_row, (int, np.integer)) or steps_per_row < 1:
-        raise ValueError(f"steps_per_row must be a positive integer, got {steps_per_row!r}")
-    dt = float(dt)
-    if not (math.isfinite(dt) and dt > 0):
-        raise ValueError(f"dt must be positive, got {dt}")
-    if blowup is not None and not (math.isfinite(float(blowup)) and float(blowup) > 0):
-        raise ValueError(f"blowup must be a positive number or None, got {blowup!r}")
-    x_val = torch.as_tensor(x_val)
-    if x_val.dim() != 3 or x_val.shape[-1] != lib.dim:
-        raise ValueError(f"x_val must be (n_traj, T, {lib.dim}), got {tuple(x_val.shape)}")
+    x_val, dt = _check_rollout_args(lib, x_val, "x_val", dt, steps_per_row, method, blowup)
     n_traj, T, d = x_val.shape
-    if T < 2 or n_traj < 1:
-        raise ValueError(f"x_val needs at least one trajectory of T >= 2 rows, got {tuple(x_val.shape)}")
-    if not bool(torch.isfinite(x_val).all()):
-        raise ValueError("x_val has non-finite values")
     W, masks = path["xi"], path["mask"]
     if W.dim() != 3 or W.shape[1:] != (d, lib.K) or masks.shape != W.shape:
         raise ValueError(f"path['xi'] / path['mask'] must be (P, {d}, {lib.K}), got {tuple(W.shape)} / "
@@ -691,6 +676,152 @@ def score_path(library, path, x_val, dt, steps_per_row=1, method='rk4', blowup=N
     c = crit[criterion].numpy()
     order = np.lexsort((-thr.numpy(), k.numpy(), c))                      # last key sorts first
     out["chosen"] = int(order[0]) if c[order[0]] < math.inf else None
+    return out
+
+
+def _check_rollout_args(lib, x, name, dt, steps_per_row, method, blowup):
+    """The checks score_path and refine_path share; returns (x as a tensor, dt)."""
+    if method not in ('euler', 'rk4'):
+        raise ValueError(f"method must be 'euler' or 'rk4', got {method!r}")
+    if isinstance(steps_per_row, bool) or not isinstance(steps_per_row, (int, np.integer)) or steps_per_row < 1:
+        raise ValueError(f"steps_per_row must be a positive integer, got {steps_per_row!r}")
+    dt = float(dt)
+    if not (math.isfinite(dt) and dt > 0):
+        raise ValueError(f"dt must be positive, got {dt}")
+    if blowup is not None and not (math.isfinite(float(blowup)) and float(blowup) > 0):
+        raise ValueError(f"blowup must be a positive number or None, got {blowup!r}")
+    x = torch.as_tensor(x)
+    if x.dim() != 3 or x.shape[-1] != lib.dim:
+        raise ValueError(f"{name} must be (n_traj, T, {lib.dim}), got {tuple(x.shape)}")
+    if x.shape[1] < 2 or x.shape[0] < 1:
+        raise ValueError(f"{name} needs at least one trajectory of T >= 2 rows, got {tuple(x.shape)}")
+    if not bool(torch.isfinite(x).all()):
+        raise ValueError(f"{name} has non-finite values")
+    return x, dt
+
+
+def refine_path(regressor, path, x_fit, dt, steps_per_row=1, method='rk4', blowup=None, max_iter=50, tol=1e-7):
+    """Trajectory refit of the candidates of `stlsq_path` / `WSINDyWrapper.solve_path`: every distinct candidate's
+    coefficients are refit on its own support by minimising the simulation error on the fitting trajectories,
+      loss = SSE / n_obs of the rollouts from x_fit[:, 0] (step dt) against rows 1..T−1, n_obs = n_traj·(T−1)·d,
+    the objective `score_path` ranks by. Derivative regression leaves a bias that grows with the noise of the smoothed
+    derivatives; this refit judges a support by its best coefficients rather than by the ones regression gave it.
+
+    All candidates advance together: one `native.rollout_score_grad` launch gives every loss and gradient (discrete
+    adjoint of the fp32 rollout), the L-BFGS direction is `sweep.BatchedLBFGS.direction` over the candidate axis, and a
+    per-candidate backtracking (Armijo) line search evaluates the trial points of every candidate still searching in one
+    `native.rollout_score` launch; a trial that diverges (fewer rows than T−1 compared) counts as +inf. A candidate stops
+    after max_iter iterations, when its loss falls by less than tol·loss, or when no step length decreases it; its best
+    iterate is kept, so sse_after <= sse_before. Masks are fixed: dead coefficients stay exactly 0. An
+    equivariance-constrained regressor is refit in its parameters (β, const), vec(Ξ) = A·[β, const], A from
+    `sweep.param_map`, and the returned path carries the new beta / const for `apply_candidate`.
+
+    Returns a copy of `path` with xi refit and sse_before, sse_after (P,) fp64 and iterations (P,) added; a candidate that
+    diverges from the start keeps its coefficients (sse_before = sse_after = +inf)."""
+    import sweep
+    lib = getattr(regressor, 'library', regressor)
+    if not isinstance(lib, Library):
+        raise ValueError(f"regressor must be a SINDyRegression or a native.Library, got {type(regressor).__name__}")
+    constrained = bool(getattr(regressor, 'constraint', False))
+    x_fit, dt = _check_rollout_args(lib, x_fit, "x_fit", dt, steps_per_row, method, blowup)
+    if isinstance(max_iter, bool) or not isinstance(max_iter, (int, np.integer)) or max_iter < 1:
+        raise ValueError(f"max_iter must be a positive integer, got {max_iter!r}")
+    if not (math.isfinite(float(tol)) and float(tol) >= 0):
+        raise ValueError(f"tol must be a non-negative number, got {tol!r}")
+    n_traj, T, d = x_fit.shape
+    W0, masks = path["xi"], path["mask"]
+    if W0.dim() != 3 or W0.shape[1:] != (d, lib.K) or masks.shape != W0.shape:
+        raise ValueError(f"path['xi'] / path['mask'] must be (P, {d}, {lib.K}), got {tuple(W0.shape)} / "
+                         f"{tuple(masks.shape)}")
+    if constrained and ("beta" not in path or "const" not in path):
+        raise ValueError("an equivariance-constrained regressor needs path['beta'] and path['const']")
+    P, dK = W0.shape[0], d * lib.K
+    dev = W0.device
+    xf = x_fit.to(device=dev, dtype=torch.float32)
+    x0, y = xf[:, 0].contiguous(), xf[:, 1:].transpose(0, 1).contiguous()
+    n_obs = n_traj * (T - 1) * d
+    # distinct candidates (coefficients and mask), each refit once
+    key = torch.cat([W0.reshape(P, -1), masks.reshape(P, -1).to(W0.dtype)], 1)
+    _, inverse = torch.unique(key, dim=0, return_inverse=True)
+    U = int(inverse.max()) + 1
+    first = torch.full((U,), P, dtype=torch.long, device=dev).scatter_reduce(0, inverse.to(dev),
+                                                                            torch.arange(P, device=dev), 'amin')
+    mk = masks[first].reshape(U, dK).to(torch.float64)
+    if constrained:
+        A, _ = sweep.param_map(regressor)
+        A = A.to(dev)
+        p = torch.cat([path["beta"][first].reshape(U, -1), path["const"][first].reshape(U, -1)], 1).to(dev, torch.float64)
+    else:
+        A = None
+        p = W0[first].reshape(U, dK).to(torch.float64)
+
+    def W_of(q, m):
+        v = q if A is None else q @ A.T
+        return (v * m).to(torch.float32).view(-1, d, lib.K)
+
+    def loss_grad(q):
+        sse, valid, g = native.rollout_score_grad(x0, W_of(q, mk), lib, dt, int(steps_per_row), y, method, blowup)
+        f = sse.sum(1) / n_obs
+        f = torch.where((valid < T - 1).any(1), torch.full_like(f, math.inf), f)
+        g = g.reshape(-1, dK) * mk / n_obs
+        return f, (g if A is None else g @ A)
+
+    def loss(q, rows):
+        sse, valid = native.rollout_score(x0, W_of(q, mk[rows]), lib, dt, int(steps_per_row), y, method, blowup)
+        f = sse.sum(1) / n_obs
+        return torch.where((valid < T - 1).any(1), torch.full_like(f, math.inf), f)
+
+    with torch.no_grad():
+        f, g = loss_grad(p)
+        f_before = f.clone()
+        opt = sweep.BatchedLBFGS(p, 1.0, history_size=10)
+        iters = torch.zeros(U, dtype=torch.long, device=dev)
+        active = torch.isfinite(f) & (g.abs().amax(1) > 0)
+        c1, max_ls = 1e-4, 30
+        for _ in range(max_iter):
+            if not bool(active.any()):
+                break
+            dirn = opt.direction(g)
+            if A is None:
+                dirn = dirn * mk
+            gtd = (g * dirn).sum(1)
+            restart = gtd >= 0                                       # not a descent direction: steepest descent
+            dirn = torch.where(restart.unsqueeze(1), -g, dirn)
+            gtd = torch.where(restart, -(g * g).sum(1), gtd)
+            t = torch.where(opt.hist == 0, torch.clamp(1.0 / g.abs().sum(1), max=1.0), torch.ones_like(f))
+            searching, accepted = active.clone(), torch.zeros_like(active)
+            for _ls in range(max_ls):
+                idx = torch.nonzero(searching).flatten()
+                if idx.numel() == 0:
+                    break
+                trial = p[idx] + t[idx].unsqueeze(1) * dirn[idx]
+                ft = loss(trial, idx)
+                ok = ft <= f[idx] + c1 * t[idx] * gtd[idx]
+                accepted[idx[ok]] = True
+                searching[idx[ok]] = False
+                t[idx[~ok]] *= 0.5
+            active &= accepted                                        # no step length decreased the loss: done
+            p_new = torch.where(active.unsqueeze(1), p + t.unsqueeze(1) * dirn, p)
+            f_new, g_new = loss_grad(p_new)
+            f_new = torch.where(active, f_new, f)
+            g_new = torch.where(active.unsqueeze(1), g_new, g)
+            sv, yv = p_new - p, g_new - g
+            ys = (sv * yv).sum(1)
+            opt.push(yv, sv, active & (ys > 1e-10), ys)
+            iters += active.long()
+            small = (f - f_new) <= tol * f.abs()
+            p, f, g = p_new, f_new, g_new
+            active &= ~small & (g.abs().amax(1) > 0)
+        out = dict(path)
+        inv = inverse.to(dev)
+        out["xi"] = (W_of(p, mk)[inv] * masks).to(W0.dtype)
+        if constrained:
+            nb = path["beta"].shape[1]
+            out["beta"] = p[inv, :nb].to(path["beta"].dtype)
+            out["const"] = p[inv, nb:].reshape(P, d, 1).to(path["const"].dtype)
+        out["sse_before"] = (f_before * n_obs)[inv].cpu()
+        out["sse_after"] = (f * n_obs)[inv].cpu()
+        out["iterations"] = iters[inv].cpu()
     return out
 
 

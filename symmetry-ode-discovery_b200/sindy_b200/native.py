@@ -73,6 +73,10 @@ _SIGNATURES = {
                            c_int, c_int, c_void_p, c_void_p, c_void_p, c_void_p]),
     "sb_rollout_score": (c_int, [c_void_p, c_int64, POINTER(_CLibrary), c_void_p, c_int, c_double, c_int64, c_int64,
                                  c_int, c_void_p, c_float, c_void_p, c_void_p, c_void_p]),
+    "sb_rollout_score_grad_workspace_bytes": (c_int64, [c_int64, POINTER(_CLibrary), c_int, c_int64, c_int64]),
+    "sb_rollout_score_grad": (c_int, [c_void_p, c_int64, POINTER(_CLibrary), c_void_p, c_int, c_double, c_int64,
+                                      c_int64, c_int, c_void_p, c_float, c_void_p, c_void_p, c_void_p, c_void_p, c_int64,
+                                      c_void_p]),
     "sb_wsindy_integrals": (c_int, [c_void_p, c_int64, c_int64, POINTER(_CLibrary), c_float, c_double, c_int,
                                     c_void_p, c_void_p, c_void_p]),
     "sb_wsindy_local_integrals": (c_int, [c_void_p, c_int64, c_int64, POINTER(_CLibrary), c_void_p, c_void_p, c_int,
@@ -534,13 +538,8 @@ def rollout(x0: torch.Tensor, w: torch.Tensor, lib: Library, dt: float, n_steps:
     return x_out, dx_out, x_last
 
 
-def rollout_score(x0: torch.Tensor, W: torch.Tensor, lib: Library, dt: float, steps_per_row: int, y_obs: torch.Tensor,
-                  method: str = "rk4", blowup: Optional[float] = None) -> Tuple[torch.Tensor, torch.Tensor]:
-    """Every model W[m] (M × d × K, already masked; one d × K model is M = 1) integrated in fp32 from every initial
-    condition x0 (N × d) and compared with y_obs (n_rows × N × d: the states after steps_per_row, 2·steps_per_row, ...
-    steps). Returns sse (M × N fp64, summed over the rows compared) and valid_rows (M × N int32: rows compared before
-    the first non-finite state or |x_j| > blowup; n_rows if none). The compared states are bit-identical to
-    rollout(x0, W[m], lib, dt, n_rows·steps_per_row, stride=steps_per_row, method). See sb_rollout_score."""
+def _score_args(x0, W, lib, dt, steps_per_row, y_obs, method, blowup):
+    """The argument checks and conversions shared by rollout_score and rollout_score_grad."""
     x0f = _flat(_f32c(x0, "x0"), lib.dim, "x0")
     n_ics, d = x0f.shape
     dev = x0f.device
@@ -563,6 +562,18 @@ def rollout_score(x0: torch.Tensor, W: torch.Tensor, lib: Library, dt: float, st
         raise ValueError(f"dt must be positive, got {dt}")
     if blowup is not None and not blowup > 0:
         raise ValueError(f"blowup must be positive or None, got {blowup}")
+    return x0f, W, y, meth, dev
+
+
+def rollout_score(x0: torch.Tensor, W: torch.Tensor, lib: Library, dt: float, steps_per_row: int, y_obs: torch.Tensor,
+                  method: str = "rk4", blowup: Optional[float] = None) -> Tuple[torch.Tensor, torch.Tensor]:
+    """Every model W[m] (M × d × K, already masked; one d × K model is M = 1) integrated in fp32 from every initial
+    condition x0 (N × d) and compared with y_obs (n_rows × N × d: the states after steps_per_row, 2·steps_per_row, ...
+    steps). Returns sse (M × N fp64, summed over the rows compared) and valid_rows (M × N int32: rows compared before
+    the first non-finite state or |x_j| > blowup; n_rows if none). The compared states are bit-identical to
+    rollout(x0, W[m], lib, dt, n_rows·steps_per_row, stride=steps_per_row, method). See sb_rollout_score."""
+    x0f, W, y, meth, dev = _score_args(x0, W, lib, dt, steps_per_row, y_obs, method, blowup)
+    n_ics = x0f.shape[0]
     n_models = W.shape[0]
     sse = torch.empty(n_models, n_ics, dtype=torch.float64, device=dev)
     valid = torch.empty(n_models, n_ics, dtype=torch.int32, device=dev)
@@ -574,6 +585,33 @@ def rollout_score(x0: torch.Tensor, W: torch.Tensor, lib: Library, dt: float, st
                                        0.0 if blowup is None else float(blowup), sse.data_ptr(), valid.data_ptr(),
                                        _stream(dev)), "sb_rollout_score")
     return sse, valid
+
+
+def rollout_score_grad(x0: torch.Tensor, W: torch.Tensor, lib: Library, dt: float, steps_per_row: int,
+                       y_obs: torch.Tensor, method: str = "rk4", blowup: Optional[float] = None):
+    """rollout_score and the gradient of its scores: returns (sse, valid_rows, grad) with sse / valid_rows
+    bit-identical to rollout_score's and grad (M × d × K fp64) = ∂/∂W[m] of sse[m].sum(), each pair's SSE over the rows
+    it compared (discrete adjoint of the fp32 recurrence). See sb_rollout_score_grad."""
+    x0f, W, y, meth, dev = _score_args(x0, W, lib, dt, steps_per_row, y_obs, method, blowup)
+    n_ics, d = x0f.shape
+    n_models = W.shape[0]
+    sse = torch.empty(n_models, n_ics, dtype=torch.float64, device=dev)
+    valid = torch.empty(n_models, n_ics, dtype=torch.int32, device=dev)
+    grad = torch.zeros(n_models, d, lib.K, dtype=torch.float64, device=dev)
+    if n_models == 0 or n_ics == 0:
+        return sse, valid, grad
+    sl = load()
+    nb = int(sl.sb_rollout_score_grad_workspace_bytes(n_ics, ctypes.byref(lib.c()), n_models, int(steps_per_row),
+                                                      y.shape[0]))
+    if nb < 0:
+        _check(nb, "sb_rollout_score_grad_workspace_bytes")
+    ws = torch.empty(max(nb, 1), dtype=torch.uint8, device=dev)
+    with torch.cuda.device(dev):
+        _check(sl.sb_rollout_score_grad(x0f.data_ptr(), n_ics, ctypes.byref(lib.c()), W.data_ptr(), n_models,
+                                        float(dt), int(steps_per_row), y.shape[0], meth, y.data_ptr(),
+                                        0.0 if blowup is None else float(blowup), sse.data_ptr(), valid.data_ptr(),
+                                        grad.data_ptr(), ws.data_ptr(), nb, _stream(dev)), "sb_rollout_score_grad")
+    return sse, valid, grad
 
 
 def wsindy_integrals(x: torch.Tensor, lib: Library, dt: float, t_max: float, n_test: int = 50):

@@ -25,7 +25,7 @@ import torch
 import torch.distributed as dist
 
 __all__ = ["evaluate", "aggregate", "run_seed_sweep", "lbfgs_fit", "BatchedLBFGS", "batched_lbfgs_fits",
-           "run_seed_sweep_batched"]
+           "run_seed_sweep_batched", "param_map"]
 
 
 def evaluate(regressor, truth) -> Dict[str, np.ndarray]:
@@ -161,6 +161,43 @@ class BatchedLBFGS:
         if bool(which.all()):
             self._hist_bound = 0
 
+    def push(self, y: torch.Tensor, sv: torch.Tensor, upd: torch.Tensor, ys: torch.Tensor):
+        """Appends the curvature pair (s = sv, y) with ys = yᵀs to the history of the problems selected by `upd`
+        (dropping their oldest pair when the history is full) and sets their initial Hessian scale to ys / yᵀy."""
+        S = y.shape[0]
+        full = upd & (self.hist == self.H)
+        if self._hist_bound >= self.H and bool(full.any()):       # limited memory: drop the oldest pair
+            self.old_y[full] = torch.roll(self.old_y[full], -1, 1)
+            self.old_s[full] = torch.roll(self.old_s[full], -1, 1)
+            self.ro[full] = torch.roll(self.ro[full], -1, 1)
+            self.hist[full] -= 1
+        pos = self.hist.clamp(max=self.H - 1)
+        u = torch.arange(S, device=y.device)[upd]
+        self.old_y[u, pos[u]] = y[u]
+        self.old_s[u, pos[u]] = sv[u]
+        self.ro[u, pos[u]] = 1.0 / ys[u]
+        self.H_diag = torch.where(upd, ys / (y * y).sum(1).clamp_min(torch.finfo(y.dtype).tiny), self.H_diag)
+        self.hist += upd.long()
+        self._hist_bound = min(self.H, self._hist_bound + 1)
+
+    def direction(self, g: torch.Tensor) -> torch.Tensor:
+        """−H·g for every problem: the two-loop recursion over its stored pairs (entries past a problem's own history
+        count are masked out), with H₀ = H_diag·I."""
+        q = -g
+        al = []
+        for i in range(self._hist_bound - 1, -1, -1):
+            valid = (i < self.hist)
+            a_i = torch.where(valid, (self.old_s[:, i] * q).sum(1) * self.ro[:, i], torch.zeros_like(self.t))
+            q = q - a_i.unsqueeze(1) * self.old_y[:, i]
+            al.append(a_i)
+        al.reverse()
+        r = q * self.H_diag.unsqueeze(1)
+        for i in range(self._hist_bound):
+            valid = (i < self.hist)
+            b_i = (self.old_y[:, i] * r).sum(1) * self.ro[:, i]
+            r = r + torch.where(valid, al[i] - b_i, torch.zeros_like(b_i)).unsqueeze(1) * self.old_s[:, i]
+        return r
+
     @torch.no_grad()
     def step(self, closure, enabled: Optional[torch.Tensor] = None):
         """One `optimizer.step(closure)` for every enabled problem; returns the loss of the first evaluation."""
@@ -170,7 +207,6 @@ class BatchedLBFGS:
         first_loss = loss.clone()
         active = torch.ones(S, dtype=torch.bool, device=x.device) if enabled is None else enabled.clone()
         active &= ~(g.abs().amax(1) <= self.tg)                       # optimal condition before the loop
-        rows = torch.arange(S, device=x.device)
         for it in range(1, self.max_iter + 1):
             self.n_iter += active.long()
             first = active & (self.n_iter == 1)
@@ -179,35 +215,8 @@ class BatchedLBFGS:
             y = g - self.prev_g
             sv = self.d * self.t.unsqueeze(1)
             ys = (y * sv).sum(1)
-            upd = later & (ys > 1e-10)
-            full = upd & (self.hist == self.H)
-            if self._hist_bound >= self.H and bool(full.any()):       # limited memory: drop the oldest pair
-                self.old_y[full] = torch.roll(self.old_y[full], -1, 1)
-                self.old_s[full] = torch.roll(self.old_s[full], -1, 1)
-                self.ro[full] = torch.roll(self.ro[full], -1, 1)
-                self.hist[full] -= 1
-            pos = self.hist.clamp(max=self.H - 1)
-            u = rows[upd]
-            self.old_y[u, pos[u]] = y[u]
-            self.old_s[u, pos[u]] = sv[u]
-            self.ro[u, pos[u]] = 1.0 / ys[u]
-            self.H_diag = torch.where(upd, ys / (y * y).sum(1).clamp_min(torch.finfo(x.dtype).tiny), self.H_diag)
-            self.hist += upd.long()
-            self._hist_bound = min(self.H, self._hist_bound + 1)
-            q = -g
-            al = []
-            for i in range(self._hist_bound - 1, -1, -1):
-                valid = (i < self.hist)
-                a_i = torch.where(valid, (self.old_s[:, i] * q).sum(1) * self.ro[:, i], torch.zeros_like(self.t))
-                q = q - a_i.unsqueeze(1) * self.old_y[:, i]
-                al.append(a_i)
-            al.reverse()
-            r = q * self.H_diag.unsqueeze(1)
-            for i in range(self._hist_bound):
-                valid = (i < self.hist)
-                b_i = (self.old_y[:, i] * r).sum(1) * self.ro[:, i]
-                r = r + torch.where(valid, al[i] - b_i, torch.zeros_like(b_i)).unsqueeze(1) * self.old_s[:, i]
-            d_new = torch.where(first.unsqueeze(1), -g, r)
+            self.push(y, sv, later & (ys > 1e-10), ys)
+            d_new = torch.where(first.unsqueeze(1), -g, self.direction(g))
             self.d = torch.where(active.unsqueeze(1), d_new, self.d)
             self.prev_g = torch.where(active.unsqueeze(1), g, self.prev_g)
             self.prev_loss = torch.where(active, loss, self.prev_loss)
@@ -290,6 +299,32 @@ def batched_lbfgs_fits(G, b, yy, n, xi0, lr_sindy=0.1, st_freq=50, threshold=0.0
     return x, mask, epochs
 
 
+def param_map(reg):
+    """(A, groups) of an equivariance-constrained regressor: vec(Ξ) = A·[β, const] (d·K × (nb + d), fp64; the constant
+    columns are zero unless the regressor allows a free constant) and the parameter index ranges of β and const."""
+    d, K = reg.latent_dim, reg.library.K
+    Q = reg.Q.detach().to(torch.float64)                          # vec(Ξ) (equation-major) = layout(Q β) [+ constants]
+    nb = Q.shape[1]
+    cols = []
+    for j in range(nb):                                            # Ξ is LINEAR in β: read the map off unit vectors
+        e = torch.zeros(nb, dtype=reg.beta.dtype, device=reg.beta.device)
+        e[j] = 1.0
+        flat = reg.Q @ e
+        Xi = flat.view(d, -1) if reg.use_kron_product else flat.view(-1, d).transpose(0, 1)
+        cols.append(Xi.reshape(-1).double())
+    groups = [(0, nb)]
+    if reg.allow_constant:
+        for i in range(d):
+            c = torch.zeros(d * K, dtype=torch.float64, device=Q.device)
+            c[i * K] = 1.0
+            cols.append(c)
+    groups.append((nb, nb + d))                                    # `const` is a parameter even when unused (sindy.py:59-60)
+    A = torch.stack(cols, dim=1)
+    if not reg.allow_constant:
+        A = torch.cat([A, torch.zeros(d * K, d, dtype=torch.float64, device=A.device)], dim=1)
+    return A, groups
+
+
 def run_seed_sweep_batched(x: torch.Tensor, dx: torch.Tensor, truth, seeds: Iterable[int],
                            make_regressor: Callable[[], object], subsample: float = 0.5, lr_sindy=0.1, st_freq=50,
                            threshold=0.05, num_epochs=200, draw: Optional[Callable] = None) -> List[Dict]:
@@ -320,25 +355,7 @@ def run_seed_sweep_batched(x: torch.Tensor, dx: torch.Tensor, truth, seeds: Iter
     reg0 = regs[0]
     d, K = reg0.latent_dim, reg0.library.K
     if reg0.constraint:
-        Q = reg0.Q.detach().to(torch.float64)                     # vec(Ξ) (equation-major) = layout(Q β) [+ constants]
-        nb = Q.shape[1]
-        cols = []
-        for j in range(nb):                                        # Ξ is LINEAR in β: read the map off unit vectors
-            e = torch.zeros(nb, dtype=reg0.beta.dtype, device=reg0.beta.device)
-            e[j] = 1.0
-            flat = reg0.Q @ e
-            Xi = flat.view(d, -1) if reg0.use_kron_product else flat.view(-1, d).transpose(0, 1)
-            cols.append(Xi.reshape(-1).double())
-        groups = [(0, nb)]
-        if reg0.allow_constant:
-            for i in range(d):
-                c = torch.zeros(d * K, dtype=torch.float64, device=Q.device)
-                c[i * K] = 1.0
-                cols.append(c)
-        groups.append((nb, nb + d))                                # `const` is a parameter even when unused (sindy.py:59-60)
-        A = torch.stack(cols, dim=1)
-        if not reg0.allow_constant:
-            A = torch.cat([A, torch.zeros(d * K, d, dtype=torch.float64, device=A.device)], dim=1)
+        A, groups = param_map(reg0)
         p0 = torch.stack([torch.cat([r.beta.detach().reshape(-1), r.const.detach().reshape(-1)]) for r in regs])
     else:
         A, groups = None, None
