@@ -291,6 +291,27 @@ int sb_rollout_score_grad(const float* x0, int64_t n_ics, const sb_library* lib,
                           float blowup, double* sse, int32_t* valid_rows, double* grad, void* ws, int64_t ws_bytes,
                           void* stream);
 
+/* sb_rollout_score with per-model initial conditions (output-error fits that estimate each trajectory's start):
+ * x0_per_model = 0 is sb_rollout_score (x0: n_ics × d, shared by all models; the same bits), 1 reads model m's starts
+ * from x0 + m·n_ics·d (x0: n_models × n_ics × d). A pair's outputs depend only on its own start, W_m and the data.
+ * SB_ERR_INVALID for x0_per_model outside {0, 1}; otherwise the status codes of sb_rollout_score. */
+int sb_rollout_score_ics(const float* x0, int x0_per_model, int64_t n_ics, const sb_library* lib, const float* w,
+                         int n_models, double dt, int64_t steps_per_row, int64_t n_rows, int method,
+                         const float* y_obs, float blowup, double* sse, int32_t* valid_rows, void* stream);
+
+/* sb_rollout_score_grad with per-model initial conditions (x0_per_model as in sb_rollout_score_ics) and the gradient
+ * with respect to them: grad_x0 (n_models × n_ics × d fp64) = ∂sse[m, n]/∂x0 of the pair (m, n), the adjoint state after
+ * the first step is reversed, widened from fp32. A pair with valid_rows = 0 gets exact zeros. Each element has one
+ * writer and no sum, so its bits do not depend on the batch, the model order or how the ICs are split. grad and grad_x0
+ * may each be NULL: with grad NULL the kernel keeps no W̄ accumulators and reduces nothing (the start-only variant,
+ * same sse / valid_rows / grad_x0 bits). Both NULL, or x0_per_model outside {0, 1}, is SB_ERR_INVALID; the workspace
+ * size and the other status codes are those of sb_rollout_score_grad. sb_rollout_score_grad is this call with
+ * x0_per_model = 0 and grad_x0 = NULL. */
+int sb_rollout_score_grad_ics(const float* x0, int x0_per_model, int64_t n_ics, const sb_library* lib, const float* w,
+                              int n_models, double dt, int64_t steps_per_row, int64_t n_rows, int method,
+                              const float* y_obs, float blowup, double* sse, int32_t* valid_rows, double* grad,
+                              double* grad_x0, void* ws, int64_t ws_bytes, void* stream);
+
 /* WSINDy weak-form integrals with trigonometric test functions (`sindy.py:332-347,361-362`):
  *   V[j,t]  = dt·sqrt(2/T)·sin((j+1)π t/T),  V'[j,t] = dt·sqrt(2/T)·(j+1)π/T·cos((j+1)π t/T),  t = t_idx·dt
  *   G[traj,j,k] = sum_t V[j,t]·Θ_k(x[traj,t]),   b[traj,j,i] = −sum_t V'[j,t]·x[traj,t,i]

@@ -390,8 +390,26 @@ int sb_rollout(const void* x0, int64_t n_ics, const sb_library* lib, const void*
 int sb_rollout_score(const float* x0, int64_t n_ics, const sb_library* lib, const float* w, int n_models, double dt,
                      int64_t steps_per_row, int64_t n_rows, int method, const float* y_obs, float blowup,
                      double* sse, int32_t* valid_rows, void* stream) {
+  return sb_rollout_score_ics(x0, 0, n_ics, lib, w, n_models, dt, steps_per_row, n_rows, method, y_obs, blowup, sse,
+                              valid_rows, stream);
+}
+
+namespace {
+int check_x0_per_model(int x0_per_model) {
+  if (x0_per_model != 0 && x0_per_model != 1) {
+    set_error("x0_per_model=%d is neither 0 nor 1", x0_per_model);
+    return SB_ERR_INVALID;
+  }
+  return SB_OK;
+}
+}  // namespace
+
+int sb_rollout_score_ics(const float* x0, int x0_per_model, int64_t n_ics, const sb_library* lib, const float* w,
+                         int n_models, double dt, int64_t steps_per_row, int64_t n_rows, int method,
+                         const float* y_obs, float blowup, double* sse, int32_t* valid_rows, void* stream) {
   LibTab t;
   SB_TRY(build_table(lib, &t));
+  SB_TRY(check_x0_per_model(x0_per_model));
   if (n_ics < 0 || n_models < 1 || steps_per_row < 1 || n_rows < 1 || n_rows > INT32_MAX ||
       steps_per_row > INT64_MAX / n_rows) {
     set_error("bad rollout_score sizes n_ics=%lld n_models=%d steps_per_row=%lld n_rows=%lld", (long long)n_ics,
@@ -403,8 +421,8 @@ int sb_rollout_score(const float* x0, int64_t n_ics, const sb_library* lib, cons
   SB_TRY(check_ptr(x0, "x0")); SB_TRY(check_ptr(w, "w")); SB_TRY(check_ptr(y_obs, "y_obs"));
   SB_TRY(check_ptr(sse, "sse")); SB_TRY(check_ptr(valid_rows, "valid_rows"));
   if (n_ics == 0) return SB_OK;
-  return rollout_score(x0, n_ics, t, w, n_models, dt, steps_per_row, n_rows, method, y_obs, blowup, sse, valid_rows,
-                       (cudaStream_t)stream);
+  return rollout_score(x0, x0_per_model ? n_ics * t.d : 0, n_ics, t, w, n_models, dt, steps_per_row, n_rows, method,
+                       y_obs, blowup, sse, valid_rows, (cudaStream_t)stream);
 }
 
 namespace {
@@ -433,20 +451,32 @@ int sb_rollout_score_grad(const float* x0, int64_t n_ics, const sb_library* lib,
                           double dt, int64_t steps_per_row, int64_t n_rows, int method, const float* y_obs,
                           float blowup, double* sse, int32_t* valid_rows, double* grad, void* ws, int64_t ws_bytes,
                           void* stream) {
+  return sb_rollout_score_grad_ics(x0, 0, n_ics, lib, w, n_models, dt, steps_per_row, n_rows, method, y_obs, blowup,
+                                   sse, valid_rows, grad, nullptr, ws, ws_bytes, stream);
+}
+
+int sb_rollout_score_grad_ics(const float* x0, int x0_per_model, int64_t n_ics, const sb_library* lib, const float* w,
+                              int n_models, double dt, int64_t steps_per_row, int64_t n_rows, int method,
+                              const float* y_obs, float blowup, double* sse, int32_t* valid_rows, double* grad,
+                              double* grad_x0, void* ws, int64_t ws_bytes, void* stream) {
   LibTab t;
   SB_TRY(build_table(lib, &t));
+  SB_TRY(check_x0_per_model(x0_per_model));
   SB_TRY(check_score_sizes(n_ics, n_models, steps_per_row, n_rows));
   if (method != SB_EULER && method != SB_RK4) { set_error("unknown method %d", method); return SB_ERR_INVALID; }
   if (!(dt > 0.0)) { set_error("dt=%g is not positive", dt); return SB_ERR_INVALID; }
   SB_TRY(check_ptr(x0, "x0")); SB_TRY(check_ptr(w, "w")); SB_TRY(check_ptr(y_obs, "y_obs"));
-  SB_TRY(check_ptr(sse, "sse")); SB_TRY(check_ptr(valid_rows, "valid_rows")); SB_TRY(check_ptr(grad, "grad"));
+  SB_TRY(check_ptr(sse, "sse")); SB_TRY(check_ptr(valid_rows, "valid_rows"));
+  if (!grad && !grad_x0) { set_error("grad and grad_x0 are both NULL"); return SB_ERR_INVALID; }
   SB_TRY(check_ptr(ws, "workspace"));
-  if (n_ics == 0) {   // no pair: the objective is the empty sum
-    SB_CUDA_TRY(cudaMemsetAsync(grad, 0, sizeof(double) * (size_t)n_models * t.d * t.K, (cudaStream_t)stream));
+  if (n_ics == 0) {   // no pair: the objective is the empty sum (grad_x0 has no element)
+    if (grad)
+      SB_CUDA_TRY(cudaMemsetAsync(grad, 0, sizeof(double) * (size_t)n_models * t.d * t.K, (cudaStream_t)stream));
     return SB_OK;
   }
-  return rollout_score_grad(x0, n_ics, t, w, n_models, dt, steps_per_row, n_rows, method, y_obs, blowup, sse,
-                            valid_rows, grad, ws, ws_bytes, (cudaStream_t)stream);
+  return rollout_score_grad(x0, x0_per_model ? n_ics * t.d : 0, n_ics, t, w, n_models, dt, steps_per_row, n_rows,
+                            method, y_obs, blowup, sse, valid_rows, grad, grad_x0, ws, ws_bytes,
+                            (cudaStream_t)stream);
 }
 
 int sb_wsindy_integrals(const float* x, int64_t n_traj, int64_t T, const sb_library* lib, float dt,

@@ -334,17 +334,20 @@ int rollout(const void* x0, int64_t n_ics, const LibTab& t, const void* w, doubl
             cudaStream_t s);
 
 // M models × N ICs integrated and scored against observed rows with the rollout's own step and right-hand sides
-// (sb_rollout.cu), so the compared states are the ones `rollout` stores; arguments validated by the caller
-int rollout_score(const float* x0, int64_t n_ics, const LibTab& t, const float* w, int n_models, double dt,
-                  int64_t steps_per_row, int64_t n_rows, int method, const float* y_obs, float blowup, double* sse,
-                  int32_t* valid_rows, cudaStream_t s);
-// the same scores and ∂/∂W_m Σ_n sse[m, n] by the discrete adjoint of the scored recurrence; arguments validated by the
-// caller. The workspace size is -1 when it does not fit in int64.
+// (sb_rollout.cu), so the compared states are the ones `rollout` stores; arguments validated by the caller. Model m starts
+// from x0 + m·x0_model_stride (0: one start set shared by all models, n_ics·d: one set per model).
+int rollout_score(const float* x0, int64_t x0_model_stride, int64_t n_ics, const LibTab& t, const float* w,
+                  int n_models, double dt, int64_t steps_per_row, int64_t n_rows, int method, const float* y_obs,
+                  float blowup, double* sse, int32_t* valid_rows, cudaStream_t s);
+// the same scores, ∂/∂W_m Σ_n sse[m, n] (grad) and ∂sse[m, n]/∂x0 of the pair (grad_x0, n_models × n_ics × d) by the
+// discrete adjoint of the scored recurrence; either output may be NULL, not both. Arguments validated by the caller. The
+// workspace size is -1 when it does not fit in int64.
 int64_t rollout_score_grad_workspace_bytes(int64_t n_ics, const LibTab& t, int n_models, int64_t steps_per_row,
                                            int64_t n_rows);
-int rollout_score_grad(const float* x0, int64_t n_ics, const LibTab& t, const float* w, int n_models, double dt,
-                       int64_t steps_per_row, int64_t n_rows, int method, const float* y_obs, float blowup, double* sse,
-                       int32_t* valid_rows, double* grad, void* ws, int64_t ws_bytes, cudaStream_t s);
+int rollout_score_grad(const float* x0, int64_t x0_model_stride, int64_t n_ics, const LibTab& t, const float* w,
+                       int n_models, double dt, int64_t steps_per_row, int64_t n_rows, int method, const float* y_obs,
+                       float blowup, double* sse, int32_t* valid_rows, double* grad, double* grad_x0, void* ws,
+                       int64_t ws_bytes, cudaStream_t s);
 
 // WSINDy integrals
 int wsindy_integrals(const float* x, int64_t n_traj, int64_t T, const LibTab& t, float dt, double t_max,

@@ -373,7 +373,8 @@ __global__ void __launch_bounds__(kMultiThreads) rollout_rk4_multi_kernel(RollAr
 constexpr int kMaxGridY = 65535;
 
 struct ScoreArgs {
-  const float* x0;
+  const float* x0;   // starts of the first model of this launch
+  int64_t x0_model_stride;   // elements from one model's starts to the next: 0 (shared) or n_ics·d
   int64_t n_ics;
   double dt;
   int64_t steps_per_row;
@@ -425,6 +426,7 @@ __global__ void __launch_bounds__(kMultiThreads) rollout_score_spec_kernel(Score
   __syncthreads();
   const int64_t base = (int64_t)blockIdx.x * (kThreads * NB) + threadIdx.x;
   if (base >= a.n_ics) return;
+  const float* x0 = a.x0 + model * a.x0_model_stride;
   float x[NB][D];
   bool track[NB];
   double sse[NB];
@@ -435,7 +437,7 @@ __global__ void __launch_bounds__(kMultiThreads) rollout_score_spec_kernel(Score
     track[b] = ic < a.n_ics;
     sse[b] = 0.0;
     valid[b] = a.n_rows;
-    static_for<0, D>([&](auto j) { x[b][j] = track[b] ? a.x0[ic * D + j] : 0.f; });
+    static_for<0, D>([&](auto j) { x[b][j] = track[b] ? x0[ic * D + j] : 0.f; });
   });
   const bool live1 = track[1];
   const Odeint<float> ode(a.dt);
@@ -476,9 +478,10 @@ __global__ void __launch_bounds__(kThreads) rollout_score_gen_kernel(LibTab t, i
   const int64_t model = blockIdx.y;
   const int d = t.d;
   const GenRhs<float, KMAX> rhs{t, a.w + model * d * t.K};
+  const float* x0 = a.x0 + model * a.x0_model_stride;
   float x[1][DN];
 #pragma unroll
-  for (int j = 0; j < DN; ++j) x[0][j] = (j < d) ? a.x0[ic * d + j] : 0.f;
+  for (int j = 0; j < DN; ++j) x[0][j] = (j < d) ? x0[ic * d + j] : 0.f;
   const Odeint<float> ode(a.dt);
   double sse = 0.0;
   int64_t valid = a.n_rows, row = 0, until = a.steps_per_row;
@@ -510,6 +513,11 @@ __global__ void __launch_bounds__(kThreads) rollout_score_gen_kernel(LibTab t, i
 //             warp order into one fp64 partial row per (model, IC block), and grad_sum_kernel adds those in block order.
 // Nothing depends on which other models share the launch: a model's gradient has the same bits alone, in any batch and
 // any model order, on every repeat (not across IC batch splits, which regroup the sums).
+//   starts:   λ after step 1 is reversed is ∂sse/∂x0 of the pair; it is written, widened to fp64, when grad_x0 is wanted.
+//             One writer per element and no sum, so those bits do not depend on the batch, the model order or the IC
+//             split. A pair with valid_rows = 0 reverses no step and writes exact zeros.
+//   WG:       false drops everything that exists only for W̄ (the d·K accumulators, the shared rows, the segment-end
+//             warp sums and the partial rows): the start-only variant for a caller that keeps W fixed.
 constexpr int kCkpt = 32;             // checkpoint interval: kCkpt + 1 states per thread in local memory
 constexpr int kGradThreads = kMultiThreads;
 constexpr int kGradWarps = kGradThreads / 32;
@@ -519,7 +527,8 @@ struct GradArgs {
   int64_t n_models;    // models of the whole call (checkpoint layout)
   int64_t model0;      // first model of this launch
   float* ckpt;         // [checkpoint][model][ic][d]
-  double* partial;     // [model][IC block][d·K], from this launch's first model
+  double* partial;     // [model][IC block][d·K], from this launch's first model (WG only)
+  double* grad_x0;     // [model][ic][d], from this launch's first model; NULL: not wanted
 };
 
 // specialised library: W from the block-staged shared copy (SharedW rows of KQ float4)
@@ -534,8 +543,9 @@ struct SpecGrad {
     eval_pairs<D, PC, 1>(SharedW<K>{sw + off}, reinterpret_cast<const float (&)[1][D]>(y),
                          reinterpret_cast<float (&)[1][D]>(k));
   }
-  // xb = J_h(y)ᵀu = J_Θ(y)ᵀ(Wᵀu);  acc += u ⊗ Θ(y)
-  __device__ __forceinline__ void vjp(const float (&y)[D], const float (&u)[D], float (&xb)[D], float (&acc)[ACC],
+  // xb = J_h(y)ᵀu = J_Θ(y)ᵀ(Wᵀu);  acc += u ⊗ Θ(y) when WG
+  template <bool WG, int NA>
+  __device__ __forceinline__ void vjp(const float (&y)[D], const float (&u)[D], float (&xb)[D], float (&acc)[NA],
                                       int off) const {
     const float* w = reinterpret_cast<const float*>(sw + off);
     float m[K], mb[K];
@@ -546,7 +556,7 @@ struct SpecGrad {
       static_for<0, D>([&](auto ic) {
         constexpr int i = ic;
         s = fmaf(w[i * KQ * 4 + k], u[i], s);
-        acc[i * K + k] = fmaf(u[i], m[k], acc[i * K + k]);
+        if constexpr (WG) acc[i * K + k] = fmaf(u[i], m[k], acc[i * K + k]);
       });
       mb[k] = s;
     });
@@ -567,7 +577,8 @@ struct GenGrad {
   __device__ __forceinline__ void eval(const float (&y)[DN], float (&k)[DN], int) const {
     GenRhs<float, KMAX>{t, w}.eval(y, k);
   }
-  __device__ __forceinline__ void vjp(const float (&y)[DN], const float (&u)[DN], float (&xb)[DN], float (&acc)[ACC],
+  template <bool WG, int NA>
+  __device__ __forceinline__ void vjp(const float (&y)[DN], const float (&u)[DN], float (&xb)[DN], float (&acc)[NA],
                                       int) const {
     float m[KMAX], mb[KMAX];
     expand_table(t, y, m);
@@ -575,7 +586,7 @@ struct GenGrad {
       float s = 0.f;
       for (int i = 0; i < t.d; ++i) {
         s = fmaf(__ldg(w + i * t.K + k), u[i], s);
-        acc[i * t.K + k] = fmaf(u[i], m[k], acc[i * t.K + k]);
+        if constexpr (WG) acc[i * t.K + k] = fmaf(u[i], m[k], acc[i * t.K + k]);
       }
       mb[k] = s;
     }
@@ -594,8 +605,8 @@ __device__ __forceinline__ int64_t warp_max(int64_t v) {
   return v;
 }
 
-// every thread of the block takes part (warp shuffles, block barrier), including those past the last IC
-template <class G>
+// with WG every thread of the block takes part (warp shuffles, block barrier), including those past the last IC
+template <bool WG, class G>
 __device__ __forceinline__ void grad_body(const G& g, int method, const GradArgs& a, double* sacc) {
   constexpr int DN = G::DN;
   const int d = g.dim(), dk = g.dk();
@@ -613,7 +624,7 @@ __device__ __forceinline__ void grad_body(const G& g, int method, const GradArgs
   // ---- forward: the scorer's loop, with checkpoints ----
   float x[1][DN];
 #pragma unroll
-  for (int j = 0; j < DN; ++j) x[0][j] = (live && j < d) ? sa.x0[ic * d + j] : 0.f;
+  for (int j = 0; j < DN; ++j) x[0][j] = (live && j < d) ? sa.x0[model * sa.x0_model_stride + ic * d + j] : 0.f;
   int64_t valid = 0;
   if (live) {
     double sse = 0.0;
@@ -641,10 +652,14 @@ __device__ __forceinline__ void grad_body(const G& g, int method, const GradArgs
 
   // ---- backward over the segments of [0, S) ----
   const int64_t S = valid * spr;
-  const int64_t n_seg = warp_max((S + kCkpt - 1) / kCkpt);
-  float acc[G::ACC];
-  if constexpr (G::kStatic) static_for<0, G::ACC>([&](auto e) { acc[e] = 0.f; });
-  else for (int e = 0; e < dk; ++e) acc[e] = 0.f;
+  const int64_t n_seg = WG ? warp_max((S + kCkpt - 1) / kCkpt) : (S + kCkpt - 1) / kCkpt;
+  float acc[WG ? G::ACC : 1];
+  if constexpr (!WG) {
+  } else if constexpr (G::kStatic) {
+    static_for<0, G::ACC>([&](auto e) { acc[e] = 0.f; });
+  } else {
+    for (int e = 0; e < dk; ++e) acc[e] = 0.f;
+  }
   float lam[DN];
 #pragma unroll
   for (int j = 0; j < DN; ++j) lam[j] = 0.f;
@@ -684,7 +699,7 @@ __device__ __forceinline__ void grad_body(const G& g, int method, const GradArgs
           float u[DN];
 #pragma unroll
           for (int j = 0; j < DN; ++j) u[j] = ode.dt * lam[j];
-          g.vjp(y1, u, xb, acc, off);
+          g.template vjp<WG>(y1, u, xb, acc, off);
 #pragma unroll
           for (int j = 0; j < DN; ++j) lam[j] += xb[j];
           continue;
@@ -711,7 +726,7 @@ __device__ __forceinline__ void grad_body(const G& g, int method, const GradArgs
           float ysd[DN];
 #pragma unroll
           for (int j = 0; j < DN; ++j) ysd[j] = ys[st][j];
-          g.vjp(ysd, k, xb, acc, off);
+          g.template vjp<WG>(ysd, k, xb, acc, off);
           const float route = st == 3 ? ode.dt : ode.hdt, base = st == 1 ? 1.f : 2.f;
 #pragma unroll
           for (int j = 0; j < DN; ++j) { lam[j] += xb[j]; k[j] = base * av[j] + route * xb[j]; }   // k̄_{st}
@@ -719,7 +734,8 @@ __device__ __forceinline__ void grad_body(const G& g, int method, const GradArgs
       }
     }
     // segment end: fp32 sums into the warp's fp64 row
-    if constexpr (G::kStatic) {
+    if constexpr (!WG) {
+    } else if constexpr (G::kStatic) {
       static_for<0, G::ACC>([&](auto e) {
         const double v = warp_sum((double)acc[e]);
         if (lane0) mine[e] += v;
@@ -733,22 +749,30 @@ __device__ __forceinline__ void grad_body(const G& g, int method, const GradArgs
       }
     }
   }
-  __syncthreads();
-  double* part = a.partial + (model * gridDim.x + blockIdx.x) * dk;
-  for (int e = threadIdx.x; e < dk; e += kGradThreads) {
-    double v = 0.0;
+  if (a.grad_x0 && live) {
+    double* gx = a.grad_x0 + (model * N + ic) * d;
 #pragma unroll
-    for (int w = 0; w < kGradWarps; ++w) v += sacc[w * G::ACC + e];
-    part[e] = v;
+    for (int j = 0; j < DN; ++j)
+      if (j < d) gx[j] = (double)lam[j];
+  }
+  if constexpr (WG) {
+    __syncthreads();
+    double* part = a.partial + (model * gridDim.x + blockIdx.x) * dk;
+    for (int e = threadIdx.x; e < dk; e += kGradThreads) {
+      double v = 0.0;
+#pragma unroll
+      for (int w = 0; w < kGradWarps; ++w) v += sacc[w * G::ACC + e];
+      part[e] = v;
+    }
   }
 }
 
-template <int D, int PC, int METHOD>
+template <int D, int PC, int METHOD, bool WG>
 __global__ void __launch_bounds__(kGradThreads) rollout_grad_spec_kernel(GradArgs a) {
   using G = SpecGrad<D, PC>;
-  constexpr int K = G::K, KQ = G::KQ;
+  constexpr int K = G::K, KQ = G::KQ, NS = WG ? kGradWarps * G::ACC : 1;
   __shared__ float4 sw[D * KQ];
-  __shared__ double sacc[kGradWarps * G::ACC];
+  __shared__ double sacc[NS];
   {
     const float* wm = a.s.w + (int64_t)blockIdx.y * (D * K);
     float* s = reinterpret_cast<float*>(sw);
@@ -756,19 +780,23 @@ __global__ void __launch_bounds__(kGradThreads) rollout_grad_spec_kernel(GradArg
       const int i = q / (KQ * 4), c = q % (KQ * 4);
       s[q] = c < K ? wm[i * K + c] : 0.f;
     }
-    for (int q = threadIdx.x; q < kGradWarps * G::ACC; q += kGradThreads) sacc[q] = 0.0;
+    if constexpr (WG)
+      for (int q = threadIdx.x; q < NS; q += kGradThreads) sacc[q] = 0.0;
   }
   __syncthreads();
-  grad_body(G{sw}, METHOD, a, sacc);
+  grad_body<WG>(G{sw}, METHOD, a, sacc);
 }
 
-template <int KMAX>
+template <int KMAX, bool WG>
 __global__ void __launch_bounds__(kGradThreads) rollout_grad_gen_kernel(LibTab t, int method, GradArgs a) {
   using G = GenGrad<KMAX>;
-  __shared__ double sacc[kGradWarps * G::ACC];
-  for (int q = threadIdx.x; q < kGradWarps * G::ACC; q += kGradThreads) sacc[q] = 0.0;
-  __syncthreads();
-  grad_body(G{t, a.s.w + (int64_t)blockIdx.y * t.d * t.K}, method, a, sacc);
+  constexpr int NS = WG ? kGradWarps * G::ACC : 1;
+  __shared__ double sacc[NS];
+  if constexpr (WG) {
+    for (int q = threadIdx.x; q < NS; q += kGradThreads) sacc[q] = 0.0;
+    __syncthreads();
+  }
+  grad_body<WG>(G{t, a.s.w + (int64_t)blockIdx.y * t.d * t.K}, method, a, sacc);
 }
 
 // grad[m, e] = Σ_b partial[m, b, e] in block order
@@ -851,24 +879,25 @@ int launch_score(const LibTab& t, const ScoreArgs& a, int method, int n_models, 
 
 int64_t grad_blocks(int64_t n_ics) { return (n_ics + kGradThreads - 1) / kGradThreads; }
 
-template <int D, int PC>
+template <int D, int PC, bool WG>
 int launch_grad_spec(const GradArgs& a, int method, int n_models, cudaStream_t s) {
   const dim3 grid((unsigned)grad_blocks(a.s.n_ics), (unsigned)n_models);
-  if (method == SB_EULER) rollout_grad_spec_kernel<D, PC, SB_EULER><<<grid, kGradThreads, 0, s>>>(a);
-  else rollout_grad_spec_kernel<D, PC, SB_RK4><<<grid, kGradThreads, 0, s>>>(a);
+  if (method == SB_EULER) rollout_grad_spec_kernel<D, PC, SB_EULER, WG><<<grid, kGradThreads, 0, s>>>(a);
+  else rollout_grad_spec_kernel<D, PC, SB_RK4, WG><<<grid, kGradThreads, 0, s>>>(a);
   SB_LAUNCH_CHECK("rollout_grad_spec_kernel");
   return SB_OK;
 }
 
+template <bool WG>
 int launch_grad(const LibTab& t, const GradArgs& a, int method, int n_models, cudaStream_t s) {
 #define X(D, PC) \
-  if (lib_matches<D, PC>(t)) return launch_grad_spec<D, PC>(a, method, n_models, s);
+  if (lib_matches<D, PC>(t)) return launch_grad_spec<D, PC, WG>(a, method, n_models, s);
   SB_SPEC_SHAPES(X)
 #undef X
   const dim3 grid((unsigned)grad_blocks(a.s.n_ics), (unsigned)n_models);
-  if (t.K <= 16) rollout_grad_gen_kernel<16><<<grid, kGradThreads, 0, s>>>(t, method, a);
-  else if (t.K <= 64) rollout_grad_gen_kernel<64><<<grid, kGradThreads, 0, s>>>(t, method, a);
-  else rollout_grad_gen_kernel<256><<<grid, kGradThreads, 0, s>>>(t, method, a);
+  if (t.K <= 16) rollout_grad_gen_kernel<16, WG><<<grid, kGradThreads, 0, s>>>(t, method, a);
+  else if (t.K <= 64) rollout_grad_gen_kernel<64, WG><<<grid, kGradThreads, 0, s>>>(t, method, a);
+  else rollout_grad_gen_kernel<256, WG><<<grid, kGradThreads, 0, s>>>(t, method, a);
   SB_LAUNCH_CHECK("rollout_grad_gen_kernel");
   return SB_OK;
 }
@@ -902,9 +931,10 @@ int64_t rollout_score_grad_workspace_bytes(int64_t n_ics, const LibTab& t, int n
   return L.partial_bytes + L.ckpt_bytes;
 }
 
-int rollout_score_grad(const float* x0, int64_t n_ics, const LibTab& t, const float* w, int n_models, double dt,
-                       int64_t steps_per_row, int64_t n_rows, int method, const float* y_obs, float blowup, double* sse,
-                       int32_t* valid_rows, double* grad, void* ws, int64_t ws_bytes, cudaStream_t s) {
+int rollout_score_grad(const float* x0, int64_t x0_model_stride, int64_t n_ics, const LibTab& t, const float* w,
+                       int n_models, double dt, int64_t steps_per_row, int64_t n_rows, int method, const float* y_obs,
+                       float blowup, double* sse, int32_t* valid_rows, double* grad, double* grad_x0, void* ws,
+                       int64_t ws_bytes, cudaStream_t s) {
   GradLayout L;
   if (!grad_layout(n_ics, t, n_models, steps_per_row, n_rows, &L)) {
     set_error("rollout_score_grad workspace size overflows int64");
@@ -919,21 +949,25 @@ int rollout_score_grad(const float* x0, int64_t n_ics, const LibTab& t, const fl
   const int64_t nblk = grad_blocks(n_ics);
   double* partial = reinterpret_cast<double*>(ws);
   GradArgs a{};
-  a.s.x0 = x0; a.s.n_ics = n_ics; a.s.dt = dt; a.s.steps_per_row = steps_per_row; a.s.n_rows = n_rows;
+  a.s.x0_model_stride = x0_model_stride;
+  a.s.n_ics = n_ics; a.s.dt = dt; a.s.steps_per_row = steps_per_row; a.s.n_rows = n_rows;
   a.s.y_obs = y_obs; a.s.blowup = blowup; a.s.opaque = 0;
   a.n_models = n_models;
   a.ckpt = reinterpret_cast<float*>(reinterpret_cast<char*>(ws) + L.partial_bytes);
   // more models than gridDim.y allows: further launches on the same stream
   for (int m0 = 0; m0 < n_models; m0 += kMaxGridY) {
     const int nm = n_models - m0 < kMaxGridY ? n_models - m0 : kMaxGridY;
+    a.s.x0 = x0 + (int64_t)m0 * x0_model_stride;
     a.s.w = w + (int64_t)m0 * dk;
     a.s.sse = sse + (int64_t)m0 * n_ics;
     a.s.valid = valid_rows + (int64_t)m0 * n_ics;
     a.model0 = m0;
     a.partial = partial + (int64_t)m0 * nblk * dk;
-    const int st = launch_grad(t, a, method, nm, s);
+    a.grad_x0 = grad_x0 ? grad_x0 + (int64_t)m0 * n_ics * t.d : nullptr;
+    const int st = grad ? launch_grad<true>(t, a, method, nm, s) : launch_grad<false>(t, a, method, nm, s);
     if (st != SB_OK) return st;
   }
+  if (!grad) return SB_OK;
   const int64_t n = (int64_t)n_models * dk;
   grad_sum_kernel<<<(unsigned)((n + 255) / 256), 256, 0, s>>>(partial, nblk, dk, n, grad);
   SB_LAUNCH_CHECK("grad_sum_kernel");
@@ -950,15 +984,16 @@ int rollout(const void* x0, int64_t n_ics, const LibTab& t, const void* w, doubl
   return launch_rollout<double>(t, w, a, s);
 }
 
-int rollout_score(const float* x0, int64_t n_ics, const LibTab& t, const float* w, int n_models, double dt,
-                  int64_t steps_per_row, int64_t n_rows, int method, const float* y_obs, float blowup, double* sse,
-                  int32_t* valid_rows, cudaStream_t s) {
+int rollout_score(const float* x0, int64_t x0_model_stride, int64_t n_ics, const LibTab& t, const float* w,
+                  int n_models, double dt, int64_t steps_per_row, int64_t n_rows, int method, const float* y_obs,
+                  float blowup, double* sse, int32_t* valid_rows, cudaStream_t s) {
   ScoreArgs a{};
-  a.x0 = x0; a.n_ics = n_ics; a.dt = dt; a.steps_per_row = steps_per_row; a.n_rows = n_rows; a.y_obs = y_obs;
+  a.x0_model_stride = x0_model_stride; a.n_ics = n_ics; a.dt = dt; a.steps_per_row = steps_per_row; a.n_rows = n_rows; a.y_obs = y_obs;
   a.blowup = blowup; a.opaque = 0;
   // more models than gridDim.y allows: further launches on the same stream
   for (int m0 = 0; m0 < n_models; m0 += kMaxGridY) {
     const int nm = n_models - m0 < kMaxGridY ? n_models - m0 : kMaxGridY;
+    a.x0 = x0 + (int64_t)m0 * x0_model_stride;
     a.w = w + (int64_t)m0 * t.d * t.K;
     a.sse = sse + (int64_t)m0 * n_ics;
     a.valid = valid_rows + (int64_t)m0 * n_ics;

@@ -635,7 +635,8 @@ def stlsq_path(regressor, x, y, thresholds, w_sindy_reg=0.0, max_iter=5, **kwarg
     return out
 
 
-def score_path(library, path, x_val, dt, steps_per_row=1, method='rk4', blowup=None, criterion='aicc'):
+def score_path(library, path, x_val, dt, steps_per_row=1, method='rk4', blowup=None, criterion='aicc', fit_ic=False,
+               window=None, ic_iter=20):
     """Scores the candidates of `stlsq_path` / `WSINDyWrapper.solve_path` by simulation on held-out trajectories.
 
     x_val (n_traj, T, d): trajectories with rows dt·steps_per_row apart. Every distinct candidate model is integrated
@@ -645,13 +646,25 @@ def score_path(library, path, x_val, dt, steps_per_row=1, method='rk4', blowup=N
       AIC = n·ln(SSE/n) + 2k,  AICc = AIC + 2k(k+1)/(n−k−1),  BIC = n·ln(SSE/n) + k·ln n
     (+inf for a diverged candidate; AICc also when n−k−1 ≤ 0). `chosen` is the argmin of `criterion` ('aic', 'aicc' or
     'bic'); ties go to the smaller k, then the larger threshold; None if every candidate scores +inf. `library` is a
-    `native.Library` or a SINDyRegression."""
+    `native.Library` or a SINDyRegression.
+
+    window=R (an integer ≥ 2 dividing T) splits every trajectory into T/R consecutive windows of R rows, each scored as
+    a trajectory of its own (n_starts = n_traj·T/R starts); None is R = T.
+
+    fit_ic=True estimates every start: with the candidate's W fixed, each (candidate, start) pair's x̂0 minimises
+    ‖rollout from x̂0 − rows 1..R−1‖² + ‖x̂0 − row 0‖², an independent d-dimensional problem. All pairs of all
+    candidates run as one batch of `ic_iter` lock-step L-BFGS iterations (gradients from the start-only variant of
+    `native.rollout_score_grad`, trial points from one per-model-start `native.rollout_score` launch; a trial that
+    diverges counts as +inf, so `diverged` can only shrink). x̂0 starts at row 0 and each pair keeps its best iterate, so
+    every candidate's sse (which now includes the row-0 residuals) is at most its fixed-start sse. The criteria use
+    n = n_starts·R·d and k_eff = k + k_ic, k_ic = n_starts·d; `k` stays the live-coefficient count. Adds k_ic and x0
+    (P, n_starts, d) fp32."""
     lib = getattr(library, 'library', library)
     if not isinstance(lib, Library):
         raise ValueError(f"library must be a native.Library or a SINDyRegression, got {type(library).__name__}")
     if criterion not in ('aic', 'aicc', 'bic'):
         raise ValueError(f"criterion must be 'aic', 'aicc' or 'bic', got {criterion!r}")
-    x_val, dt = _check_rollout_args(lib, x_val, "x_val", dt, steps_per_row, method, blowup)
+    x_val, dt = _check_rollout_args(lib, x_val, "x_val", dt, steps_per_row, method, blowup, fit_ic, window, ic_iter)
     n_traj, T, d = x_val.shape
     W, masks = path["xi"], path["mask"]
     if W.dim() != 3 or W.shape[1:] != (d, lib.K) or masks.shape != W.shape:
@@ -662,25 +675,74 @@ def score_path(library, path, x_val, dt, steps_per_row=1, method='rk4', blowup=N
     dev = W.device
     xv = x_val.to(device=dev, dtype=torch.float32)
     models, inverse = torch.unique(W.reshape(P, -1), dim=0, return_inverse=True)
+    x0, y = xv[:, 0].contiguous(), xv[:, 1:].transpose(0, 1).contiguous()
     with torch.no_grad():
-        sse, valid = native.rollout_score(xv[:, 0].contiguous(), models.view(-1, d, lib.K), lib, dt, int(steps_per_row),
-                                          xv[:, 1:].transpose(0, 1).contiguous(), method, blowup)
+        sse, valid = native.rollout_score(x0, models.view(-1, d, lib.K), lib, dt, int(steps_per_row), y, method, blowup)
+        if fit_ic:
+            sse, valid, x0_hat = _fit_starts(lib, models.view(-1, d, lib.K), x0, y, dt, int(steps_per_row), method,
+                                             blowup, sse, valid, int(ic_iter))
     sse = sse.sum(1).cpu()[inverse.cpu()]
     diverged = (valid < T - 1).any(1).cpu()[inverse.cpu()]
     k = masks.flatten(1).sum(1).cpu().to(torch.float64)
-    n = n_traj * (T - 1) * d
-    crit = information_criteria(sse, n, k)
+    n, k_ic = _obs_counts(n_traj, T, d, fit_ic)
+    crit = information_criteria(sse, n, k + k_ic)
     for c in crit.values():
         c[diverged] = math.inf
     out = {"sse": sse, "diverged": diverged, "n_obs": n, "k": k.to(torch.int64), **crit, "criterion": criterion}
+    if fit_ic:
+        out["k_ic"] = k_ic
+        out["x0"] = x0_hat[inverse.to(dev)]
     c = crit[criterion].numpy()
     order = np.lexsort((-thr.numpy(), k.numpy(), c))                      # last key sorts first
     out["chosen"] = int(order[0]) if c[order[0]] < math.inf else None
     return out
 
 
-def _check_rollout_args(lib, x, name, dt, steps_per_row, method, blowup):
-    """The checks score_path and refine_path share; returns (x as a tensor, dt)."""
+def _obs_counts(n_starts, R, d, fit_ic):
+    """(n_obs, k_ic) of n_starts trajectories of R rows: rows 1..R−1 are compared, and with start estimation row 0 is
+    one more residual and every start adds d parameters."""
+    return (n_starts * R * d, n_starts * d) if fit_ic else (n_starts * (R - 1) * d, 0)
+
+
+def _fit_starts(lib, W, x0, y, dt, spr, method, blowup, sse0, valid0, max_iter):
+    """score_path(fit_ic=True): per (model, start) pair, x̂0 minimising (pair SSE from x̂0 + ‖x̂0 − x0‖²) / (R·d) with W
+    fixed, all pairs through `_lockstep_lbfgs` at once. Returns the pair totals (sse + start residual, M × N fp64), the
+    valid rows at x̂0 and x̂0 (M × N × d fp32). sse0 / valid0 are the fixed-start scores: a pair that diverged there
+    keeps x0."""
+    M, (N, d), R = W.shape[0], x0.shape, y.shape[0] + 1
+    nrm = R * d
+    x0d = x0.to(torch.float64).expand(M, N, d).reshape(M * N, d)
+
+    def loss_grad(q):
+        sse, valid, _, gx = native.rollout_score_grad(q.view(M, N, d).float(), W, lib, dt, spr, y, method, blowup,
+                                                       x0_grad=True, w_grad=False)
+        r = q - x0d
+        f = (sse.reshape(-1) + (r * r).sum(1)) / nrm
+        f = torch.where(valid.reshape(-1) < R - 1, torch.full_like(f, math.inf), f)
+        return f, (gx.reshape(-1, d) + 2 * r) / nrm
+
+    def loss(q, rows):
+        full = x0d.clone()                       # the pairs outside `rows` are evaluated at x0 and discarded
+        full[rows] = q
+        sse, valid = native.rollout_score(full.view(M, N, d).float(), W, lib, dt, spr, y, method, blowup)
+        r = q - x0d[rows]
+        f = (sse.reshape(-1)[rows] + (r * r).sum(1)) / nrm
+        return torch.where(valid.reshape(-1)[rows] < R - 1, torch.full_like(f, math.inf), f)
+
+    q, _, _, iters = _lockstep_lbfgs(x0d.clone(), loss_grad, loss, max_iter, 1e-7)
+    x0_hat = q.view(M, N, d).float()
+    sse, valid = native.rollout_score(x0_hat, W, lib, dt, spr, y, method, blowup)
+    r = q.view(M, N, d) - x0d.view(M, N, d)
+    moved = (iters > 0).view(M, N)
+    # a pair that never accepted a step is exactly at x0 (start residual 0, the fixed-start scores); a pair that did
+    # has a strictly lower objective
+    tot = torch.where(moved, sse + (r * r).sum(2), sse0)
+    return tot, torch.where(moved, valid, valid0), x0_hat
+
+
+def _check_rollout_args(lib, x, name, dt, steps_per_row, method, blowup, fit_ic=False, window=None, ic_iter=1):
+    """The checks score_path and refine_path share; returns (x as a tensor, dt). With window=R the returned x holds
+    the n_traj·T/R windows of R consecutive rows as trajectories."""
     if method not in ('euler', 'rk4'):
         raise ValueError(f"method must be 'euler' or 'rk4', got {method!r}")
     if isinstance(steps_per_row, bool) or not isinstance(steps_per_row, (int, np.integer)) or steps_per_row < 1:
@@ -690,31 +752,104 @@ def _check_rollout_args(lib, x, name, dt, steps_per_row, method, blowup):
         raise ValueError(f"dt must be positive, got {dt}")
     if blowup is not None and not (math.isfinite(float(blowup)) and float(blowup) > 0):
         raise ValueError(f"blowup must be a positive number or None, got {blowup!r}")
+    if not isinstance(fit_ic, (bool, np.bool_)):
+        raise ValueError(f"fit_ic must be True or False, got {fit_ic!r}")
+    if isinstance(ic_iter, bool) or not isinstance(ic_iter, (int, np.integer)) or ic_iter < 1:
+        raise ValueError(f"ic_iter must be a positive integer, got {ic_iter!r}")
     x = torch.as_tensor(x)
     if x.dim() != 3 or x.shape[-1] != lib.dim:
         raise ValueError(f"{name} must be (n_traj, T, {lib.dim}), got {tuple(x.shape)}")
     if x.shape[1] < 2 or x.shape[0] < 1:
         raise ValueError(f"{name} needs at least one trajectory of T >= 2 rows, got {tuple(x.shape)}")
+    if window is not None:
+        T = x.shape[1]
+        if isinstance(window, bool) or not isinstance(window, (int, np.integer)) or window < 2 or T % window:
+            raise ValueError(f"window must be an integer >= 2 that divides T = {T}, got {window!r}")
+        x = x.reshape(x.shape[0] * (T // int(window)), int(window), x.shape[2])
     if not bool(torch.isfinite(x).all()):
         raise ValueError(f"{name} has non-finite values")
     return x, dt
 
 
-def refine_path(regressor, path, x_fit, dt, steps_per_row=1, method='rk4', blowup=None, max_iter=50, tol=1e-7):
+def _lockstep_lbfgs(p, loss_grad, loss, max_iter, tol, dir_mask=None):
+    """Minimises U independent problems in lock-step: p (U, n) fp64 starting parameters; loss_grad(q) gives the losses
+    (U,) and gradients (U, n) of all problems in one batch, loss(q, rows) the losses of the problems `rows` at q (one row
+    each); +inf marks a diverged point. Per iteration: the L-BFGS direction (`sweep.BatchedLBFGS.direction`, times
+    dir_mask when given), steepest descent where that is not a descent direction, then a backtracking (Armijo) line
+    search whose trial points of every problem still searching are evaluated by one `loss` call. A problem stops after
+    max_iter iterations, when its loss falls by less than tol·loss, or when no step length decreases it; its best
+    iterate is kept. Returns (p, loss, loss at the start, accepted iterations), the last three per problem."""
+    import sweep
+    U = p.shape[0]
+    f, g = loss_grad(p)
+    f_before = f.clone()
+    opt = sweep.BatchedLBFGS(p, 1.0, history_size=10)
+    iters = torch.zeros(U, dtype=torch.long, device=p.device)
+    active = torch.isfinite(f) & (g.abs().amax(1) > 0)
+    c1, max_ls = 1e-4, 30
+    for _ in range(max_iter):
+        if not bool(active.any()):
+            break
+        dirn = opt.direction(g)
+        if dir_mask is not None:
+            dirn = dirn * dir_mask
+        gtd = (g * dirn).sum(1)
+        restart = gtd >= 0                                       # not a descent direction: steepest descent
+        dirn = torch.where(restart.unsqueeze(1), -g, dirn)
+        gtd = torch.where(restart, -(g * g).sum(1), gtd)
+        t = torch.where(opt.hist == 0, torch.clamp(1.0 / g.abs().sum(1), max=1.0), torch.ones_like(f))
+        searching, accepted = active.clone(), torch.zeros_like(active)
+        for _ls in range(max_ls):
+            idx = torch.nonzero(searching).flatten()
+            if idx.numel() == 0:
+                break
+            trial = p[idx] + t[idx].unsqueeze(1) * dirn[idx]
+            ft = loss(trial, idx)
+            ok = ft <= f[idx] + c1 * t[idx] * gtd[idx]
+            accepted[idx[ok]] = True
+            searching[idx[ok]] = False
+            t[idx[~ok]] *= 0.5
+        active &= accepted                                        # no step length decreased the loss: done
+        p_new = torch.where(active.unsqueeze(1), p + t.unsqueeze(1) * dirn, p)
+        f_new, g_new = loss_grad(p_new)
+        f_new = torch.where(active, f_new, f)
+        g_new = torch.where(active.unsqueeze(1), g_new, g)
+        sv, yv = p_new - p, g_new - g
+        ys = (sv * yv).sum(1)
+        opt.push(yv, sv, active & (ys > 1e-10), ys)
+        iters += active.long()
+        small = (f - f_new) <= tol * f.abs()
+        p, f, g = p_new, f_new, g_new
+        active &= ~small & (g.abs().amax(1) > 0)
+    return p, f, f_before, iters
+
+
+def refine_path(regressor, path, x_fit, dt, steps_per_row=1, method='rk4', blowup=None, max_iter=50, tol=1e-7,
+                fit_ic=False, window=None):
     """Trajectory refit of the candidates of `stlsq_path` / `WSINDyWrapper.solve_path`: every distinct candidate's
     coefficients are refit on its own support by minimising the simulation error on the fitting trajectories,
       loss = SSE / n_obs of the rollouts from x_fit[:, 0] (step dt) against rows 1..T−1, n_obs = n_traj·(T−1)·d,
     the objective `score_path` ranks by. Derivative regression leaves a bias that grows with the noise of the smoothed
     derivatives; this refit judges a support by its best coefficients rather than by the ones regression gave it.
 
-    All candidates advance together: one `native.rollout_score_grad` launch gives every loss and gradient (discrete
-    adjoint of the fp32 rollout), the L-BFGS direction is `sweep.BatchedLBFGS.direction` over the candidate axis, and a
-    per-candidate backtracking (Armijo) line search evaluates the trial points of every candidate still searching in one
-    `native.rollout_score` launch; a trial that diverges (fewer rows than T−1 compared) counts as +inf. A candidate stops
-    after max_iter iterations, when its loss falls by less than tol·loss, or when no step length decreases it; its best
-    iterate is kept, so sse_after <= sse_before. Masks are fixed: dead coefficients stay exactly 0. An
-    equivariance-constrained regressor is refit in its parameters (β, const), vec(Ξ) = A·[β, const], A from
+    All candidates advance together (`_lockstep_lbfgs`): one `native.rollout_score_grad` launch gives every loss and
+    gradient (discrete adjoint of the fp32 rollout), the L-BFGS direction is `sweep.BatchedLBFGS.direction` over the
+    candidate axis, and a per-candidate backtracking (Armijo) line search evaluates the trial points of every candidate
+    still searching in one `native.rollout_score` launch; a trial that diverges (fewer rows than T−1 compared) counts as
+    +inf. A candidate stops after max_iter iterations, when its loss falls by less than tol·loss, or when no step length
+    decreases it; its best iterate is kept, so sse_after <= sse_before. Masks are fixed: dead coefficients stay exactly
+    0. An equivariance-constrained regressor is refit in its parameters (β, const), vec(Ξ) = A·[β, const], A from
     `sweep.param_map`, and the returned path carries the new beta / const for `apply_candidate`.
+
+    window=R (an integer ≥ 2 dividing T) fits on the n_traj·T/R consecutive windows of R rows as trajectories of their
+    own (n_starts of them; None is R = T): over a long horizon the single-shooting SSE is dominated by phase drift.
+
+    fit_ic=True also estimates every start, since row 0 is an observation with the noise of the others: each
+    candidate's parameters become [coefficients (or β, const), x̂0 of every start] and the loss
+      (Σ SSE of the rollouts from x̂0 against rows 1..R−1 + Σ ‖x̂0 − row 0‖²) / n_obs,  n_obs = n_starts·R·d,
+    with ∂/∂x̂0 from `native.rollout_score_grad(x0_grad=True)` (per-model starts) plus 2(x̂0 − row 0). x̂0 starts at
+    row 0, so sse_before is the fixed-start value; the starts are unconstrained (also for a constrained regressor),
+    and one step length moves coefficients and starts together. Adds x0 (P, n_starts, d) fp32.
 
     Returns a copy of `path` with xi refit and sse_before, sse_after (P,) fp64 and iterations (P,) added; a candidate that
     diverges from the start keeps its coefficients (sse_before = sse_after = +inf)."""
@@ -723,7 +858,7 @@ def refine_path(regressor, path, x_fit, dt, steps_per_row=1, method='rk4', blowu
     if not isinstance(lib, Library):
         raise ValueError(f"regressor must be a SINDyRegression or a native.Library, got {type(regressor).__name__}")
     constrained = bool(getattr(regressor, 'constraint', False))
-    x_fit, dt = _check_rollout_args(lib, x_fit, "x_fit", dt, steps_per_row, method, blowup)
+    x_fit, dt = _check_rollout_args(lib, x_fit, "x_fit", dt, steps_per_row, method, blowup, fit_ic, window)
     if isinstance(max_iter, bool) or not isinstance(max_iter, (int, np.integer)) or max_iter < 1:
         raise ValueError(f"max_iter must be a positive integer, got {max_iter!r}")
     if not (math.isfinite(float(tol)) and float(tol) >= 0):
@@ -759,59 +894,59 @@ def refine_path(regressor, path, x_fit, dt, steps_per_row=1, method='rk4', blowu
         v = q if A is None else q @ A.T
         return (v * m).to(torch.float32).view(-1, d, lib.K)
 
-    def loss_grad(q):
-        sse, valid, g = native.rollout_score_grad(x0, W_of(q, mk), lib, dt, int(steps_per_row), y, method, blowup)
-        f = sse.sum(1) / n_obs
-        f = torch.where((valid < T - 1).any(1), torch.full_like(f, math.inf), f)
-        g = g.reshape(-1, dK) * mk / n_obs
-        return f, (g if A is None else g @ A)
-
-    def loss(q, rows):
-        sse, valid = native.rollout_score(x0, W_of(q, mk[rows]), lib, dt, int(steps_per_row), y, method, blowup)
-        f = sse.sum(1) / n_obs
+    def diverged(f, valid):
         return torch.where((valid < T - 1).any(1), torch.full_like(f, math.inf), f)
 
     with torch.no_grad():
-        f, g = loss_grad(p)
-        f_before = f.clone()
-        opt = sweep.BatchedLBFGS(p, 1.0, history_size=10)
-        iters = torch.zeros(U, dtype=torch.long, device=dev)
-        active = torch.isfinite(f) & (g.abs().amax(1) > 0)
-        c1, max_ls = 1e-4, 30
-        for _ in range(max_iter):
-            if not bool(active.any()):
-                break
-            dirn = opt.direction(g)
-            if A is None:
-                dirn = dirn * mk
-            gtd = (g * dirn).sum(1)
-            restart = gtd >= 0                                       # not a descent direction: steepest descent
-            dirn = torch.where(restart.unsqueeze(1), -g, dirn)
-            gtd = torch.where(restart, -(g * g).sum(1), gtd)
-            t = torch.where(opt.hist == 0, torch.clamp(1.0 / g.abs().sum(1), max=1.0), torch.ones_like(f))
-            searching, accepted = active.clone(), torch.zeros_like(active)
-            for _ls in range(max_ls):
-                idx = torch.nonzero(searching).flatten()
-                if idx.numel() == 0:
-                    break
-                trial = p[idx] + t[idx].unsqueeze(1) * dirn[idx]
-                ft = loss(trial, idx)
-                ok = ft <= f[idx] + c1 * t[idx] * gtd[idx]
-                accepted[idx[ok]] = True
-                searching[idx[ok]] = False
-                t[idx[~ok]] *= 0.5
-            active &= accepted                                        # no step length decreased the loss: done
-            p_new = torch.where(active.unsqueeze(1), p + t.unsqueeze(1) * dirn, p)
-            f_new, g_new = loss_grad(p_new)
-            f_new = torch.where(active, f_new, f)
-            g_new = torch.where(active.unsqueeze(1), g_new, g)
-            sv, yv = p_new - p, g_new - g
-            ys = (sv * yv).sum(1)
-            opt.push(yv, sv, active & (ys > 1e-10), ys)
-            iters += active.long()
-            small = (f - f_new) <= tol * f.abs()
-            p, f, g = p_new, f_new, g_new
-            active &= ~small & (g.abs().amax(1) > 0)
+        if not fit_ic:
+            def loss_grad(q):
+                sse, valid, g = native.rollout_score_grad(x0, W_of(q, mk), lib, dt, int(steps_per_row), y, method,
+                                                          blowup)
+                g = g.reshape(-1, dK) * mk / n_obs
+                return diverged(sse.sum(1) / n_obs, valid), (g if A is None else g @ A)
+
+            def loss(q, rows):
+                sse, valid = native.rollout_score(x0, W_of(q, mk[rows]), lib, dt, int(steps_per_row), y, method,
+                                                  blowup)
+                return diverged(sse.sum(1) / n_obs, valid)
+
+            p, f, f_before, iters = _lockstep_lbfgs(p, loss_grad, loss, max_iter, tol, mk if A is None else None)
+            sse_before, sse_after = f_before * n_obs, f * n_obs
+        else:
+            nc, n_ic = p.shape[1], _obs_counts(n_traj, T, d, True)[0]
+            x0d = x0.to(torch.float64).reshape(1, -1)
+            first_sse = []
+
+            def split(q):
+                return q[:, :nc], q[:, nc:]
+
+            def objective(q_ic, sse, valid):
+                r = q_ic - x0d
+                return diverged((sse.sum(1) + (r * r).sum(1)) / n_ic, valid), r
+
+            def loss_grad(q):
+                c, s = split(q)
+                sse, valid, g, gx = native.rollout_score_grad(s.view(-1, n_traj, d).float(), W_of(c, mk), lib, dt,
+                                                              int(steps_per_row), y, method, blowup, x0_grad=True)
+                if not first_sse:
+                    first_sse.append(diverged(sse.sum(1) / n_obs, valid) * n_obs)   # the fixed-start sse_before
+                f, r = objective(s, sse, valid)
+                g = g.reshape(-1, dK) * mk / n_ic
+                return f, torch.cat([g if A is None else g @ A, (gx.reshape(-1, n_traj * d) + 2 * r) / n_ic], 1)
+
+            def loss(q, rows):
+                c, s = split(q)
+                sse, valid = native.rollout_score(s.view(-1, n_traj, d).float(), W_of(c, mk[rows]), lib, dt,
+                                                  int(steps_per_row), y, method, blowup)
+                return objective(s, sse, valid)[0]
+
+            q0 = torch.cat([p, x0d.expand(U, -1)], 1)
+            dmask = torch.cat([mk, torch.ones_like(q0[:, nc:])], 1) if A is None else None
+            q, f, _, iters = _lockstep_lbfgs(q0, loss_grad, loss, max_iter, tol, dmask)
+            p, x0_hat = split(q)
+            sse_before = first_sse[0]
+            # a candidate that accepted no step is where it started: its sse is sse_before
+            sse_after = torch.where(iters > 0, f * n_ic, sse_before)
         out = dict(path)
         inv = inverse.to(dev)
         out["xi"] = (W_of(p, mk)[inv] * masks).to(W0.dtype)
@@ -819,9 +954,11 @@ def refine_path(regressor, path, x_fit, dt, steps_per_row=1, method='rk4', blowu
             nb = path["beta"].shape[1]
             out["beta"] = p[inv, :nb].to(path["beta"].dtype)
             out["const"] = p[inv, nb:].reshape(P, d, 1).to(path["const"].dtype)
-        out["sse_before"] = (f_before * n_obs)[inv].cpu()
-        out["sse_after"] = (f * n_obs)[inv].cpu()
+        out["sse_before"] = sse_before[inv].cpu()
+        out["sse_after"] = sse_after[inv].cpu()
         out["iterations"] = iters[inv].cpu()
+        if fit_ic:
+            out["x0"] = x0_hat[inv].reshape(P, n_traj, d).to(torch.float32)
     return out
 
 

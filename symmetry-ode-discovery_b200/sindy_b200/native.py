@@ -77,6 +77,11 @@ _SIGNATURES = {
     "sb_rollout_score_grad": (c_int, [c_void_p, c_int64, POINTER(_CLibrary), c_void_p, c_int, c_double, c_int64,
                                       c_int64, c_int, c_void_p, c_float, c_void_p, c_void_p, c_void_p, c_void_p, c_int64,
                                       c_void_p]),
+    "sb_rollout_score_ics": (c_int, [c_void_p, c_int, c_int64, POINTER(_CLibrary), c_void_p, c_int, c_double, c_int64,
+                                     c_int64, c_int, c_void_p, c_float, c_void_p, c_void_p, c_void_p]),
+    "sb_rollout_score_grad_ics": (c_int, [c_void_p, c_int, c_int64, POINTER(_CLibrary), c_void_p, c_int, c_double,
+                                          c_int64, c_int64, c_int, c_void_p, c_float, c_void_p, c_void_p, c_void_p,
+                                          c_void_p, c_void_p, c_int64, c_void_p]),
     "sb_wsindy_integrals": (c_int, [c_void_p, c_int64, c_int64, POINTER(_CLibrary), c_float, c_double, c_int,
                                     c_void_p, c_void_p, c_void_p]),
     "sb_wsindy_local_integrals": (c_int, [c_void_p, c_int64, c_int64, POINTER(_CLibrary), c_void_p, c_void_p, c_int,
@@ -539,15 +544,20 @@ def rollout(x0: torch.Tensor, w: torch.Tensor, lib: Library, dt: float, n_steps:
 
 
 def _score_args(x0, W, lib, dt, steps_per_row, y_obs, method, blowup):
-    """The argument checks and conversions shared by rollout_score and rollout_score_grad."""
-    x0f = _flat(_f32c(x0, "x0"), lib.dim, "x0")
-    n_ics, d = x0f.shape
+    """The argument checks and conversions shared by rollout_score and rollout_score_grad. x0 is (N, d), shared by all
+    models, or (M, N, d), one start set per model; returns x0 as (N, d) or (M, N, d) and whether it is per model."""
+    x0 = _f32c(x0, "x0")
+    per_model = x0.dim() == 3
+    x0f = x0 if per_model else _flat(x0, lib.dim, "x0")
+    n_ics, d = x0f.shape[-2:]
     dev = x0f.device
     W = _f32c(W, "W")
     if W.dim() == 2:
         W = W.unsqueeze(0)
     if W.dim() != 3 or W.shape[1:] != (d, lib.K):
         raise ValueError(f"W has shape {tuple(W.shape)}, expected (n_models, {d}, {lib.K})")
+    if per_model and (d != lib.dim or x0f.shape[0] != W.shape[0]):
+        raise ValueError(f"per-model x0 has shape {tuple(x0f.shape)}, expected ({W.shape[0]}, n_ics, {lib.dim})")
     y = _f32c(y_obs, "y_obs")
     if y.dim() != 3 or y.shape[1:] != (n_ics, d) or y.shape[0] < 1:
         raise ValueError(f"y_obs has shape {tuple(y.shape)}, expected (n_rows >= 1, {n_ics}, {d})")
@@ -562,44 +572,52 @@ def _score_args(x0, W, lib, dt, steps_per_row, y_obs, method, blowup):
         raise ValueError(f"dt must be positive, got {dt}")
     if blowup is not None and not blowup > 0:
         raise ValueError(f"blowup must be positive or None, got {blowup}")
-    return x0f, W, y, meth, dev
+    return x0f, per_model, W, y, meth, dev
 
 
 def rollout_score(x0: torch.Tensor, W: torch.Tensor, lib: Library, dt: float, steps_per_row: int, y_obs: torch.Tensor,
                   method: str = "rk4", blowup: Optional[float] = None) -> Tuple[torch.Tensor, torch.Tensor]:
     """Every model W[m] (M × d × K, already masked; one d × K model is M = 1) integrated in fp32 from every initial
-    condition x0 (N × d) and compared with y_obs (n_rows × N × d: the states after steps_per_row, 2·steps_per_row, ...
-    steps). Returns sse (M × N fp64, summed over the rows compared) and valid_rows (M × N int32: rows compared before
-    the first non-finite state or |x_j| > blowup; n_rows if none). The compared states are bit-identical to
-    rollout(x0, W[m], lib, dt, n_rows·steps_per_row, stride=steps_per_row, method). See sb_rollout_score."""
-    x0f, W, y, meth, dev = _score_args(x0, W, lib, dt, steps_per_row, y_obs, method, blowup)
-    n_ics = x0f.shape[0]
+    condition x0 (N × d, or M × N × d: model m starts from x0[m]) and compared with y_obs (n_rows × N × d: the states
+    after steps_per_row, 2·steps_per_row, ... steps). Returns sse (M × N fp64, summed over the rows compared) and
+    valid_rows (M × N int32: rows compared before the first non-finite state or |x_j| > blowup; n_rows if none). The
+    compared states are bit-identical to rollout(x0[m], W[m], lib, dt, n_rows·steps_per_row, stride=steps_per_row,
+    method). See sb_rollout_score_ics."""
+    x0f, per_model, W, y, meth, dev = _score_args(x0, W, lib, dt, steps_per_row, y_obs, method, blowup)
+    n_ics = x0f.shape[-2]
     n_models = W.shape[0]
     sse = torch.empty(n_models, n_ics, dtype=torch.float64, device=dev)
     valid = torch.empty(n_models, n_ics, dtype=torch.int32, device=dev)
     if n_models == 0 or n_ics == 0:
         return sse, valid
     with torch.cuda.device(dev):
-        _check(load().sb_rollout_score(x0f.data_ptr(), n_ics, ctypes.byref(lib.c()), W.data_ptr(), n_models, float(dt),
-                                       int(steps_per_row), y.shape[0], meth, y.data_ptr(),
-                                       0.0 if blowup is None else float(blowup), sse.data_ptr(), valid.data_ptr(),
-                                       _stream(dev)), "sb_rollout_score")
+        _check(load().sb_rollout_score_ics(x0f.data_ptr(), int(per_model), n_ics, ctypes.byref(lib.c()), W.data_ptr(),
+                                           n_models, float(dt), int(steps_per_row), y.shape[0], meth, y.data_ptr(),
+                                           0.0 if blowup is None else float(blowup), sse.data_ptr(), valid.data_ptr(),
+                                           _stream(dev)), "sb_rollout_score_ics")
     return sse, valid
 
 
 def rollout_score_grad(x0: torch.Tensor, W: torch.Tensor, lib: Library, dt: float, steps_per_row: int,
-                       y_obs: torch.Tensor, method: str = "rk4", blowup: Optional[float] = None):
+                       y_obs: torch.Tensor, method: str = "rk4", blowup: Optional[float] = None, x0_grad: bool = False,
+                       w_grad: bool = True):
     """rollout_score and the gradient of its scores: returns (sse, valid_rows, grad) with sse / valid_rows
     bit-identical to rollout_score's and grad (M × d × K fp64) = ∂/∂W[m] of sse[m].sum(), each pair's SSE over the rows
-    it compared (discrete adjoint of the fp32 recurrence). See sb_rollout_score_grad."""
-    x0f, W, y, meth, dev = _score_args(x0, W, lib, dt, steps_per_row, y_obs, method, blowup)
-    n_ics, d = x0f.shape
+    it compared (discrete adjoint of the fp32 recurrence). With x0_grad it returns (sse, valid_rows, grad, grad_x0),
+    grad_x0 (M × N × d fp64) = ∂sse[m, n]/∂x0 of the pair (x0 shared or per model as in rollout_score); w_grad=False
+    then gives grad = None and runs the start-only kernel variant. See sb_rollout_score_grad_ics."""
+    if not (w_grad or x0_grad):
+        raise ValueError("rollout_score_grad needs w_grad or x0_grad")
+    x0f, per_model, W, y, meth, dev = _score_args(x0, W, lib, dt, steps_per_row, y_obs, method, blowup)
+    n_ics, d = x0f.shape[-2:]
     n_models = W.shape[0]
     sse = torch.empty(n_models, n_ics, dtype=torch.float64, device=dev)
     valid = torch.empty(n_models, n_ics, dtype=torch.int32, device=dev)
-    grad = torch.zeros(n_models, d, lib.K, dtype=torch.float64, device=dev)
+    grad = torch.zeros(n_models, d, lib.K, dtype=torch.float64, device=dev) if w_grad else None
+    gx0 = torch.zeros(n_models, n_ics, d, dtype=torch.float64, device=dev) if x0_grad else None
+    done = (sse, valid, grad, gx0) if x0_grad else (sse, valid, grad)
     if n_models == 0 or n_ics == 0:
-        return sse, valid, grad
+        return done
     sl = load()
     nb = int(sl.sb_rollout_score_grad_workspace_bytes(n_ics, ctypes.byref(lib.c()), n_models, int(steps_per_row),
                                                       y.shape[0]))
@@ -607,11 +625,12 @@ def rollout_score_grad(x0: torch.Tensor, W: torch.Tensor, lib: Library, dt: floa
         _check(nb, "sb_rollout_score_grad_workspace_bytes")
     ws = torch.empty(max(nb, 1), dtype=torch.uint8, device=dev)
     with torch.cuda.device(dev):
-        _check(sl.sb_rollout_score_grad(x0f.data_ptr(), n_ics, ctypes.byref(lib.c()), W.data_ptr(), n_models,
-                                        float(dt), int(steps_per_row), y.shape[0], meth, y.data_ptr(),
-                                        0.0 if blowup is None else float(blowup), sse.data_ptr(), valid.data_ptr(),
-                                        grad.data_ptr(), ws.data_ptr(), nb, _stream(dev)), "sb_rollout_score_grad")
-    return sse, valid, grad
+        _check(sl.sb_rollout_score_grad_ics(x0f.data_ptr(), int(per_model), n_ics, ctypes.byref(lib.c()), W.data_ptr(),
+                                            n_models, float(dt), int(steps_per_row), y.shape[0], meth, y.data_ptr(),
+                                            0.0 if blowup is None else float(blowup), sse.data_ptr(), valid.data_ptr(),
+                                            _ptr(grad), _ptr(gx0), ws.data_ptr(), nb, _stream(dev)),
+               "sb_rollout_score_grad_ics")
+    return done
 
 
 def wsindy_integrals(x: torch.Tensor, lib: Library, dt: float, t_max: float, n_test: int = 50):
