@@ -312,6 +312,38 @@ int sb_rollout_score_grad_ics(const float* x0, int x0_per_model, int64_t n_ics, 
                               const float* y_obs, float blowup, double* sse, int32_t* valid_rows, double* grad,
                               double* grad_x0, void* ws, int64_t ws_bytes, void* stream);
 
+/* Most tangent columns of sb_rollout_score_gn: n_params, plus d when the start blocks are requested. (3,5)'s full
+ * d·K = 168 coefficients and 3 starts need 171. */
+#define SB_GN_MAX_COLS 176
+
+/* Gauss–Newton information of the fused scores (coefficient standard errors of a trajectory refit, Cov(θ) ≈
+ * σ̂²·(JᵀJ)⁻¹): with the arguments of sb_rollout_score_ics, sse and valid_rows are bit-identical to what it returns, and
+ * for the n_params coefficients params[m, ·] of each model (int32 indices into the flat d×K W_m, −1 = padding) with
+ * J = ∂x_r/∂θ at every compared row r ≤ valid_rows of a pair and E = x_r − y_r:
+ *   jtj (n_models × n_params × n_params fp64, symmetric) = Σ_n Σ_r JᵀJ,   jtr (n_models × n_params fp64) = Σ_n Σ_r JᵀE.
+ * With jtj_px, jtj_xx and jtr_x (all given or all NULL) the start x0 of each pair is a parameter too, J_x = ∂x_r/∂x0:
+ *   jtj_px (n_models × n_ics × n_params × d) = Σ_r JᵀJ_x,  jtj_xx (n_models × n_ics × d × d) = Σ_r J_xᵀJ_x,
+ *   jtr_x (n_models × n_ics × d) = Σ_r J_xᵀE,  per pair.
+ * J is the tangent-linear of the fp32 recurrence that was scored (same step, same right-hand side), so it is its exact
+ * derivative up to fp32 rounding. Rows and columns of padded indices, and every block of a pair with valid_rows = 0,
+ * are exact zeros. Each row's products are summed in fp32 over a block's pairs and added to fp64 sums in a fixed order
+ * with no atomics on values: a model's outputs have the same bits alone, in any batch, in any model order and on every
+ * repeat (for the same n_params and n_ics). It costs about n_params'·2d² + d library sweeps per RK4 stage and pair and
+ * n_params'²·d per compared row, n_params' = n_params (+ d).
+ * ws: device workspace of at least sb_rollout_score_gn_workspace_bytes(n_ics, lib, n_models, n_params, x0_blocks)
+ * bytes (one fp64 row of n_params(n_params+1)/2 + n_params sums per model and block of at most 32 per model); it need
+ * not be initialised; SB_ERR_WORKSPACE if it is shorter. SB_ERR_INVALID for the size and pointer errors of
+ * sb_rollout_score_ics, n_params < 1, only some of the start outputs given, or an index outside [−1, d·K) (params are
+ * read back to the host for this check: the call synchronises the stream); SB_ERR_UNSUPPORTED for n_params (+ d) above
+ * SB_GN_MAX_COLS. n_ics = 0 sets jtj and jtr to 0. The workspace size is negative (a status) for invalid sizes. */
+int64_t sb_rollout_score_gn_workspace_bytes(int64_t n_ics, const sb_library* lib, int n_models, int n_params,
+                                            int x0_blocks);
+int sb_rollout_score_gn(const float* x0, int x0_per_model, int64_t n_ics, const sb_library* lib, const float* w,
+                        int n_models, const int32_t* params, int n_params, double dt, int64_t steps_per_row,
+                        int64_t n_rows, int method, const float* y_obs, float blowup, double* sse,
+                        int32_t* valid_rows, double* jtj, double* jtr, double* jtj_px, double* jtj_xx, double* jtr_x,
+                        void* ws, int64_t ws_bytes, void* stream);
+
 /* WSINDy weak-form integrals with trigonometric test functions (`sindy.py:332-347,361-362`):
  *   V[j,t]  = dt·sqrt(2/T)·sin((j+1)π t/T),  V'[j,t] = dt·sqrt(2/T)·(j+1)π/T·cos((j+1)π t/T),  t = t_idx·dt
  *   G[traj,j,k] = sum_t V[j,t]·Θ_k(x[traj,t]),   b[traj,j,i] = −sum_t V'[j,t]·x[traj,t,i]

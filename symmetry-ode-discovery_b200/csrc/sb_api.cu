@@ -479,6 +479,83 @@ int sb_rollout_score_grad_ics(const float* x0, int x0_per_model, int64_t n_ics, 
                             (cudaStream_t)stream);
 }
 
+namespace {
+int check_gn_params(const LibTab& t, int n_params, int x0_blocks) {
+  if (n_params < 1) { set_error("n_params=%d is not positive", n_params); return SB_ERR_INVALID; }
+  if (n_params > SB_GN_MAX_COLS - (x0_blocks ? t.d : 0)) {
+    set_error("n_params=%d%s exceeds SB_GN_MAX_COLS=%d", n_params, x0_blocks ? " plus the start columns" : "",
+              SB_GN_MAX_COLS);
+    return SB_ERR_UNSUPPORTED;
+  }
+  return SB_OK;
+}
+}  // namespace
+
+int64_t sb_rollout_score_gn_workspace_bytes(int64_t n_ics, const sb_library* lib, int n_models, int n_params,
+                                            int x0_blocks) {
+  LibTab t;
+  SB_TRY(build_table(lib, &t));
+  SB_TRY(check_score_sizes(n_ics, n_models, 1, 1));
+  SB_TRY(check_gn_params(t, n_params, x0_blocks));
+  const int64_t b = rollout_score_gn_workspace_bytes(n_ics, t, n_models, n_params, x0_blocks != 0);
+  if (b < 0) { set_error("rollout_score_gn workspace size overflows int64"); return SB_ERR_INVALID; }
+  return b;
+}
+
+int sb_rollout_score_gn(const float* x0, int x0_per_model, int64_t n_ics, const sb_library* lib, const float* w,
+                        int n_models, const int32_t* params, int n_params, double dt, int64_t steps_per_row,
+                        int64_t n_rows, int method, const float* y_obs, float blowup, double* sse,
+                        int32_t* valid_rows, double* jtj, double* jtr, double* jtj_px, double* jtj_xx, double* jtr_x,
+                        void* ws, int64_t ws_bytes, void* stream) {
+  LibTab t;
+  SB_TRY(build_table(lib, &t));
+  SB_TRY(check_x0_per_model(x0_per_model));
+  SB_TRY(check_score_sizes(n_ics, n_models, steps_per_row, n_rows));
+  if (method != SB_EULER && method != SB_RK4) { set_error("unknown method %d", method); return SB_ERR_INVALID; }
+  if (!(dt > 0.0)) { set_error("dt=%g is not positive", dt); return SB_ERR_INVALID; }
+  SB_TRY(check_ptr(x0, "x0")); SB_TRY(check_ptr(w, "w")); SB_TRY(check_ptr(y_obs, "y_obs"));
+  SB_TRY(check_ptr(params, "params"));
+  SB_TRY(check_ptr(sse, "sse")); SB_TRY(check_ptr(valid_rows, "valid_rows"));
+  SB_TRY(check_ptr(jtj, "jtj")); SB_TRY(check_ptr(jtr, "jtr"));
+  const int n_x = (jtj_px != nullptr) + (jtj_xx != nullptr) + (jtr_x != nullptr);
+  if (n_x != 0 && n_x != 3) {
+    set_error("jtj_px, jtj_xx and jtr_x must all be given or all be NULL");
+    return SB_ERR_INVALID;
+  }
+  SB_TRY(check_gn_params(t, n_params, n_x != 0));
+  SB_TRY(check_ptr(ws, "workspace"));
+  const int64_t need = rollout_score_gn_workspace_bytes(n_ics, t, n_models, n_params, n_x != 0);
+  if (need < 0) { set_error("rollout_score_gn workspace size overflows int64"); return SB_ERR_INVALID; }
+  if (ws_bytes < need) {
+    set_error("workspace too small: %lld < %lld bytes", (long long)ws_bytes, (long long)need);
+    return SB_ERR_WORKSPACE;
+  }
+  cudaStream_t s = (cudaStream_t)stream;
+  {   // every index in [−1, d·K)
+    const size_t n = (size_t)n_models * n_params;
+    int32_t* h = (int32_t*)malloc(n * sizeof(int32_t));
+    if (!h) { set_error("out of host memory"); return SB_ERR_INVALID; }
+    cudaError_t e = cudaMemcpyAsync(h, params, n * sizeof(int32_t), cudaMemcpyDefault, s);
+    if (e == cudaSuccess) e = cudaStreamSynchronize(s);
+    if (e != cudaSuccess) { free(h); return cuda_fail(e, "copying params to the host"); }
+    for (size_t i = 0; i < n; ++i)
+      if (h[i] < -1 || h[i] >= t.d * t.K) {
+        set_error("params[%lld]=%d is outside [-1, %d)", (long long)i, h[i], t.d * t.K);
+        free(h);
+        return SB_ERR_INVALID;
+      }
+    free(h);
+  }
+  if (n_ics == 0) {   // no pair: empty sums
+    SB_CUDA_TRY(cudaMemsetAsync(jtj, 0, sizeof(double) * (size_t)n_models * n_params * n_params, s));
+    SB_CUDA_TRY(cudaMemsetAsync(jtr, 0, sizeof(double) * (size_t)n_models * n_params, s));
+    return SB_OK;
+  }
+  return rollout_score_gn(x0, x0_per_model ? n_ics * t.d : 0, n_ics, t, w, n_models, params, n_params, dt,
+                          steps_per_row, n_rows, method, y_obs, blowup, sse, valid_rows, jtj, jtr, jtj_px, jtj_xx,
+                          jtr_x, ws, ws_bytes, s);
+}
+
 int sb_wsindy_integrals(const float* x, int64_t n_traj, int64_t T, const sb_library* lib, float dt,
                         double t_max, int n_test, double* G, double* b, void* stream) {
   LibTab t;

@@ -348,6 +348,16 @@ int rollout_score_grad(const float* x0, int64_t x0_model_stride, int64_t n_ics, 
                        int n_models, double dt, int64_t steps_per_row, int64_t n_rows, int method, const float* y_obs,
                        float blowup, double* sse, int32_t* valid_rows, double* grad, double* grad_x0, void* ws,
                        int64_t ws_bytes, cudaStream_t s);
+// the same scores and the Gauss–Newton information of the listed coefficients (params: n_models × n_params indices
+// into d×K, −1 padding) and, when jtj_px is given, of each pair's start, from tangent-linear rollouts. Arguments
+// validated by the caller (n_params + start columns ≤ SB_GN_MAX_COLS). The workspace size is -1 when it does not fit
+// in int64.
+int64_t rollout_score_gn_workspace_bytes(int64_t n_ics, const LibTab& t, int n_models, int n_params, int x0_blocks);
+int rollout_score_gn(const float* x0, int64_t x0_model_stride, int64_t n_ics, const LibTab& t, const float* w,
+                     int n_models, const int32_t* params, int n_params, double dt, int64_t steps_per_row,
+                     int64_t n_rows, int method, const float* y_obs, float blowup, double* sse, int32_t* valid_rows,
+                     double* jtj, double* jtr, double* jtj_px, double* jtj_xx, double* jtr_x, void* ws,
+                     int64_t ws_bytes, cudaStream_t s);
 
 // WSINDy integrals
 int wsindy_integrals(const float* x, int64_t n_traj, int64_t T, const LibTab& t, float dt, double t_max,

@@ -536,6 +536,7 @@ template <int D, int PC>
 struct SpecGrad {
   static constexpr bool kStatic = true;
   static constexpr int DN = D, K = LibCode<D, PC>::K, ACC = D * K, KQ = SharedW<K>::KQ;
+  static constexpr int THL = 1;   // Θ row of jac: in shared memory
   const float4* sw;
   __device__ __forceinline__ int dim() const { return D; }
   __device__ __forceinline__ int dk() const { return D * K; }
@@ -563,6 +564,29 @@ struct SpecGrad {
     static_for<0, D>([&](auto j) { xb[j] = 0.f; });
     reverse_lib<D, PC>(y, m, mb, xb);
   }
+  // J_h(y) row by row, row i = J_Θ(y)ᵀW_i (one reverse sweep each), and Θ(y) into th (a per-thread shared row). The
+  // sweeps read Θ back from that row: K values held in registers through d sweeps spill at (3,5)
+  __device__ __forceinline__ void jac(const float (&y)[D], float (&jh)[D][D], float* th, int off) const {
+    const float* w = reinterpret_cast<const float*>(sw + off);
+    {
+      float m[K];
+      expand_lib<D, PC>(y, m);
+      static_for<0, K>([&](auto k) { th[k] = m[k]; });
+    }
+    asm volatile("" ::: "memory");   // no store-to-load forwarding: the sweeps load Θ from shared memory
+    const float (&m)[K] = *reinterpret_cast<const float (*)[K]>(th);
+    // one sweep at a time: unrolled, the d independent sweeps are interleaved with d·K cotangents live
+#pragma unroll 1
+    for (int i = 0; i < D; ++i) {
+      float mb[K], xb[D];
+      static_for<0, K>([&](auto k) { mb[k] = w[i * KQ * 4 + k]; });
+      static_for<0, D>([&](auto j) { xb[j] = 0.f; });
+      reverse_lib<D, PC>(y, m, mb, xb);
+      static_for<0, D>([&](auto ic) {
+        if (ic == i) static_for<0, D>([&](auto j) { jh[ic][j] = xb[j]; });
+      });
+    }
+  }
 };
 
 // runtime-table library: GenRhs with the model's W in global memory
@@ -570,6 +594,7 @@ template <int KMAX>
 struct GenGrad {
   static constexpr bool kStatic = false;
   static constexpr int DN = SB_MAX_DIM, ACC = SB_MAX_DIM * KMAX;
+  static constexpr int THL = KMAX;   // Θ row of jac: per-thread local array
   const LibTab& t;
   const float* w;
   __device__ __forceinline__ int dim() const { return t.d; }
@@ -593,6 +618,19 @@ struct GenGrad {
 #pragma unroll
     for (int j = 0; j < DN; ++j) xb[j] = 0.f;
     reverse_table(t, y, m, mb, xb);
+  }
+  __device__ __forceinline__ void jac(const float (&y)[DN], float (&jh)[DN][DN], float* th, int) const {
+    expand_table(t, y, th);
+    float mb[KMAX], xb[DN];
+    for (int i = 0; i < t.d; ++i) {
+      for (int k = 0; k < t.K; ++k) mb[k] = __ldg(w + i * t.K + k);
+#pragma unroll
+      for (int j = 0; j < DN; ++j) xb[j] = 0.f;
+      reverse_table(t, y, th, mb, xb);
+      // jh is in local memory here (DN = SB_MAX_DIM): index the row directly
+#pragma unroll
+      for (int j = 0; j < DN; ++j) jh[i][j] = xb[j];
+    }
   }
 };
 
@@ -811,6 +849,280 @@ __global__ void __launch_bounds__(256) grad_sum_kernel(const double* partial, in
   grad[i] = v;
 }
 
+// ---- Gauss–Newton information of the scores -------------------------------------------------------------------------
+// For the listed coefficients θ of each model (indices into the flat d×K W, −1 = padding) and optionally each pair's
+// start: J = ∂x_r/∂(θ, x0) at every compared row r of the pair, F_θθ = Σ_pairs Σ_r JθᵀJθ, g_θ = Σ JθᵀE (E = x_r − y_r),
+// and per pair F_θx = Σ_r JθᵀJx, F_xx = Σ_r JxᵀJx, g_x = Σ_r JxᵀE. J is carried forward with the states: the tangent-
+// linear of the same fp32 recurrence the scorer runs (not of the continuous sensitivity equation), in Odeint::step's
+// stage order,
+//   S' = S + sdt·(((K1 + 2K2) + 2K3) + K4),  K_s = J_h(y_s)·S_s + E(Θ(y_s)),  S_1 = S, S_2 = S + hdt·K1, ...
+// where coefficient (i, k) has the source column e_i·Θ_k(y_s) and a start column none; S(0) = [0 | I_d]. J_h(y_s) is
+// formed from d value-only reverse sweeps of the library (row i = J_Θᵀ W_i), Θ(y_s) goes to a per-thread shared row.
+//   layout:  grid = (IC-group blocks, models). A block holds G pairs × T chunks of C directions: thread (g, t)
+//            integrates pair g's state (repeated across its chunks) and directions t·C .. t·C + C − 1 of
+//            P' = n_params + (d if start blocks). The primal is the scorer's loop, so sse / valid are its bits.
+//   rows:    at each compared row every thread writes its d × C slice of J and chunk 0 the residual to shared memory
+//            (a pair that has stopped, or is past the last IC, writes zeros, so it adds exact zeros); after a barrier
+//            each thread adds, for the entries it owns, the fp32 sum over the block's pairs (in pair order) of that
+//            row's products to an fp64 accumulator in shared memory: the upper triangle of F_θθ and g_θ, and the per-pair
+//            blocks. So no fp32 sum spans more than one row.
+//   sums:    a block walks IC groups blockIdx.x, blockIdx.x + gridDim.x, ... in order; gridDim.x depends only on n_ics
+//            and P', never on the number of models. Its θ sums go to one fp64 row per (model, block), gn_sum_kernel adds
+//            those in block order. The per-pair blocks have one writer each. A model's outputs have the same bits
+//            alone, in any batch, in any model order and on every repeat (for the same n_params).
+// tangent directions per thread: 8, or 4 for a specialised library of K ≥ 32 columns ((3,5): 255 registers and 644
+// bytes of spill stores at 8, none at 4)
+template <int K> constexpr int gn_chunk() { return K >= 32 ? 4 : 8; }
+constexpr int kGnC = 8;               // the runtime-table kernels
+constexpr int kGnThreads = 128;       // block target: G = max(1, kGnThreads / T) pairs of T chunks
+constexpr int kGnMaxBlocks = 32;      // IC-group blocks per model
+constexpr int kGnMaxCols = SB_GN_MAX_COLS;
+static_assert(kGnMaxCols % 8 == 0, "whole chunks");
+
+struct GnArgs {
+  ScoreArgs s;            // this launch's models, as the scorer gets them
+  const int32_t* params;  // [model][P], from this launch's first model
+  int P, X, T, G;         // listed coefficients, start columns (d or 0), chunks per pair, pairs per block
+  int64_t n_groups;       // ⌈n_ics / G⌉
+  double* partial;        // [model][block][P(P+1)/2 + P], from this launch's first model
+  double* jtj_px;         // [model][ic][P][d], from this launch's first model (X only)
+  double* jtj_xx;         // [model][ic][d][d]
+  double* jtr_x;          // [model][ic][d]
+};
+
+// shared memory of one block: [θ sums: P(P+1)/2 + P fp64][pair sums: G·(P·d + d² + d) fp64 when X]
+// [J slices: G·d·T·C fp32][residuals: G·d fp32][Θ rows: threads·(K|1) fp32, specialised libraries only]
+__host__ __device__ inline int64_t gn_tri(int P) { return (int64_t)P * (P + 1) / 2; }
+__host__ __device__ inline int64_t gn_pair_elems(int P, int d) { return (int64_t)P * d + d * d + d; }
+
+template <int C, class G>
+__device__ __forceinline__ void gn_body(const G& g, int method, const GnArgs& a, int K) {
+  extern __shared__ double gn_smem[];
+  constexpr int DN = G::DN;
+  const int d = g.dim(), P = a.P, NG = a.G, nt = blockDim.x, tid = threadIdx.x;
+  const int gp = tid / a.T, ch = tid % a.T, cols = a.T * C;
+  const int tri = (int)gn_tri(P), PE = (int)gn_pair_elems(P, d);   // < 2^31 below SB_GN_MAX_COLS
+  const ScoreArgs& sa = a.s;
+  const int64_t model = blockIdx.y, N = sa.n_ics, spr = sa.steps_per_row;
+  double* acc = gn_smem;
+  double* pacc = acc + tri + P;
+  float* jsh = reinterpret_cast<float*>(pacc + (a.X ? NG * PE : 0));
+  float* esh = jsh + NG * d * cols;
+  float* th;
+  float thl[G::THL];
+  if constexpr (G::kStatic) th = esh + NG * d + tid * (K | 1);
+  else th = thl;
+  for (int e = tid; e < tri + P; e += nt) acc[e] = 0.0;
+  if (a.X)
+    for (int e = tid; e < NG * PE; e += nt) pacc[e] = 0.0;
+
+  // this thread's directions: code = component << 16 | column of a listed coefficient, −1 for a start column or padding
+  const int32_t* prm = a.params + model * P;
+  int code[C];
+#pragma unroll
+  for (int c = 0; c < C; ++c) {
+    const int q = ch * C + c;
+    const int p = q < P ? prm[q] : -1;
+    code[c] = p < 0 ? -1 : (p / K) << 16 | (p % K);
+  }
+  const Odeint<float> ode(sa.dt);
+  const int n_stage = method == SB_EULER ? 1 : 4;
+  float* Jg = jsh + gp * d * cols;
+
+  for (int64_t grp = blockIdx.x; grp < a.n_groups; grp += gridDim.x) {
+    const int64_t ic = grp * NG + gp;
+    const bool live = ic < N;
+    float x[DN], S[C][DN];
+#pragma unroll
+    for (int j = 0; j < DN; ++j) x[j] = (live && j < d) ? sa.x0[model * sa.x0_model_stride + ic * d + j] : 0.f;
+#pragma unroll
+    for (int c = 0; c < C; ++c) {
+      const int q = ch * C + c - P;   // start column q: S(0) = e_q
+#pragma unroll
+      for (int j = 0; j < DN; ++j) S[c][j] = (a.X && q == j) ? 1.f : 0.f;
+    }
+    bool track = live;
+    double sse = 0.0;
+    int64_t valid = sa.n_rows, row = 0, s = 0;
+    for (;;) {
+      if (track) {
+        for (int64_t q = 0; q < spr; ++q) {
+          const int off = (int)(++s & sa.opaque);
+          float acc_t[C][DN], dy[C][DN], y[DN], k[DN], kacc[DN], jh[DN][DN];
+#pragma unroll
+          for (int j = 0; j < DN; ++j) y[j] = x[j];
+#pragma unroll
+          for (int c = 0; c < C; ++c)
+#pragma unroll
+            for (int j = 0; j < DN; ++j) dy[c][j] = S[c][j];
+          // one copy of the stage: J_h and the library sweeps inlined four times do not fit the register file at (3,5)
+#pragma unroll 1
+          for (int st = 0; st < n_stage; ++st) {
+            g.jac(y, jh, th, off);
+            g.eval(y, k, off);
+            const float wgt = (st == 1 || st == 2) ? 2.f : 1.f;
+            const float hn = st == 2 ? ode.dt : ode.hdt;   // from this stage to the next stage's state
+#pragma unroll
+            for (int c = 0; c < C; ++c) {
+              const int comp = code[c] >> 16;   // −1: no source
+              const float src = th[code[c] < 0 ? 0 : code[c] & 0xffff];
+              float v[DN];
+#pragma unroll
+              for (int i = 0; i < DN; ++i) {
+                v[i] = i == comp ? src : 0.f;
+#pragma unroll
+                for (int j = 0; j < DN; ++j)
+                  if (i < d && j < d) v[i] = fmaf(jh[i][j], dy[c][j], v[i]);
+              }
+#pragma unroll
+              for (int i = 0; i < DN; ++i) {
+                acc_t[c][i] = st == 0 ? v[i] : fmaf(wgt, v[i], acc_t[c][i]);
+                dy[c][i] = fmaf(hn, v[i], S[c][i]);
+              }
+            }
+            // the primal: Odeint::step's operations in its order
+#pragma unroll
+            for (int j = 0; j < DN; ++j) {
+              kacc[j] = st == 0 ? k[j] : add_rn(kacc[j], st == 3 ? k[j] : mul_rn(2.f, k[j]));
+              y[j] = add_rn(x[j], mul_rn(hn, k[j]));
+            }
+          }
+          const float h = method == SB_EULER ? ode.dt : ode.sdt;
+#pragma unroll
+          for (int j = 0; j < DN; ++j) {
+            x[j] = add_rn(x[j], mul_rn(h, kacc[j]));
+#pragma unroll
+            for (int c = 0; c < C; ++c) S[c][j] = fmaf(h, acc_t[c][j], S[c][j]);
+          }
+        }
+        if (!score_row<DN>(x, d, sa.y_obs + (row * N + ic) * d, sa.blowup, sse)) { track = false; valid = row; }
+      }
+      // this row's slice of J and the residual
+      for (int i = 0; i < d; ++i) {
+#pragma unroll
+        for (int c = 0; c < C; ++c) {
+          float v = 0.f;
+#pragma unroll
+          for (int j = 0; j < DN; ++j)
+            if (j == i) v = S[c][j];
+          Jg[i * cols + ch * C + c] = track ? v : 0.f;
+        }
+      }
+      if (ch == 0) {
+        const float* yr = sa.y_obs + (row * N + (live ? ic : 0)) * d;
+#pragma unroll
+        for (int j = 0; j < DN; ++j)
+          if (j < d) esh[gp * d + j] = track ? x[j] - __ldg(yr + j) : 0.f;
+      }
+      const int any = __syncthreads_or(track);
+      // F_θθ upper triangle (row-major: row a holds b = a..P−1) and g_θ
+      {
+        int ra = 0, cb = tid;
+        while (cb >= P && ra < P) { ++ra; cb += ra - P; }
+        for (int e = tid; e < tri; e += nt) {
+          float v = 0.f;
+          for (int q = 0; q < NG; ++q)
+            for (int i = 0; i < d; ++i) {
+              const float* r = jsh + (q * d + i) * cols;
+              v = fmaf(r[ra], r[cb], v);
+            }
+          acc[e] += (double)v;
+          cb += nt;
+          while (cb >= P && ra < P) { ++ra; cb += ra - P; }
+        }
+        for (int e = tid; e < P; e += nt) {
+          float v = 0.f;
+          for (int q = 0; q < NG; ++q)
+            for (int i = 0; i < d; ++i) v = fmaf(jsh[(q * d + i) * cols + e], esh[q * d + i], v);
+          acc[tri + e] += (double)v;
+        }
+      }
+      if (a.X) {
+        for (int e = tid; e < NG * PE; e += nt) {
+          const int q = e / PE, r = e - q * PE;
+          const float* Jq = jsh + q * d * cols;
+          int c1, c2 = -1;   // column pair, or c2 = −1: the residual
+          if (r < P * d) { c1 = r / d; c2 = P + r % d; }
+          else if (r < P * d + d * d) { c1 = P + (r - P * d) / d; c2 = P + (r - P * d) % d; }
+          else c1 = P + r - P * d - d * d;
+          float v = 0.f;
+          for (int i = 0; i < d; ++i) v = fmaf(Jq[i * cols + c1], c2 < 0 ? esh[q * d + i] : Jq[i * cols + c2], v);
+          pacc[e] += (double)v;
+        }
+      }
+      __syncthreads();
+      if (++row == sa.n_rows || !any) break;
+    }
+    if (live && ch == 0) {
+      sa.sse[model * N + ic] = sse;
+      sa.valid[model * N + ic] = (int32_t)valid;
+    }
+    if (a.X) {   // the group's per-pair blocks, by the threads that own them (so no barrier)
+      for (int e = tid; e < NG * PE; e += nt) {
+        const int q = e / PE, r = e - q * PE;
+        const int64_t icq = grp * NG + q, pr = model * N + icq;
+        if (icq < N) {
+          if (r < P * d) a.jtj_px[pr * P * d + r] = prm[r / d] < 0 ? 0.0 : pacc[e];
+          else if (r < P * d + d * d) a.jtj_xx[pr * d * d + r - P * d] = pacc[e];
+          else a.jtr_x[pr * d + r - P * d - d * d] = pacc[e];
+        }
+        pacc[e] = 0.0;
+      }
+    }
+  }
+  double* part = a.partial + (model * gridDim.x + blockIdx.x) * (tri + P);
+  for (int e = tid; e < tri + P; e += nt) part[e] = acc[e];
+}
+
+template <int D, int PC, int METHOD>
+__global__ void __launch_bounds__(kGnThreads, 1) rollout_gn_spec_kernel(GnArgs a) {
+  using G = SpecGrad<D, PC>;
+  constexpr int K = G::K, KQ = G::KQ;
+  __shared__ float4 sw[D * KQ];
+  {
+    const float* wm = a.s.w + (int64_t)blockIdx.y * (D * K);
+    float* s = reinterpret_cast<float*>(sw);
+    for (int q = threadIdx.x; q < D * KQ * 4; q += blockDim.x) {
+      const int i = q / (KQ * 4), c = q % (KQ * 4);
+      s[q] = c < K ? wm[i * K + c] : 0.f;
+    }
+  }
+  __syncthreads();
+  gn_body<gn_chunk<K>()>(G{sw}, METHOD, a, K);
+}
+
+template <int KMAX>
+__global__ void __launch_bounds__(kGnThreads) rollout_gn_gen_kernel(LibTab t, int method, GnArgs a) {
+  gn_body<kGnC>(GenGrad<KMAX>{t, a.s.w + (int64_t)blockIdx.y * t.d * t.K}, method, a, t.K);
+}
+
+// jtj[m] (P × P, both triangles from the same sums) and jtr[m]: Σ_b partial[m, b, ·] in block order; rows and columns of
+// padded indices are exact zeros
+__global__ void __launch_bounds__(256) gn_sum_kernel(const double* partial, int64_t n_blocks, int P,
+                                                     const int32_t* params, int64_t n, double* jtj, double* jtr) {
+  const int64_t i = (int64_t)blockIdx.x * 256 + threadIdx.x;
+  if (i >= n) return;
+  const int64_t per = (int64_t)P * P + P, tri = gn_tri(P), m = i / per, r = i % per;
+  const int32_t* prm = params + m * P;
+  int64_t e;
+  bool dead;
+  if (r < (int64_t)P * P) {
+    const int a = (int)(r / P), b = (int)(r % P), lo = a < b ? a : b, hi = a < b ? b : a;
+    e = (int64_t)lo * P - (int64_t)lo * (lo - 1) / 2 + (hi - lo);
+    dead = prm[a] < 0 || prm[b] < 0;
+  } else {
+    e = tri + (r - (int64_t)P * P);
+    dead = prm[r - (int64_t)P * P] < 0;
+  }
+  double v = 0.0;
+  if (!dead) {
+    const double* p = partial + m * n_blocks * (tri + P) + e;
+    for (int64_t b = 0; b < n_blocks; ++b) v += p[b * (tri + P)];
+  }
+  if (r < (int64_t)P * P) jtj[m * P * P + r] = v;
+  else jtr[m * P + r - (int64_t)P * P] = v;
+}
+
 // ---- launch ---------------------------------------------------------------------------------------------------------
 // The specialised libraries as (D, library code PC): the polynomials and, for config 3 (Lotka-Volterra in canonical
 // coordinates, `data_utils/lotka.py:33-41`), degree 2 + exp. Everything else runs on the runtime table.
@@ -902,6 +1214,57 @@ int launch_grad(const LibTab& t, const GradArgs& a, int method, int n_models, cu
   return SB_OK;
 }
 
+// The Gauss–Newton block shape and shared memory for P listed coefficients and X start columns, as gn_body lays it out
+struct GnShape {
+  int T, G, threads;
+  int64_t n_groups, blocks, smem;
+};
+GnShape gn_shape(int64_t n_ics, const LibTab& t, int P, int X, bool spec) {
+  GnShape g;
+  const int C = spec && t.K >= 32 ? 4 : kGnC;   // gn_chunk
+  g.T = (P + X + C - 1) / C;
+  g.G = kGnThreads / g.T > 1 ? kGnThreads / g.T : 1;
+  g.threads = g.G * g.T;
+  g.n_groups = (n_ics + g.G - 1) / g.G;
+  g.blocks = g.n_groups < kGnMaxBlocks ? g.n_groups : kGnMaxBlocks;
+  g.smem = 8 * (gn_tri(P) + P + (X ? g.G * gn_pair_elems(P, t.d) : 0)) +
+           4 * ((int64_t)g.G * t.d * g.T * C + g.G * t.d + (spec ? (int64_t)g.threads * (t.K | 1) : 0));
+  return g;
+}
+
+bool gn_spec(const LibTab& t) {
+#define X(D, PC) \
+  if (lib_matches<D, PC>(t)) return true;
+  SB_SPEC_SHAPES(X)
+#undef X
+  return false;
+}
+
+template <class Kern, class... Args>
+int launch_gn_kernel(Kern kern, const GnShape& g, int n_models, cudaStream_t s, Args... args) {
+  // always: the default dynamic limit is 48 KB less the kernel's static shared memory
+  SB_CUDA_TRY(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)g.smem));
+  kern<<<dim3((unsigned)g.blocks, (unsigned)n_models), g.threads, (size_t)g.smem, s>>>(args...);
+  SB_LAUNCH_CHECK("rollout_gn_kernel");
+  return SB_OK;
+}
+
+template <int D, int PC>
+int launch_gn_spec(const GnArgs& a, const GnShape& g, int method, int n_models, cudaStream_t s) {
+  if (method == SB_EULER) return launch_gn_kernel(rollout_gn_spec_kernel<D, PC, SB_EULER>, g, n_models, s, a);
+  return launch_gn_kernel(rollout_gn_spec_kernel<D, PC, SB_RK4>, g, n_models, s, a);
+}
+
+int launch_gn(const LibTab& t, const GnArgs& a, const GnShape& g, int method, int n_models, cudaStream_t s) {
+#define X(D, PC) \
+  if (lib_matches<D, PC>(t)) return launch_gn_spec<D, PC>(a, g, method, n_models, s);
+  SB_SPEC_SHAPES(X)
+#undef X
+  if (t.K <= 16) return launch_gn_kernel(rollout_gn_gen_kernel<16>, g, n_models, s, t, method, a);
+  if (t.K <= 64) return launch_gn_kernel(rollout_gn_gen_kernel<64>, g, n_models, s, t, method, a);
+  return launch_gn_kernel(rollout_gn_gen_kernel<256>, g, n_models, s, t, method, a);
+}
+
 // workspace: [partial rows: n_models × IC blocks × d·K fp64, padded to 256 bytes][checkpoints: n_ckpt × n_models ×
 // n_ics × d fp32], n_ckpt = ⌈n_rows·steps_per_row / kCkpt⌉
 struct GradLayout {
@@ -971,6 +1334,68 @@ int rollout_score_grad(const float* x0, int64_t x0_model_stride, int64_t n_ics, 
   const int64_t n = (int64_t)n_models * dk;
   grad_sum_kernel<<<(unsigned)((n + 255) / 256), 256, 0, s>>>(partial, nblk, dk, n, grad);
   SB_LAUNCH_CHECK("grad_sum_kernel");
+  return SB_OK;
+}
+
+// workspace: one fp64 row of P(P+1)/2 + P θ sums per (model, IC-group block)
+int64_t rollout_score_gn_workspace_bytes(int64_t n_ics, const LibTab& t, int n_models, int n_params, int x0_blocks) {
+  const GnShape g = gn_shape(n_ics, t, n_params, x0_blocks ? t.d : 0, gn_spec(t));
+  int64_t b;
+  if (__builtin_mul_overflow((int64_t)n_models * g.blocks, (gn_tri(n_params) + n_params) * 8, &b)) return -1;
+  return b;
+}
+
+int rollout_score_gn(const float* x0, int64_t x0_model_stride, int64_t n_ics, const LibTab& t, const float* w,
+                     int n_models, const int32_t* params, int n_params, double dt, int64_t steps_per_row,
+                     int64_t n_rows, int method, const float* y_obs, float blowup, double* sse, int32_t* valid_rows,
+                     double* jtj, double* jtr, double* jtj_px, double* jtj_xx, double* jtr_x, void* ws,
+                     int64_t ws_bytes, cudaStream_t s) {
+  const int X = jtj_px ? t.d : 0;
+  const int64_t need = rollout_score_gn_workspace_bytes(n_ics, t, n_models, n_params, X != 0);
+  if (need < 0) {
+    set_error("rollout_score_gn workspace size overflows int64");
+    return SB_ERR_INVALID;
+  }
+  if (ws_bytes < need) {
+    set_error("workspace too small: %lld < %lld bytes", (long long)ws_bytes, (long long)need);
+    return SB_ERR_WORKSPACE;
+  }
+  const GnShape g = gn_shape(n_ics, t, n_params, X, gn_spec(t));
+  int dev = 0, smem_max = 0;
+  SB_CUDA_TRY(cudaGetDevice(&dev));
+  SB_CUDA_TRY(cudaDeviceGetAttribute(&smem_max, cudaDevAttrMaxSharedMemoryPerBlockOptin, dev));
+  if (g.smem + 1024 > smem_max) {
+    set_error("rollout_score_gn needs %lld bytes of shared memory per block, the device has %d", (long long)g.smem,
+              smem_max);
+    return SB_ERR_UNSUPPORTED;
+  }
+  const int64_t per = gn_tri(n_params) + n_params;
+  double* partial = reinterpret_cast<double*>(ws);
+  GnArgs a{};
+  a.s.x0_model_stride = x0_model_stride;
+  a.s.n_ics = n_ics; a.s.dt = dt; a.s.steps_per_row = steps_per_row; a.s.n_rows = n_rows;
+  a.s.y_obs = y_obs; a.s.blowup = blowup; a.s.opaque = 0;
+  a.P = n_params; a.X = X; a.T = g.T; a.G = g.G; a.n_groups = g.n_groups;
+  // more models than gridDim.y allows: further launches on the same stream
+  for (int m0 = 0; m0 < n_models; m0 += kMaxGridY) {
+    const int nm = n_models - m0 < kMaxGridY ? n_models - m0 : kMaxGridY;
+    a.s.x0 = x0 + (int64_t)m0 * x0_model_stride;
+    a.s.w = w + (int64_t)m0 * t.d * t.K;
+    a.s.sse = sse + (int64_t)m0 * n_ics;
+    a.s.valid = valid_rows + (int64_t)m0 * n_ics;
+    a.params = params + (int64_t)m0 * n_params;
+    a.partial = partial + (int64_t)m0 * g.blocks * per;
+    if (X) {
+      a.jtj_px = jtj_px + (int64_t)m0 * n_ics * n_params * X;
+      a.jtj_xx = jtj_xx + (int64_t)m0 * n_ics * X * X;
+      a.jtr_x = jtr_x + (int64_t)m0 * n_ics * X;
+    }
+    const int st = launch_gn(t, a, g, method, nm, s);
+    if (st != SB_OK) return st;
+  }
+  const int64_t n = (int64_t)n_models * ((int64_t)n_params * n_params + n_params);
+  gn_sum_kernel<<<(unsigned)((n + 255) / 256), 256, 0, s>>>(partial, g.blocks, n_params, params, n, jtj, jtr);
+  SB_LAUNCH_CHECK("gn_sum_kernel");
   return SB_OK;
 }
 

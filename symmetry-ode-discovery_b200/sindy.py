@@ -962,6 +962,145 @@ def refine_path(regressor, path, x_fit, dt, steps_per_row=1, method='rk4', blowu
     return out
 
 
+def _schur_starts(jtj, jtj_px, jtj_xx):
+    """S = F_θθ − Σ_n F_θx,n (F_xx,n + I)⁻¹ F_θx,nᵀ: the information of θ with every start x_n eliminated, the +I from
+    the row-0 residual x_n − row 0. jtj (U, P, P), jtj_px (U, N, P, d), jtj_xx (U, N, d, d), fp64."""
+    eye = torch.eye(jtj_xx.shape[-1], dtype=jtj_xx.dtype, device=jtj_xx.device)
+    Z = torch.linalg.solve(jtj_xx + eye, jtj_px.transpose(-1, -2))              # (U, N, d, P)
+    return jtj - torch.einsum('unpd,undq->upq', jtj_px, Z)
+
+
+def _gn_covariance(S, sigma2, A=None):
+    """σ²·A (AᵀSA)⁻¹ Aᵀ (A = None: σ²·S⁻¹) from a Cholesky factorisation of the equilibrated D·AᵀSA·D, D = diag^(−1/2);
+    columns of A that are zero are dropped first. Returns (covariance, condition number of the equilibrated matrix), or
+    (None, inf) when it is not positive definite."""
+    if A is not None:
+        A = A[:, A.abs().sum(0) > 0]                        # parameters that reach no listed coefficient
+        S = A.T @ S @ A
+    dg = torch.diagonal(S)
+    if S.shape[0] == 0 or not bool(torch.isfinite(S).all()) or not bool((dg > 0).all()):
+        return None, math.inf
+    Dm = dg.rsqrt()
+    Se = Dm[:, None] * S * Dm[None, :]
+    L, info = torch.linalg.cholesky_ex(Se)
+    if int(info) != 0:
+        return None, math.inf
+    ev = torch.linalg.eigvalsh(Se)
+    cond = float(ev[-1] / ev[0]) if float(ev[0]) > 0 else math.inf
+    cov = sigma2 * (Dm[:, None] * torch.cholesky_inverse(L) * Dm[None, :])
+    return (cov if A is None else A @ cov @ A.T), cond
+
+
+def coefficient_covariance(regressor, path, x, dt, steps_per_row=1, method='rk4', blowup=None, fit_ic=False,
+                           window=None):
+    """Gauss–Newton covariance of the coefficients of a `refine_path` result (with its arguments: the same
+    trajectories, step, method, fit_ic and window; with fit_ic=True, path['x0'] holds the fitted starts).
+
+    The refit minimises the simulation SSE with iid Gaussian residuals on every compared row (and on row 0 for the
+    starts), so Cov(θ) ≈ σ̂²·S⁻¹ with S = JᵀJ, J the Jacobian of every compared state with respect to the parameters.
+    Every distinct candidate (coefficients and mask, and starts with fit_ic) is evaluated once, all of them in one
+    `native.rollout_score_gn` launch (tangent-linear rollouts of the fp32 recurrence that was scored), which gives
+    F_θθ = Σ JθᵀJθ over the live coefficients and, with fit_ic, the per-start blocks F_θx,n and F_xx,n. The starts are
+    eliminated by the Schur complement S = F_θθ − Σ_n F_θx,n (F_xx,n + I)⁻¹ F_θx,nᵀ (the +I is the row-0 residual);
+    without fit_ic S = F_θθ and the starts count as exact. σ̂² = SSE / (n_obs − k_eff), n_obs and k_eff = live
+    coefficients (+ n_starts·d) as `score_path` counts them. S⁻¹ comes from a Cholesky factorisation of D·S·D,
+    D = diag(S)^(−1/2), in fp64. An equivariance-constrained regressor is parametrised by (β, const): vec(Ξ) = A·q with A
+    from `sweep.param_map` restricted to the live rows (and to the columns that reach them), S_q = AᵀSA and
+    Cov(vec Ξ) = A·Cov_q·Aᵀ.
+
+    Returns, per path entry: sse (P,) fp64 (rows compared, plus the row-0 residuals with fit_ic), sigma2 (P,), cov
+    (P, d·K, d·K) fp64 over vec(Ξ) (equation-major), zero off the mask; stderr (P, d, K), the square root of its
+    diagonal, zero off the mask; tstat = Ξ / stderr on the mask; cond (P,), the condition number of D·S·D;
+    identifiable (P,) bool, False when the factorisation fails (stderr is then +inf and cov NaN on the mask); diverged
+    (P,) bool as in `score_path` (stderr and cov are then NaN on the mask); n_obs. All on the host."""
+    import sweep
+    lib = getattr(regressor, 'library', regressor)
+    if not isinstance(lib, Library):
+        raise ValueError(f"regressor must be a SINDyRegression or a native.Library, got {type(regressor).__name__}")
+    constrained = bool(getattr(regressor, 'constraint', False))
+    x, dt = _check_rollout_args(lib, x, "x", dt, steps_per_row, method, blowup, fit_ic, window)
+    n_traj, T, d = x.shape
+    K, dK = lib.K, d * lib.K
+    W0, masks = path["xi"], path["mask"]
+    if W0.dim() != 3 or W0.shape[1:] != (d, K) or masks.shape != W0.shape:
+        raise ValueError(f"path['xi'] / path['mask'] must be (P, {d}, {K}), got {tuple(W0.shape)} / "
+                         f"{tuple(masks.shape)}")
+    P = W0.shape[0]
+    dev = W0.device
+    if fit_ic:
+        if "x0" not in path:
+            raise ValueError("fit_ic=True needs the fitted starts path['x0'] (refine_path(fit_ic=True) adds them)")
+        x0p = torch.as_tensor(path["x0"])
+        if x0p.shape != (P, n_traj, d):
+            raise ValueError(f"path['x0'] must be ({P}, {n_traj}, {d}), got {tuple(x0p.shape)}")
+        if not bool(torch.isfinite(x0p).all()):
+            raise ValueError("path['x0'] has non-finite values")
+        x0p = x0p.to(device=dev, dtype=torch.float32)
+    n_live_max = int(masks.flatten(1).sum(1).max()) if P else 0
+    if n_live_max + (d if fit_ic else 0) > native.GN_MAX_COLS:
+        raise ValueError(f"{n_live_max} live coefficients{' and ' + str(d) + ' start columns' if fit_ic else ''} "
+                         f"exceed the {native.GN_MAX_COLS} tangent columns of native.rollout_score_gn")
+    xf = x.to(device=dev, dtype=torch.float32)
+    x0, y = xf[:, 0].contiguous(), xf[:, 1:].transpose(0, 1).contiguous()
+    n_obs, k_ic = _obs_counts(n_traj, T, d, fit_ic)
+    # distinct candidates (coefficients, mask and starts), each evaluated once
+    key = [W0.reshape(P, -1), masks.reshape(P, -1).to(W0.dtype)] + ([x0p.reshape(P, -1).to(W0.dtype)] if fit_ic else [])
+    _, inverse = torch.unique(torch.cat(key, 1), dim=0, return_inverse=True)
+    U = int(inverse.max()) + 1
+    first = torch.full((U,), P, dtype=torch.long, device=dev).scatter_reduce(0, inverse.to(dev),
+                                                                            torch.arange(P, device=dev), 'amin')
+    mk = masks[first].reshape(U, dK)
+    live = [torch.nonzero(mk[u]).flatten() for u in range(U)]
+    n_par = max(1, max(int(v.numel()) for v in live))
+    params = torch.full((U, n_par), -1, dtype=torch.int32, device=dev)
+    for u, v in enumerate(live):
+        params[u, :v.numel()] = v.to(torch.int32)
+    Wu = (W0[first].reshape(U, dK) * mk).to(torch.float32).view(U, d, K)
+    with torch.no_grad():
+        gn = native.rollout_score_gn(x0p[first] if fit_ic else x0, Wu, params, lib, dt, int(steps_per_row), y, method,
+                                     blowup, x0_blocks=fit_ic)
+        sse = gn["sse"].sum(1)
+        S = gn["jtj"]
+        if fit_ic:
+            r = x0p[first].to(torch.float64) - x0.to(torch.float64)
+            sse = sse + (r * r).sum((1, 2))
+            S = _schur_starts(S, gn["jtj_px"], gn["jtj_xx"])
+        diverged = (gn["valid_rows"] < T - 1).any(1)
+        A = sweep.param_map(regressor)[0].to(dev) if constrained else None
+        k_eff = mk.sum(1).to(torch.float64) + k_ic
+        den = n_obs - k_eff
+        sigma2 = torch.where(den > 0, sse / den.clamp_min(1.0), torch.full_like(sse, math.nan))
+        cov = torch.zeros(U, dK, dK, dtype=torch.float64)
+        cond = torch.full((U,), math.inf, dtype=torch.float64)
+        ident = torch.zeros(U, dtype=torch.bool)
+        S, sigma2_h, div_h = S.cpu(), sigma2.cpu(), diverged.cpu()
+        for u, v in enumerate(live):
+            n, vc = int(v.numel()), v.cpu()
+            if n == 0:
+                ident[u] = True
+                cond[u] = 1.0
+                continue
+            blk = torch.full((n, n), math.nan, dtype=torch.float64)
+            if not bool(div_h[u]):
+                c, cond[u] = _gn_covariance(S[u, :n, :n], float(sigma2_h[u]), None if A is None else A.cpu()[vc])
+                if c is not None:
+                    blk, ident[u] = c, True
+            cov[u][vc[:, None], vc[None, :]] = blk
+        inv = inverse.cpu()
+        cov = cov[inv]
+        mflat = masks.reshape(P, dK).cpu()
+        var = torch.diagonal(cov, dim1=1, dim2=2)
+        se = torch.where(mflat, var.sqrt(), torch.zeros_like(var))
+        ident, div_p = ident[inv], div_h[inv]
+        bad = (~ident & ~div_p)[:, None] & mflat
+        se = torch.where(bad, torch.full_like(se, math.inf), se)
+        se = se.view(P, d, K)
+        xi = (W0.reshape(P, dK).cpu().to(torch.float64) * mflat).view(P, d, K)
+        tstat = torch.where(masks.cpu(), xi / se, torch.zeros_like(xi))
+    return {"sse": sse.cpu()[inv], "sigma2": sigma2_h[inv], "cov": cov, "stderr": se, "tstat": tstat,
+            "cond": cond[inv], "identifiable": ident, "diverged": div_p, "n_obs": n_obs}
+
+
 def information_criteria(sse, n, k):
     """AIC, AICc and BIC of Gaussian residuals with sum of squares `sse` over n observations and k parameters (fp64
     tensors of one shape, or scalars): n·ln(SSE/n) + 2k, that + 2k(k+1)/(n−k−1) (+inf when n−k−1 ≤ 0), and

@@ -82,6 +82,10 @@ _SIGNATURES = {
     "sb_rollout_score_grad_ics": (c_int, [c_void_p, c_int, c_int64, POINTER(_CLibrary), c_void_p, c_int, c_double,
                                           c_int64, c_int64, c_int, c_void_p, c_float, c_void_p, c_void_p, c_void_p,
                                           c_void_p, c_void_p, c_int64, c_void_p]),
+    "sb_rollout_score_gn_workspace_bytes": (c_int64, [c_int64, POINTER(_CLibrary), c_int, c_int, c_int]),
+    "sb_rollout_score_gn": (c_int, [c_void_p, c_int, c_int64, POINTER(_CLibrary), c_void_p, c_int, c_void_p, c_int,
+                                    c_double, c_int64, c_int64, c_int, c_void_p, c_float, c_void_p, c_void_p, c_void_p,
+                                    c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int64, c_void_p]),
     "sb_wsindy_integrals": (c_int, [c_void_p, c_int64, c_int64, POINTER(_CLibrary), c_float, c_double, c_int,
                                     c_void_p, c_void_p, c_void_p]),
     "sb_wsindy_local_integrals": (c_int, [c_void_p, c_int64, c_int64, POINTER(_CLibrary), c_void_p, c_void_p, c_int,
@@ -631,6 +635,64 @@ def rollout_score_grad(x0: torch.Tensor, W: torch.Tensor, lib: Library, dt: floa
                                             _ptr(grad), _ptr(gx0), ws.data_ptr(), nb, _stream(dev)),
                "sb_rollout_score_grad_ics")
     return done
+
+
+# most tangent columns of rollout_score_gn (SB_GN_MAX_COLS): n_params, plus d with x0_blocks
+GN_MAX_COLS = 176
+
+
+def rollout_score_gn(x0: torch.Tensor, W: torch.Tensor, params: torch.Tensor, lib: Library, dt: float,
+                     steps_per_row: int, y_obs: torch.Tensor, method: str = "rk4", blowup: Optional[float] = None,
+                     x0_blocks: bool = False):
+    """rollout_score and the Gauss–Newton information of its scores. params (M × P int, or P for every model): indices
+    into the flat d×K W[m] of the coefficients θ, −1 = padding. With J = ∂x_r/∂θ at every compared row of a pair (the
+    tangent-linear of the fp32 recurrence that was scored) and E = x_r − y_r, returns a dict of sse / valid_rows
+    (bit-identical to rollout_score's), jtj (M × P × P fp64) = Σ_pairs Σ_r JᵀJ and jtr (M × P fp64) = Σ JᵀE; padded
+    rows and columns are exact zeros. x0_blocks=True also treats each pair's start as a parameter, J_x = ∂x_r/∂x0, and
+    adds jtj_px (M × N × P × d) = Σ_r JᵀJ_x, jtj_xx (M × N × d × d) = Σ_r J_xᵀJ_x and jtr_x (M × N × d) = Σ_r J_xᵀE,
+    per pair. P (+ d with x0_blocks) is at most GN_MAX_COLS. See sb_rollout_score_gn."""
+    x0f, per_model, W, y, meth, dev = _score_args(x0, W, lib, dt, steps_per_row, y_obs, method, blowup)
+    n_ics, d = x0f.shape[-2:]
+    n_models = W.shape[0]
+    if not isinstance(x0_blocks, bool):
+        raise ValueError(f"x0_blocks must be True or False, got {x0_blocks!r}")
+    prm = torch.as_tensor(params)
+    if prm.is_floating_point() or prm.dtype == torch.bool or prm.is_complex():
+        raise ValueError(f"params must be an integer tensor, got {prm.dtype}")
+    if prm.dim() == 1:
+        prm = prm.unsqueeze(0).expand(n_models, -1)
+    if prm.dim() != 2 or prm.shape[0] != n_models or prm.shape[1] < 1:
+        raise ValueError(f"params has shape {tuple(prm.shape)}, expected ({n_models}, n_params >= 1)")
+    P = prm.shape[1]
+    cols = P + (d if x0_blocks else 0)
+    if cols > GN_MAX_COLS:
+        raise ValueError(f"{P} parameters{' and ' + str(d) + ' start columns' if x0_blocks else ''} exceed the "
+                         f"{GN_MAX_COLS} tangent columns of rollout_score_gn")
+    if prm.numel() and (int(prm.min()) < -1 or int(prm.max()) >= d * lib.K):
+        raise ValueError(f"params must lie in [-1, {d * lib.K}), got [{int(prm.min())}, {int(prm.max())}]")
+    prm = prm.to(device=dev, dtype=torch.int32).contiguous()
+    f64 = dict(dtype=torch.float64, device=dev)
+    out = {"sse": torch.empty(n_models, n_ics, **f64),
+           "valid_rows": torch.empty(n_models, n_ics, dtype=torch.int32, device=dev),
+           "jtj": torch.zeros(n_models, P, P, **f64), "jtr": torch.zeros(n_models, P, **f64)}
+    if x0_blocks:
+        out.update(jtj_px=torch.zeros(n_models, n_ics, P, d, **f64), jtj_xx=torch.zeros(n_models, n_ics, d, d, **f64),
+                   jtr_x=torch.zeros(n_models, n_ics, d, **f64))
+    if n_models == 0 or n_ics == 0:
+        return out
+    sl = load()
+    nb = int(sl.sb_rollout_score_gn_workspace_bytes(n_ics, ctypes.byref(lib.c()), n_models, P, int(x0_blocks)))
+    if nb < 0:
+        _check(nb, "sb_rollout_score_gn_workspace_bytes")
+    ws = torch.empty(max(nb, 1), dtype=torch.uint8, device=dev)
+    with torch.cuda.device(dev):
+        _check(sl.sb_rollout_score_gn(x0f.data_ptr(), int(per_model), n_ics, ctypes.byref(lib.c()), W.data_ptr(),
+                                      n_models, prm.data_ptr(), P, float(dt), int(steps_per_row), y.shape[0], meth,
+                                      y.data_ptr(), 0.0 if blowup is None else float(blowup), out["sse"].data_ptr(),
+                                      out["valid_rows"].data_ptr(), out["jtj"].data_ptr(), out["jtr"].data_ptr(),
+                                      _ptr(out.get("jtj_px")), _ptr(out.get("jtj_xx")), _ptr(out.get("jtr_x")),
+                                      ws.data_ptr(), nb, _stream(dev)), "sb_rollout_score_gn")
+    return out
 
 
 def wsindy_integrals(x: torch.Tensor, lib: Library, dt: float, t_max: float, n_test: int = 50):
